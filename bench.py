@@ -25,6 +25,18 @@ eps-greedy, Basic, 1 048 576 agents per GPU (weak scaling), f32.  The same JSON 
   c2_f64  the headline configuration in the reference's own arithmetic (f64).
 `--workload X` measures one configuration alone; `--sub ''` drops the sub-records.
 
+`--dump-outputs DIR` writes, for the headline and every sub-record, what the last timed step returned to its caller
+(.npy files, at most 64 MB in all) so that two builds can be compared output for output on the same inputs:
+  <name>_<dtype>_episode_sums          device leg: per-episode sums [cells, episodes, 4] ([cells, gpus, episodes, 4],
+                                       rank 0's gather, on several GPUs)
+  <name>_<dtype>_e2e_episode_sums      e2e leg: the same sums, as copied to host memory
+  <name>_<dtype>_e2e_episodes          e2e leg: per-agent episode records (ret, td_sum, td_abs_sum, length) of a fixed,
+                                       seeded sample of rank 0's agents [cells, episodes, agents, 4]
+Each is float64 with its non-finite entries written as 0, beside a float32 <file>_nonfinite of the same shape that marks
+them (0 finite, 1 NaN, 2 +inf, 3 -inf).  Non-finite values are the reference's arithmetic, not a fault: under UCB an
+unvisited action's bonus is +inf once t >= 55, so Expected Sarsa's target is inf/inf = NaN and c3's TD sums are NaN
+(SURVEY.md 8.1 Q9, tests/test_oracle_kat.py::test_ucb_expected_sarsa_nan_quirk).
+
 `--impl reference` times the CPU oracle (the reference cannot be compiled here: no Rust
 toolchain) on the host cores, on a bounded sample of the same workload.
 """
@@ -41,6 +53,22 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the bench leaves the tree as it found it (it may be read-only)
+DUMP_BYTES = 60 * 10 ** 6        # --dump-outputs: all arrays together, below 64 MB with the .npy headers
+DUMP_ELEM_BYTES = 8 + 4          # --dump-outputs: a float64 value and its float32 _nonfinite code
+DUMP_SEED = 0x5EED               # --dump-outputs: which agents' episode records are sampled
+
+
+def save_output(out_dir, name, arr):
+    """--dump-outputs: `name`.npy holds `arr` with its non-finite entries set to 0, and `name`_nonfinite.npy says which
+    they were (0 finite, 1 NaN, 2 +inf, 3 -inf), so that every file is finite and nothing the path computed is lost."""
+    arr = np.asarray(arr, np.float64)
+    code = np.zeros(arr.shape, np.float32)
+    code[np.isnan(arr)] = 1
+    code[np.isposinf(arr)] = 2
+    code[np.isneginf(arr)] = 3
+    np.save(os.path.join(out_dir, name + ".npy"), np.where(code == 0, arr, 0.0))
+    np.save(os.path.join(out_dir, name + "_nonfinite.npy"), code)
 
 
 def _workloads():
@@ -233,9 +261,10 @@ class Job:
             self.dist.destroy_process_group()
 
 
-def measure(job, args, name, w, real, steps, warmup, with_e2e, cpu_agents, cell_streams):
+def measure(job, args, name, w, real, steps, warmup, with_e2e, cpu_agents, cell_streams, outputs=None, dump_bytes=0):
     """One configuration on this job's GPUs: W warm-up steps, K timed steps (device value), the e2e leg, the CPU
-    baseline sample.  Returns the record (rank 0) or None."""
+    baseline sample.  Returns the record (rank 0) or None.  `outputs` (a dict) receives, on rank 0, what the last
+    timed step of each leg returned, at most `dump_bytes` of it (--dump-outputs)."""
     torch = job.torch
     W = _workloads()
     rlb = importlib.import_module("rl-rust_b200")
@@ -347,6 +376,12 @@ def measure(job, args, name, w, real, steps, warmup, with_e2e, cpu_agents, cell_
         remeasured = True
     clocks["remeasured_after_slowdown"] = remeasured
     dev = dict(acc)
+    dump = outputs is not None and rank == 0
+    if dump:   # taken now: the e2e leg's untimed steps write the same device buffers
+        prefix = "%s_%s_" % (name, dtype)
+        last = (state["k"] - 1) & 1
+        outputs[prefix + "episode_sums"] = np.stack([(gathered[ci][last] if world > 1 else sums_dev[ci]).cpu().numpy()
+                                                     for ci in range(len(cells))])
 
     # ---- e2e leg: same steps through the asynchronous C-ABI call with pinned HOST buffers; two record buffers per cell
     # take turns (step k fills buffer k & 1 while the host may still be reading the other)
@@ -377,6 +412,17 @@ def measure(job, args, name, w, real, steps, warmup, with_e2e, cpu_agents, cell_
             stream.wait_stream(s_)
         e1.record(stream)
         job.barrier()
+        if dump:
+            last = (state["k"] - 1) & 1
+            sums = np.stack([(host_gath[ci] if world > 1 else host_sums[ci]).numpy() for ci in range(len(cells))])
+            outputs[prefix + "e2e_episode_sums"] = sums
+            room = dump_bytes - DUMP_ELEM_BYTES * (outputs[prefix + "episode_sums"].size + sums.size)
+            n_sample = max(0, min(N, room // (len(cells) * chunk * 4 * DUMP_ELEM_BYTES)))
+            if n_sample:
+                idx = np.sort(np.random.default_rng(DUMP_SEED).choice(N, n_sample, replace=False))
+                recs = np.stack([host_recs[ci][last].numpy().view(eng.episode_dtype).reshape(chunk, N)[:, idx]
+                                 for ci in range(len(cells))])
+                outputs[prefix + "e2e_episodes"] = np.stack([recs[f].astype(np.float64) for f in ("ret", "td_sum", "td_abs_sum", "length")], -1)
         e2e = {"ms": e0.elapsed_time(e1), "train_steps": acc["train_steps"], "kernel_ms": acc["kernel_ms"],
                "d2h": len(cells) * (rec_bytes + chunk * 32 + 64) + (len(cells) * world * chunk * 32 if (world > 1 and rank == 0) else 0),
                "h2d": 24 * len(cells), "double_buf": double_buf}
@@ -483,6 +529,8 @@ def main():
                          "'c4,c3,c2_f64' for the default headline run, none when --workload / --agents-per-gpu / --real is given")
     ap.add_argument("--sub-steps", type=int, default=10, help="timed steps of each sub-record (10 = one whole 1000-episode run)")
     ap.add_argument("--sub-warmup", type=int, default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
     W = _workloads()
     w = dict(W.WORKLOADS[args.workload])
@@ -503,8 +551,11 @@ def main():
     subs = [s for s in subs.split(",") if s]
 
     job = Job()
+    outputs = {} if args.dump_outputs else None
+    dump_bytes = DUMP_BYTES // (1 + len(subs))   # an equal share for every measured configuration
     cpu_agents = 0 if args.no_cpu_baseline else (512 if "cells" not in w else 4)   # ~10 s of single-thread CPU work
-    line = measure(job, args, args.workload, w, real, args.steps, args.warmup, not args.no_e2e, cpu_agents, args.cell_streams)
+    line = measure(job, args, args.workload, w, real, args.steps, args.warmup, not args.no_e2e, cpu_agents, args.cell_streams,
+                   outputs, dump_bytes)
     sub_records = {}
     saved_apg = args.agents_per_gpu
     for sname in subs:
@@ -514,13 +565,18 @@ def main():
         sreal = 1 if suffix == "f64" else 0
         # CPU samples of the sub-records are sized for a few seconds each (C3 executes ~6x its training steps in evaluate)
         scpu = 0 if args.no_cpu_baseline else {"c4": 512, "c3": 64, "c2": 256, "c1": 512}.get(base, 0)
-        r = measure(job, args, base, sw, sreal, args.sub_steps, max(3, args.sub_warmup), not args.no_e2e, scpu, args.cell_streams)
+        r = measure(job, args, base, sw, sreal, args.sub_steps, max(3, args.sub_warmup), not args.no_e2e, scpu, args.cell_streams,
+                    outputs, dump_bytes)
         if r is not None:
             sub_records[sname] = r
     args.agents_per_gpu = saved_apg
     if job.rank == 0:
         if sub_records:
             line["workloads"] = sub_records
+        if outputs is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for oname, arr in outputs.items():
+                save_output(args.dump_outputs, oname, arr)
         print(json.dumps(line), flush=True)
     job.close()
 

@@ -160,7 +160,8 @@ typedef struct rlb_traj_record {
 typedef struct rlb_train_out {
     /* [n_episodes][4] f64, reduced over this engine's agents per episode index:
      * sum(length), sum(return), sum(td_sum), sum(td_abs_sum).  Divide by n_agents for the
-     * reference's per-run curves.  This is what multi-GPU runs gather. */
+     * reference's per-run curves.  This is what multi-GPU runs gather.  [n_episodes][n_sets][4], one reduction
+     * per set, while rlb_engine_set_hparams sets are installed. */
     double* episode_sums;
     /* [n_episodes][n_agents] rlb_episode_f32 / rlb_episode_f64 (by rlb_config.real): the
      * raw per-agent stream (reward_history, episode_length of agent.rs:117). */
@@ -220,6 +221,40 @@ rlb_status rlb_engine_synchronize(rlb_engine* e);
 rlb_status rlb_engine_dims(const rlb_engine* e, uint32_t* n_states, uint32_t* n_actions, uint32_t* n_tables);
 /* which table store the engine picked (1 HBM, 2 shared memory thread groups, 3 hybrid, 4 HBM + lazy trace sweeps) */
 uint32_t rlb_engine_store_kind(const rlb_engine* e);
+
+/* ---- per-agent hyper-parameter sets (no reference equivalent: the bins build one agent per run and sweep the
+ * constructor arguments by hand, bin/taxi.rs:22-68) ------------------------------------------------------------------
+ * The constructor arguments the bins vary, per agent:
+ *   TabularPolicy::new(lr, default) tabular_policy.rs:15 / DoubleTabularPolicy::new(lr, default) double_tabular_policy.rs:17,
+ *   UniformEpsilonGreed::new(eps, decay, final) uniform_epsilon_greed.rs:31, UpperConfidenceBound::new(c)
+ *   upper_confidence_bound.rs:17, OneStepAgent::new(.., gamma, ..) one_step_agent.rs:16 /
+ *   ElegibilityTracesAgent::new(.., gamma, .., lambda, ..) elegibility_traces_agent.rs:21.
+ * Field for field the hyper-parameters of rlb_config. */
+typedef struct rlb_hparams {
+    double learning_rate, discount_factor, lambda_factor;
+    double initial_epsilon, epsilon_decay, final_epsilon;   /* epsilon_decay: the k of rlb_config.decay_kind */
+    double confidence_level, default_value;
+} rlb_hparams;                                             /* 64 bytes */
+#define RLB_MAX_HPARAM_SETS 65536
+/* sets [n_sets]; group [N] u32: agent i is constructed with sets[group[i]].  Host or device buffers.
+ * sets = NULL, n_sets = 0, group = NULL: back to rlb_config's values.
+ * Constructor equivalence: after this call every call gives agent i the results, bit for bit, of agent 0 of an engine
+ * created with rlb_config's eight hyper-parameters replaced by sets[group[i]], n_agents = 1 and first_agent_id + i.  So
+ * the call acts as the constructor of the agents: their tables are refilled with their own default_value, epsilon set to
+ * their initial_epsilon, UCB counts and t reset, policy_flag set (as rlb_agent_set_kind does; the env and the RNG
+ * stream carry on).  Every later reset (rlb_selector_reset, rlb_policy_reset, rlb_agent_reset, rlb_agent_set_kind,
+ * rlb_agent_set_action_selector) and compute call uses each agent's own set; decay_kind, target, agent kind, selector,
+ * policy, real type and env stay engine-wide.
+ * While sets are installed every per-episode sums output is [n_episodes][n_sets][4] (rlb_train_out.episode_sums,
+ * rlb_agent_evaluate's sums_out): entry (e, g) is the rlb_train_out reduction, in the same order, over the agents of
+ * set g in ascending local index — one set of all agents gives the [n_episodes][4] of an engine without sets, and a set
+ * of a contiguous id range the sums of an engine holding just those agents.  Gather them with
+ * rlb_comm_gather_episode_sums(.., n_episodes * n_sets, ..).
+ * RLB_ERR_INVALID_ARG, the engine untouched: n_sets == 0 with a non-NULL pointer, n_sets > 0 with a NULL one,
+ * n_sets > RLB_MAX_HPARAM_SETS, any group[i] >= n_sets.  Values are not checked.  RLB_ERR_UNSUPPORTED: a Dyna model
+ * (rlb_agent_set_model / rlb_config.planning_steps) together with sets, whichever comes second. */
+rlb_status rlb_engine_set_hparams(rlb_engine* e, const rlb_hparams* sets, uint32_t n_sets, const uint32_t* group);
+uint32_t rlb_engine_hparam_sets(const rlb_engine* e);    /* 0 while rlb_config's values apply */
 
 /* ---- Env<T,COUNT> (env.rs:19-49), batched ------------------------------------------------ */
 /* Env::reset (blackjack.rs:105, frozen_lake.rs:106, cliff_walking.rs:67, taxi.rs:135).  obs_out [N] u32 */
@@ -284,7 +319,8 @@ rlb_status rlb_agent_train_wait(rlb_engine* e);
 rlb_status rlb_agent_step(rlb_engine* e, uint8_t* kind_out, uint32_t* obs_out, uint32_t* action_out, double* reward_out,
                           uint8_t* terminated_out, void* td_out);
 /* Agent::evaluate (agent.rs:120-141).  episodes_out: [n_episodes][N] episode records
- * (td fields zero); sums_out [n_episodes][4] as in rlb_train_out.  Either may be NULL. */
+ * (td fields zero); sums_out [n_episodes][4] ([n_episodes][n_sets][4] with hyper-parameter sets) as in rlb_train_out.
+ * Either may be NULL. */
 rlb_status rlb_agent_evaluate(rlb_engine* e, uint64_t n_episodes, void* episodes_out, double* sums_out,
                               uint64_t* total_steps_out);
 

@@ -57,6 +57,15 @@ TRAJ_DTYPE = np.dtype([("kind", "u1"), ("action", "u1"), ("terminated", "u1"), (
 STATE_DTYPE = np.dtype([("epsilon", "<f8"), ("ucb_t", "<u8"), ("rng_n", "<u8"), ("policy_flag", "<i4"),
                         ("env_ready", "<i4")])
 MODEL_ENTRY = np.dtype([("obs", "<u4"), ("action", "<u4"), ("next_obs", "<u4"), ("reward", "<f4")])
+# rlb_hparams: one per-agent hyper-parameter set (rlb_engine_set_hparams), field for field rlb_config's
+HPARAM_FIELDS = ("learning_rate", "discount_factor", "lambda_factor", "initial_epsilon", "epsilon_decay", "final_epsilon",
+                 "confidence_level", "default_value")
+HPARAMS_DTYPE = np.dtype([(f, "<f8") for f in HPARAM_FIELDS])
+MAX_HPARAM_SETS = 65536
+
+
+class RlbHparams(C.Structure):
+    _fields_ = [(f, C.c_double) for f in HPARAM_FIELDS]
 
 # every symbol include/rlb.h declares
 EXPORTS = [
@@ -73,7 +82,7 @@ EXPORTS = [
     "rlb_agent_train_range_async", "rlb_agent_train_wait", "rlb_agent_step",
     "rlb_comm_unique_id", "rlb_comm_init_rank", "rlb_comm_init_all", "rlb_comm_destroy", "rlb_comm_rank", "rlb_comm_world_size",
     "rlb_comm_gather_episode_sums", "rlb_comm_allreduce_sum", "rlb_comm_group_begin", "rlb_comm_group_end",
-    "rlb_selftest_ucb_math",
+    "rlb_selftest_ucb_math", "rlb_engine_set_hparams", "rlb_engine_hparam_sets",
 ]
 
 
@@ -107,6 +116,9 @@ def _load():
     L.rlb_engine_dims.argtypes = [vp, P(u32), P(u32), P(u32)]
     L.rlb_engine_store_kind.restype = u32
     L.rlb_engine_store_kind.argtypes = [vp]
+    L.rlb_engine_set_hparams.argtypes = [vp, vp, u32, vp]
+    L.rlb_engine_hparam_sets.restype = u32
+    L.rlb_engine_hparam_sets.argtypes = [vp]
     L.rlb_env_reset.argtypes = [vp, vp]
     L.rlb_env_step.argtypes = [vp, vp, vp, vp, vp, vp]
     L.rlb_agent_get_action.argtypes = [vp, vp, vp]
@@ -232,6 +244,8 @@ class Engine:
         self.real = real
         self.rdtype = np.float32 if real == REAL_F32 else np.float64
         self.episode_dtype = EPISODE_F32 if real == REAL_F32 else EPISODE_F64
+        self.G = 0                  # hyper-parameter sets installed (set_hparams); per-episode sums are (E, G, 4) while G > 0
+        self.hparams = None         # (sets, group) as installed
 
     def close(self):
         if getattr(self, "h", None):
@@ -259,6 +273,47 @@ class Engine:
         agent's sweeps applied lazily (rlb.h: rlb_config.store_kind)."""
         return lib.rlb_engine_store_kind(self.h)
 
+    # ---- per-agent hyper-parameter sets
+    def hparams_array(self, sets):
+        """`sets` as an HPARAMS_DTYPE array: an array of that dtype as it is, or a list of dicts whose missing fields take
+        this engine's rlb_config values."""
+        if isinstance(sets, np.ndarray) and sets.dtype == HPARAMS_DTYPE:
+            return np.ascontiguousarray(sets)
+        arr = np.zeros(len(sets), HPARAMS_DTYPE)
+        for g, d in enumerate(sets):
+            unknown = set(d) - set(HPARAM_FIELDS)
+            if unknown:
+                raise ValueError("unknown hyper-parameter(s) %s; known: %s" % (sorted(unknown), ", ".join(HPARAM_FIELDS)))
+            for f in HPARAM_FIELDS:
+                arr[g][f] = float(d.get(f, getattr(self.cfg, f)))
+        return arr
+
+    def set_hparams(self, sets, group):
+        """rlb_engine_set_hparams: agent i is constructed with sets[group[i]] (fresh tables, epsilon and UCB state; see
+        include/rlb.h).  `sets`: a list of dicts (fields missing from a dict take the engine's configured value) or an
+        HPARAMS_DTYPE array; `group`: (N,) integers.  set_hparams(None, None) goes back to the configured values.
+        While sets are installed, train() and evaluate() return per-episode sums shaped (E, G, 4)."""
+        if sets is None and group is None:
+            check(lib.rlb_engine_set_hparams(self.h, None, 0, None))
+            self.G, self.hparams = 0, None
+            return
+        arr = self.hparams_array(sets)
+        grp = np.asarray(group)
+        if grp.shape != (self.N,):
+            raise ValueError("group must have shape (%d,), got %r" % (self.N, grp.shape))
+        if grp.size and (grp.min() < 0 or grp.max() >= 2 ** 32):
+            raise ValueError("group ids must be in [0, 2**32)")
+        grp = np.ascontiguousarray(grp, np.uint32)
+        check(lib.rlb_engine_set_hparams(self.h, ptr(arr) if len(arr) else None, len(arr), ptr(grp) if len(arr) else None))
+        self.G, self.hparams = len(arr), (arr.copy(), grp.copy())
+
+    def hparam_sets(self):
+        """rlb_engine_hparam_sets: the number of sets installed, 0 while the configured values apply."""
+        return lib.rlb_engine_hparam_sets(self.h)
+
+    def _sums_shape(self, n):
+        return (n, self.G, 4) if self.G else (n, 4)
+
     # ---- Agent::train / evaluate
     def train(self, n_episodes, eval_at, *, ep_begin=0, sums=True, episodes=False, traj_capacity=0, sums_out=None,
               episodes_out=None, td_capacity=0, wait=True):
@@ -274,7 +329,7 @@ class Engine:
             out.episode_sums = ptr(sums_out)
             res["sums"] = sums_out
         elif sums:
-            res["sums"] = np.zeros((n, 4), np.float64)
+            res["sums"] = np.zeros(self._sums_shape(n), np.float64)
             out.episode_sums = ptr(res["sums"])
         if episodes_out is not None:
             out.episodes = ptr(episodes_out)
@@ -330,7 +385,7 @@ class Engine:
     def evaluate(self, n_episodes, *, sums=True, episodes=False):
         """Agent::evaluate (agent.rs:120-141)."""
         res = {}
-        sums_buf = np.zeros((n_episodes, 4), np.float64) if sums else None
+        sums_buf = np.zeros(self._sums_shape(n_episodes), np.float64) if sums else None
         eps_buf = np.zeros((n_episodes, self.N), self.episode_dtype) if episodes else None
         steps = C.c_uint64()
         check(lib.rlb_agent_evaluate(self.h, n_episodes, ptr(eps_buf), ptr(sums_buf), C.byref(steps)))

@@ -88,6 +88,14 @@ struct rlb_engine {
     uint8_t* d_lz_tmat = nullptr;      //                    sweeps applied per slot  [N][VMAX]
     uint32_t d_lz_tmat_rows = 0;
     double* d_log_table = nullptr;     // ln(t) for t < RLB_LOG_TABLE_N (UCB), filled on the device by portable_log
+    // per-agent hyper-parameter sets (rlb_engine_set_hparams); hp_n = 0 while rlb_config's values apply
+    uint32_t hp_n = 0;
+    rlb_hparams* d_hp_sets = nullptr;  // [hp_n]
+    uint32_t* d_hp_group = nullptr;    // [N] set of each agent
+    uint32_t* d_hp_order = nullptr;    // [N] local agent indices, stably sorted by set: the grouped reduction's read order
+    uint32_t* d_hp_offsets = nullptr;  // [hp_n + 1] where each set starts in d_hp_order
+    void* d_hp_q0 = nullptr;           // [hp_n] default_value narrowed to Real, for the table fills
+    double* d_hp_eps0 = nullptr;       // [hp_n] initial_epsilon
     // Calls whose work is enqueued but not yet waited for (rlb_agent_train_range_async): at most two, so that the
     // kernels of call i + 1 are in the queue before the host blocks on the copies of call i.
     struct Pending {
@@ -175,8 +183,15 @@ cudaError_t fill(rlb_engine* e, V* ptr, uint64_t n, V value) {
 
 cudaError_t fill_q_default(rlb_engine* e) {
     const uint64_t n = e->q_bytes / e->real_size;
+    if (e->hp_n) return launch_fill_grouped(e->d_q, e->real_size, n / e->cfg.n_agents, e->cfg.n_agents, e->d_hp_q0, e->d_hp_group, e->stream);
     if (e->cfg.real_kind == RLB_REAL_F32) return fill<float>(e, (float*)e->d_q, n, (float)e->cfg.default_value);
     return fill<double>(e, (double*)e->d_q, n, e->cfg.default_value);
+}
+
+// UniformEpsilonGreed::new / reset: epsilon = initial_epsilon (uniform_epsilon_greed.rs:31,78-80)
+cudaError_t fill_eps_initial(rlb_engine* e) {
+    if (e->hp_n) return launch_fill_grouped(e->d_eps, sizeof(double), 1, e->cfg.n_agents, e->d_hp_eps0, e->d_hp_group, e->stream);
+    return fill<double>(e, e->d_eps, e->cfg.n_agents, e->cfg.initial_epsilon);
 }
 
 cudaError_t dispatch_run(rlb_engine* e, const DevParams& p) {
@@ -186,6 +201,15 @@ cudaError_t dispatch_run(rlb_engine* e, const DevParams& p) {
             case RLB_ENV_FROZEN_LAKE: return launch_run_model<RLB_ENV_FROZEN_LAKE>(e->variant, p, e->stream);
             case RLB_ENV_CLIFF_WALKING: return launch_run_model<RLB_ENV_CLIFF_WALKING>(e->variant, p, e->stream);
             default: return launch_run_model<RLB_ENV_TAXI>(e->variant, p, e->stream);
+        }
+    }
+    if (e->hp_n) {   // every agent with its own hyper-parameter set (never with a model: rlb_engine_set_hparams)
+        const HpParams sets{e->d_hp_sets, e->d_hp_group};
+        switch (e->cfg.env_kind) {
+            case RLB_ENV_BLACKJACK: return launch_run<RLB_ENV_BLACKJACK, true>(e->variant, p, e->store, e->stream, sets);
+            case RLB_ENV_FROZEN_LAKE: return launch_run<RLB_ENV_FROZEN_LAKE, true>(e->variant, p, e->store, e->stream, sets);
+            case RLB_ENV_CLIFF_WALKING: return launch_run<RLB_ENV_CLIFF_WALKING, true>(e->variant, p, e->store, e->stream, sets);
+            default: return launch_run<RLB_ENV_TAXI, true>(e->variant, p, e->store, e->stream, sets);
         }
     }
     switch (e->cfg.env_kind) {
@@ -272,6 +296,16 @@ rlb_status pick_store(rlb_engine* e) {
 }
 
 cudaError_t dispatch_step(rlb_engine* e, StepOp op, const StepArgs& a) {
+    if (e->hp_n) {
+        StepArgs with_sets = a;
+        with_sets.sets = HpParams{e->d_hp_sets, e->d_hp_group};
+        switch (e->cfg.env_kind) {
+            case RLB_ENV_BLACKJACK: return launch_step<RLB_ENV_BLACKJACK, true>(op, e->variant, e->dp, with_sets, e->stream);
+            case RLB_ENV_FROZEN_LAKE: return launch_step<RLB_ENV_FROZEN_LAKE, true>(op, e->variant, e->dp, with_sets, e->stream);
+            case RLB_ENV_CLIFF_WALKING: return launch_step<RLB_ENV_CLIFF_WALKING, true>(op, e->variant, e->dp, with_sets, e->stream);
+            default: return launch_step<RLB_ENV_TAXI, true>(op, e->variant, e->dp, with_sets, e->stream);
+        }
+    }
     switch (e->cfg.env_kind) {
         case RLB_ENV_BLACKJACK: return launch_step<RLB_ENV_BLACKJACK>(op, e->variant, e->dp, a, e->stream);
         case RLB_ENV_FROZEN_LAKE: return launch_step<RLB_ENV_FROZEN_LAKE>(op, e->variant, e->dp, a, e->stream);
@@ -343,7 +377,7 @@ rlb_status install_selector(rlb_engine* e, int kind) {
     const uint64_t N = e->cfg.n_agents;
     e->cfg.selector_kind = kind;
     e->variant.sel = kind;
-    CK(fill<double>(e, e->d_eps, N, e->cfg.initial_epsilon));
+    CK(fill_eps_initial(e));
     CK(fill<uint64_t>(e, e->d_ucb_t, N, 1ull));
     if (kind == RLB_SEL_UCB) {
         if (!e->d_counts) {
@@ -364,7 +398,7 @@ rlb_status install_selector(rlb_engine* e, int kind) {
 
 size_t episode_rec_size(const rlb_engine* e) { return e->cfg.real_kind == RLB_REAL_F32 ? sizeof(rlb_episode_f32) : sizeof(rlb_episode_f64); }
 
-rlb_status ensure_episode_scratch(rlb_engine* e, uint64_t episodes, uint64_t sums_episodes) {
+rlb_status ensure_episode_scratch(rlb_engine* e, uint64_t episodes, uint64_t sums_values) {
     const size_t need = (size_t)episodes * e->cfg.n_agents * episode_rec_size(e);
     if (e->episodes_cap < need) {
         if (e->d_episodes) cudaFree(e->d_episodes);
@@ -372,7 +406,7 @@ rlb_status ensure_episode_scratch(rlb_engine* e, uint64_t episodes, uint64_t sum
         CK(cudaMalloc(&e->d_episodes, need));
         e->episodes_cap = need;
     }
-    const size_t need_s = (size_t)sums_episodes * 4 * sizeof(double);
+    const size_t need_s = (size_t)sums_values * sizeof(double);
     if (e->sums_cap < need_s) {
         if (e->d_sums) cudaFree(e->d_sums);
         e->d_sums = nullptr; e->sums_cap = 0;
@@ -392,8 +426,13 @@ uint64_t chunk_episodes(const rlb_engine* e, uint64_t want) {
     return std::min<uint64_t>(chunk, std::max<uint64_t>(want, 1));
 }
 
+// sums_out [n_ep][4], or [n_ep][hp_n][4] with hyper-parameter sets
 rlb_status reduce_episodes(rlb_engine* e, uint64_t n_ep, const void* records, double* sums_out) {
     if (!n_ep) return RLB_OK;
+    if (e->hp_n) {
+        CK(launch_episode_sums_grouped(e->cfg.real_kind, records, e->cfg.n_agents, e->d_hp_order, e->d_hp_offsets, e->hp_n, n_ep, sums_out, e->stream));
+        return RLB_OK;
+    }
     if (e->cfg.real_kind == RLB_REAL_F32) k_episode_sums<float><<<(unsigned)n_ep, 256, 0, e->stream>>>(records, e->cfg.n_agents, sums_out);
     else k_episode_sums<double><<<(unsigned)n_ep, 256, 0, e->stream>>>(records, e->cfg.n_agents, sums_out);
     CK(cudaGetLastError());
@@ -511,6 +550,7 @@ rlb_status enqueue_range(rlb_engine* e, int mode, uint64_t begin, uint64_t end, 
     const uint64_t N = e->cfg.n_agents;
     const size_t rec = episode_rec_size(e);
     const uint64_t total = end - begin;
+    const uint64_t sums_per_ep = 4ull * (e->hp_n ? e->hp_n : 1u);   // [4] per episode, [n_sets][4] with hyper-parameter sets
     const bool want_records = mode == 0 ? (out && (out->episodes || out->episode_sums)) : (eval_episodes_out || eval_sums_out);
     uint64_t chunk = std::min<uint64_t>(total, 0xffffffffull);   // a launch counts its episodes in 32 bits
     // Records for a HOST buffer are pipelined: the range is cut into (at least) four launches writing alternately into
@@ -530,7 +570,7 @@ rlb_status enqueue_range(rlb_engine* e, int mode, uint64_t begin, uint64_t end, 
     // neither sends records to the host at all: then everything either call does is in main-stream order (the record
     // scratch is written by call i + 1's kernel only after call i's reduction has read it), and the blocks of totals
     // and sums are per call.
-    const bool sums_fit = 3 * total * 4 * sizeof(double) <= e->sums_cap && (size_t)chunk * N * rec <= e->episodes_cap;
+    const bool sums_fit = 3 * total * sums_per_ep * sizeof(double) <= e->sums_cap && (size_t)chunk * N * rec <= e->episodes_cap;
     const bool both_pipelined = pipelined && !e->pending.empty() && e->pending.back().pipelined && chunk == e->last_pipeline_chunk;
     const bool host_rec = rec_host && !is_device_ptr(rec_host);
     const bool both_on_device = !host_rec && !e->pending.empty() && !e->pending.back().pipelined && !e->pending.back().host_records;
@@ -545,12 +585,12 @@ rlb_status enqueue_range(rlb_engine* e, int mode, uint64_t begin, uint64_t end, 
     // kernel behind them: the whole record copy was serialised after all, profiles/r02e_e2e_probe_*.json.)
     const uint64_t slot = e->call_counter++ % 3;
     if (want_records) {
-        rlb_status st = ensure_episode_scratch(e, pipelined ? 2 * chunk : chunk, 3 * total);
+        rlb_status st = ensure_episode_scratch(e, pipelined ? 2 * chunk : chunk, 3 * total * sums_per_ep);
         if (st != RLB_OK) return st;
         if (pipelined) { st = ensure_copy_pipeline(e); if (st != RLB_OK) return st; e->last_pipeline_chunk = chunk; }
     }
     unsigned long long* const d_totals = e->d_totals + 8 * slot;
-    double* const d_sums_call = e->d_sums + (want_records ? slot * total * 4 : 0);
+    double* const d_sums_call = e->d_sums + (want_records ? slot * total * sums_per_ep : 0);
     rlb_engine::Pending pd;
     pd.mode = mode; pd.out = out; pd.eval_steps_out = eval_steps_out; pd.pipelined = pipelined;
     pd.host_records = host_rec;
@@ -610,7 +650,7 @@ rlb_status enqueue_range(rlb_engine* e, int mode, uint64_t begin, uint64_t end, 
         CK(cudaEventRecord(ev1, e->stream));
         const uint64_t n_ep = c1 - c0;
         if (sums_dst) {   // reads the records on the main stream, before that scratch is written again
-            rlb_status st = reduce_episodes(e, n_ep, scratch, d_sums_call + (c0 - begin) * 4);
+            rlb_status st = reduce_episodes(e, n_ep, scratch, d_sums_call + (c0 - begin) * sums_per_ep);
             if (st != RLB_OK) return st;
         }
         if (pipelined) {
@@ -627,16 +667,16 @@ rlb_status enqueue_range(rlb_engine* e, int mode, uint64_t begin, uint64_t end, 
     if (pipelined) {
         // kernels and reductions are in the main stream's queue; every device->host copy of this call goes to the copy stream
         const bool sums_on_device = sums_dst && is_device_ptr(sums_dst);   // e.g. about to be gathered on the caller's stream: stays in stream order
-        if (sums_on_device && total) CK(cudaMemcpyAsync(sums_dst, d_sums_call, total * 4 * sizeof(double), cudaMemcpyDeviceToDevice, e->stream));
+        if (sums_on_device && total) CK(cudaMemcpyAsync(sums_dst, d_sums_call, total * sums_per_ep * sizeof(double), cudaMemcpyDeviceToDevice, e->stream));
         CK(cudaEventRecord(pd.done, e->stream));
         CK(cudaStreamWaitEvent(e->copy_stream, pd.done, 0));
-        if (sums_dst && !sums_on_device && total) CK(cudaMemcpyAsync(sums_dst, d_sums_call, total * 4 * sizeof(double), cudaMemcpyDeviceToHost, e->copy_stream));
+        if (sums_dst && !sums_on_device && total) CK(cudaMemcpyAsync(sums_dst, d_sums_call, total * sums_per_ep * sizeof(double), cudaMemcpyDeviceToHost, e->copy_stream));
         CK(cudaMemcpyAsync(pd.h_totals, d_totals, 8 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, e->copy_stream));
         pd.copies_done = take_event(e);
         if (!pd.copies_done) { set_error("cudaEventCreate failed"); return RLB_ERR_CUDA; }
         CK(cudaEventRecord(pd.copies_done, e->copy_stream));
     } else {
-        if (sums_dst && total) CK(copy_async(e, sums_dst, d_sums_call, total * 4 * sizeof(double)));
+        if (sums_dst && total) CK(copy_async(e, sums_dst, d_sums_call, total * sums_per_ep * sizeof(double)));
         CK(cudaMemcpyAsync(pd.h_totals, d_totals, 8 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, e->stream));
         CK(cudaEventRecord(pd.done, e->stream));
     }
@@ -774,7 +814,8 @@ void rlb_engine_destroy(rlb_engine* e) {
     if (e->h_step_stage) cudaFreeHost(e->h_step_stage);
     void* bufs[] = {e->d_q, e->d_counts, e->d_etr, e->d_etr_il, e->d_vis, e->d_nvis, e->d_rng_n, e->d_eps, e->d_ucb_t, e->d_flag, e->d_env,
                     e->d_trans, e->d_thr, e->d_thr_state, e->d_totals, e->d_flagword, e->d_episodes, e->d_sums,
-                    e->d_model_ent, e->d_model_bits, e->d_model_len};
+                    e->d_model_ent, e->d_model_bits, e->d_model_len, e->d_hp_sets, e->d_hp_group, e->d_hp_order, e->d_hp_offsets,
+                    e->d_hp_q0, e->d_hp_eps0};
     for (void* b : bufs) if (b) cudaFree(b);
     for (void* b : e->d_stage) if (b) cudaFree(b);
     if (e->ev0) cudaEventDestroy(e->ev0);
@@ -811,6 +852,68 @@ rlb_status rlb_engine_dims(const rlb_engine* e, uint32_t* n_states, uint32_t* n_
     return RLB_OK;
 }
 uint32_t rlb_engine_store_kind(const rlb_engine* e) { return e ? (uint32_t)e->store : 0u; }
+
+rlb_status rlb_engine_set_hparams(rlb_engine* e, const rlb_hparams* sets, uint32_t n_sets, const uint32_t* group) {
+    if (!e) { set_error("engine is NULL"); return RLB_ERR_INVALID_ARG; }
+    if (n_sets == 0 && (sets || group)) { set_error("n_sets == 0 with a non-NULL sets or group"); return RLB_ERR_INVALID_ARG; }
+    if (n_sets > 0 && (!sets || !group)) { set_error("n_sets > 0 needs both sets and group"); return RLB_ERR_INVALID_ARG; }
+    if (n_sets > RLB_MAX_HPARAM_SETS) { set_error("n_sets = %u exceeds %d", n_sets, RLB_MAX_HPARAM_SETS); return RLB_ERR_INVALID_ARG; }
+    ENTER(e);
+    const uint64_t N = e->cfg.n_agents;
+    std::vector<rlb_hparams> h_sets(n_sets);
+    std::vector<uint32_t> h_group(n_sets ? N : 0);
+    if (n_sets) {
+        CK(cudaMemcpy(h_sets.data(), sets, (size_t)n_sets * sizeof(rlb_hparams), is_device_ptr(sets) ? cudaMemcpyDeviceToHost : cudaMemcpyHostToHost));
+        CK(cudaMemcpy(h_group.data(), group, N * sizeof(uint32_t), is_device_ptr(group) ? cudaMemcpyDeviceToHost : cudaMemcpyHostToHost));
+        for (uint64_t i = 0; i < N; ++i)
+            if (h_group[i] >= n_sets) { set_error("group[%llu] = %u >= n_sets = %u", (unsigned long long)i, h_group[i], n_sets); return RLB_ERR_INVALID_ARG; }
+        if (e->cfg.planning_steps) { set_error("per-agent hyper-parameter sets together with a Dyna model are not supported"); return RLB_ERR_UNSUPPORTED; }
+    }
+    // release the old sets (the kernels that read them have completed: ENTER waited for pending calls, and the stream
+    // is drained before the buffers go)
+    CK(cudaStreamSynchronize(e->stream));
+    void* old[] = {e->d_hp_sets, e->d_hp_group, e->d_hp_order, e->d_hp_offsets, e->d_hp_q0, e->d_hp_eps0};
+    for (void* b : old) if (b) cudaFree(b);
+    e->d_hp_sets = nullptr; e->d_hp_group = nullptr; e->d_hp_order = nullptr; e->d_hp_offsets = nullptr;
+    e->d_hp_q0 = nullptr; e->d_hp_eps0 = nullptr;
+    e->hp_n = 0;
+    if (n_sets) {
+        // the grouped reduction's read order: agents by set, ascending local index within a set (a stable counting sort)
+        std::vector<uint32_t> offsets(n_sets + 1, 0), order(N);
+        for (uint64_t i = 0; i < N; ++i) offsets[h_group[i] + 1] += 1;
+        for (uint32_t g = 0; g < n_sets; ++g) offsets[g + 1] += offsets[g];
+        std::vector<uint32_t> next(offsets.begin(), offsets.end() - 1);
+        for (uint64_t i = 0; i < N; ++i) order[next[h_group[i]]++] = (uint32_t)i;
+        // the fills' values, narrowed on the host exactly as the engine-wide fills narrow rlb_config's
+        std::vector<double> eps0(n_sets), q0d(n_sets);
+        std::vector<float> q0f(n_sets);
+        for (uint32_t g = 0; g < n_sets; ++g) { eps0[g] = h_sets[g].initial_epsilon; q0d[g] = h_sets[g].default_value; q0f[g] = (float)h_sets[g].default_value; }
+        CK(cudaMalloc(&e->d_hp_sets, (size_t)n_sets * sizeof(rlb_hparams)));
+        CK(cudaMalloc(&e->d_hp_group, N * sizeof(uint32_t)));
+        CK(cudaMalloc(&e->d_hp_order, N * sizeof(uint32_t)));
+        CK(cudaMalloc(&e->d_hp_offsets, (size_t)(n_sets + 1) * sizeof(uint32_t)));
+        CK(cudaMalloc(&e->d_hp_q0, (size_t)n_sets * e->real_size));
+        CK(cudaMalloc(&e->d_hp_eps0, (size_t)n_sets * sizeof(double)));
+        CK(cudaMemcpyAsync(e->d_hp_sets, h_sets.data(), (size_t)n_sets * sizeof(rlb_hparams), cudaMemcpyHostToDevice, e->stream));
+        CK(cudaMemcpyAsync(e->d_hp_group, h_group.data(), N * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
+        CK(cudaMemcpyAsync(e->d_hp_order, order.data(), N * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
+        CK(cudaMemcpyAsync(e->d_hp_offsets, offsets.data(), (size_t)(n_sets + 1) * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
+        if (e->cfg.real_kind == RLB_REAL_F32) CK(cudaMemcpyAsync(e->d_hp_q0, q0f.data(), (size_t)n_sets * 4, cudaMemcpyHostToDevice, e->stream));
+        else CK(cudaMemcpyAsync(e->d_hp_q0, q0d.data(), (size_t)n_sets * 8, cudaMemcpyHostToDevice, e->stream));
+        CK(cudaMemcpyAsync(e->d_hp_eps0, eps0.data(), (size_t)n_sets * sizeof(double), cudaMemcpyHostToDevice, e->stream));
+        e->hp_n = n_sets;
+    }
+    // the constructors again, with each agent's own values: fresh tables, policy_flag = true, an empty trace, a fresh
+    // selector (as rlb_agent_set_kind); the env and the RNG stream carry on
+    CK(fill_q_default(e));
+    CK(fill<uint8_t>(e, e->d_flag, N, (uint8_t)1));
+    CK(cudaMemsetAsync(e->d_nvis, 0, N * sizeof(uint32_t), e->stream));
+    rlb_status st = install_selector(e, e->cfg.selector_kind);
+    if (st != RLB_OK) return st;
+    CK(cudaStreamSynchronize(e->stream));
+    return RLB_OK;
+}
+uint32_t rlb_engine_hparam_sets(const rlb_engine* e) { return e ? e->hp_n : 0u; }
 
 // ------------------------------------------------------------------------------- Env
 rlb_status rlb_env_reset(rlb_engine* e, uint32_t* obs_out) {
@@ -975,7 +1078,7 @@ rlb_status rlb_selector_reset(rlb_engine* e) {
     ENTER(e);
     const uint64_t N = e->cfg.n_agents;
     if (e->cfg.selector_kind == RLB_SEL_EPS_GREEDY) {
-        CK(fill<double>(e, e->d_eps, N, e->cfg.initial_epsilon));               // uniform_epsilon_greed.rs:78-80
+        CK(fill_eps_initial(e));                                                // uniform_epsilon_greed.rs:78-80
     } else {
         CK(cudaMemsetAsync(e->d_counts, 0, e->counts_bytes, e->stream));        // upper_confidence_bound.rs:65-68
         CK(fill<uint64_t>(e, e->d_ucb_t, N, 1ull));
@@ -1003,6 +1106,10 @@ rlb_status rlb_agent_set_model(rlb_engine* e, uint32_t planning_steps) {
     ENTER(e);
     if (planning_steps && e->cfg.store_kind != 0 && e->cfg.store_kind != STORE_GLOBAL) {
         set_error("a Dyna model (planning_steps > 0) needs the HBM store");
+        return RLB_ERR_UNSUPPORTED;
+    }
+    if (planning_steps && e->hp_n) {
+        set_error("a Dyna model together with per-agent hyper-parameter sets is not supported");
         return RLB_ERR_UNSUPPORTED;
     }
     rlb_status st = attach_model(e, planning_steps);
@@ -1216,7 +1323,9 @@ rlb_status rlb_selector_get_exploration_probs(rlb_engine* e, const uint32_t* obs
 rlb_status rlb_selector_update(rlb_engine* e) {
     if (!e) { set_error("engine is NULL"); return RLB_ERR_INVALID_ARG; }
     ENTER(e);
-    if (e->cfg.selector_kind == RLB_SEL_EPS_GREEDY) {
+    if (e->cfg.selector_kind == RLB_SEL_EPS_GREEDY && e->hp_n) {   // each agent with its own k and floor
+        CK(launch_eps_decay_grouped(e->d_eps, e->cfg.n_agents, e->cfg.decay_kind, e->d_hp_sets, e->d_hp_group, e->stream));
+    } else if (e->cfg.selector_kind == RLB_SEL_EPS_GREEDY) {
         const uint64_t N = e->cfg.n_agents;
         k_eps_decay<<<(unsigned)((N + 255) / 256), 256, 0, e->stream>>>(e->d_eps, N, e->cfg.decay_kind, e->cfg.epsilon_decay, e->cfg.final_epsilon);
         CK(cudaGetLastError());

@@ -33,6 +33,7 @@ struct StepArgs {   // device pointers for the step-level kernels
     uint8_t* not_ready_out = nullptr;
     uint32_t* any_not_ready = nullptr;   // the engine's flag word (FLAG_* bits, rlb_step_kernels.cuh)
     int which = 0;
+    HpParams sets{};                     // launch_step<ENV, true>: every agent's hyper-parameter set
 };
 
 enum StepOp {
@@ -40,12 +41,25 @@ enum StepOp {
     OP_SELECTOR_GET_ACTION, OP_SELECTOR_PROBS, OP_AGENT_STEP
 };
 
-template <int ENV> cudaError_t launch_run(const Variant& v, const DevParams& p, int store, cudaStream_t stream);
+// HP = true: the agents run with their own hyper-parameter sets `h` (k_run_hp); instantiated in rlb_inst_<env>_hp.cu
+template <int ENV, bool HP = false> cudaError_t launch_run(const Variant& v, const DevParams& p, int store, cudaStream_t stream,
+                                                          const HpParams& h = HpParams{});
 // the same with the Dyna model attached (InternalModelAgent): HBM store only; instantiated in rlb_inst_<env>_model.cu
 template <int ENV> cudaError_t launch_run_model(const Variant& v, const DevParams& p, cudaStream_t stream);
 // bytes of dynamic shared memory one 1-warp CTA of the shared-memory / hybrid store needs (0: env not compiled for it)
 template <int ENV> size_t smem_store_bytes(const Variant& v, int store, uint32_t rows, uint32_t S, uint32_t vmax);   // rows: table rows kept on chip
-template <int ENV> cudaError_t launch_step(StepOp op, const Variant& v, const DevParams& p, const StepArgs& a, cudaStream_t stream);
-template <int ENV> cudaError_t run_kernel_attributes(const Variant& v, int store, cudaFuncAttributes* attr);
+template <int ENV, bool HP = false> cudaError_t launch_step(StepOp op, const Variant& v, const DevParams& p, const StepArgs& a, cudaStream_t stream);
+template <int ENV, bool HP = false> cudaError_t run_kernel_attributes(const Variant& v, int store, cudaFuncAttributes* attr);
+
+// ---- per-agent hyper-parameter sets (rlb_hparams.cu) ----
+// ptr[i * per_agent + k] = values[group[i]] for every agent i < n_agents and k < per_agent; elem_size 1, 4 or 8 bytes
+cudaError_t launch_fill_grouped(void* ptr, size_t elem_size, uint64_t per_agent, uint64_t n_agents, const void* values,
+                                const uint32_t* group, cudaStream_t stream);
+// ActionSelection::update of every eps-greedy agent with its own set's decay k and floor
+cudaError_t launch_eps_decay_grouped(double* eps, uint64_t n_agents, int kind, const rlb_hparams* sets, const uint32_t* group,
+                                     cudaStream_t stream);
+// out[e][g][4] for e < n_ep, g < n_sets: the k_episode_sums reduction over the agents order[offsets[g] .. offsets[g + 1])
+cudaError_t launch_episode_sums_grouped(int real_kind, const void* records, uint64_t n_agents, const uint32_t* order,
+                                        const uint32_t* offsets, uint32_t n_sets, uint64_t n_ep, double* out, cudaStream_t stream);
 
 }   // namespace rlb

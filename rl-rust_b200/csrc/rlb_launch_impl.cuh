@@ -69,18 +69,31 @@ size_t smem_store_bytes(const Variant& v, int store, uint32_t rows, uint32_t S, 
     }
 }
 
-template <int ENV>
-cudaError_t launch_run(const Variant& v, const DevParams& p, int store, cudaStream_t stream) {
+// k_run, or k_run_hp (one more parameter: the sets) when the agents hold their own hyper-parameter sets
+template <bool HP, int ENV, typename R, int P, int SL, bool T, int STORE>
+struct RunKernel {
+    static auto ptr() {
+        if constexpr (HP) return k_run_hp<ENV, R, P, SL, T, STORE>;
+        else return k_run<ENV, R, P, SL, T, STORE>;
+    }
+    static void launch(unsigned grid, unsigned block, size_t smem, cudaStream_t stream, const DevParams& p, const HpParams& h) {
+        if constexpr (HP) k_run_hp<ENV, R, P, SL, T, STORE><<<grid, block, smem, stream>>>(p, h);
+        else k_run<ENV, R, P, SL, T, STORE><<<grid, block, smem, stream>>>(p);
+    }
+};
+
+template <int ENV, bool HP>
+cudaError_t launch_run(const Variant& v, const DevParams& p, int store, cudaStream_t stream, const HpParams& h) {
     if (store == STORE_HYBRID) {
         if constexpr (SmemCapable<ENV>::value) {
             const unsigned grid = (unsigned)((p.n_agents + 31) / 32);   // one warp per CTA: 32 agents, one per lane
             const size_t smem = smem_store_bytes<ENV>(v, store, p.n_live, p.S, p.vmax);
 #define RLB_CALL(R, P, SL, T)                                                                                          \
     {                                                                                                                  \
-        auto kern = k_run<ENV, R, P, SL, T, STORE_HYBRID>;                                                             \
+        auto kern = RunKernel<HP, ENV, R, P, SL, T, STORE_HYBRID>::ptr();                                                          \
         cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);          \
         if (err != cudaSuccess) return err;                                                                            \
-        kern<<<grid, 32, smem, stream>>>(p);                                                                           \
+        RunKernel<HP, ENV, R, P, SL, T, STORE_HYBRID>::launch(grid, 32, smem, stream, p, h);                              \
     }
             RLB_VARIANT_SWITCH(v, RLB_CALL)
 #undef RLB_CALL
@@ -95,10 +108,10 @@ cudaError_t launch_run(const Variant& v, const DevParams& p, int store, cudaStre
             const size_t smem = smem_store_bytes<ENV>(v, store, p.S, p.S, p.vmax);
 #define RLB_CALL(R, P, SL, T)                                                                                          \
     {                                                                                                                  \
-        auto kern = k_run<ENV, R, P, SL, T, STORE_SMEM>;                                                               \
+        auto kern = RunKernel<HP, ENV, R, P, SL, T, STORE_SMEM>::ptr();                                                          \
         cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);          \
         if (err != cudaSuccess) return err;                                                                            \
-        kern<<<grid, 32, smem, stream>>>(p);                                                                           \
+        RunKernel<HP, ENV, R, P, SL, T, STORE_SMEM>::launch(grid, 32, smem, stream, p, h);                              \
     }
             RLB_VARIANT_SWITCH(v, RLB_CALL)
 #undef RLB_CALL
@@ -116,10 +129,10 @@ cudaError_t launch_run(const Variant& v, const DevParams& p, int store, cudaStre
         const size_t hist = ((smem + 15) & ~(size_t)15) + (size_t)p.lz_cap * kLazyBlock * (v.real == RLB_REAL_F32 ? 4 : 8);
 #define RLB_CALL(R, P, SL, T)                                                                                          \
     if constexpr (T) {                                                                                                 \
-        auto kern = k_run<ENV, R, P, SL, true, STORE_LAZY>;                                                            \
+        auto kern = RunKernel<HP, ENV, R, P, SL, true, STORE_LAZY>::ptr();                                             \
         cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hist);          \
         if (err != cudaSuccess) return err;                                                                            \
-        kern<<<lz_grid, kLazyBlock, hist, stream>>>(p);                                                                \
+        RunKernel<HP, ENV, R, P, SL, true, STORE_LAZY>::launch(lz_grid, kLazyBlock, hist, stream, p, h);               \
     }
         RLB_VARIANT_SWITCH(v, RLB_CALL)
 #undef RLB_CALL
@@ -127,9 +140,8 @@ cudaError_t launch_run(const Variant& v, const DevParams& p, int store, cudaStre
     }
 #define RLB_CALL(R, P, SL, T)                                                   \
     {                                                                           \
-        auto kern = k_run<ENV, R, P, SL, T, STORE_GLOBAL>;                      \
-        prefer_l1(kern, smem);                                                  \
-        kern<<<grid, kBlock, smem, stream>>>(p);                                \
+        prefer_l1(RunKernel<HP, ENV, R, P, SL, T, STORE_GLOBAL>::ptr(), smem);                                  \
+        RunKernel<HP, ENV, R, P, SL, T, STORE_GLOBAL>::launch(grid, kBlock, smem, stream, p, h);                \
     }
     RLB_VARIANT_SWITCH(v, RLB_CALL)
 #undef RLB_CALL
@@ -146,11 +158,11 @@ cudaError_t launch_run_model(const Variant& v, const DevParams& p, cudaStream_t 
     return cudaGetLastError();
 }
 
-template <int ENV>
+template <int ENV, bool HP>
 cudaError_t run_kernel_attributes(const Variant& v, int store, cudaFuncAttributes* attr) {
     if (store == STORE_HYBRID) {
         if constexpr (SmemCapable<ENV>::value) {
-#define RLB_CALL(R, P, SL, T) return cudaFuncGetAttributes(attr, k_run<ENV, R, P, SL, T, STORE_HYBRID>)
+#define RLB_CALL(R, P, SL, T) return cudaFuncGetAttributes(attr, RunKernel<HP, ENV, R, P, SL, T, STORE_HYBRID>::ptr())
             RLB_VARIANT_SWITCH(v, RLB_CALL)
 #undef RLB_CALL
         }
@@ -158,25 +170,33 @@ cudaError_t run_kernel_attributes(const Variant& v, int store, cudaFuncAttribute
     }
     if (store == STORE_SMEM) {
         if constexpr (SmemCapable<ENV>::value) {
-#define RLB_CALL(R, P, SL, T) return cudaFuncGetAttributes(attr, k_run<ENV, R, P, SL, T, STORE_SMEM>)
+#define RLB_CALL(R, P, SL, T) return cudaFuncGetAttributes(attr, RunKernel<HP, ENV, R, P, SL, T, STORE_SMEM>::ptr())
             RLB_VARIANT_SWITCH(v, RLB_CALL)
 #undef RLB_CALL
         }
         return cudaErrorInvalidValue;
     }
     if (store == STORE_LAZY) {
-#define RLB_CALL(R, P, SL, T) if constexpr (T) return cudaFuncGetAttributes(attr, k_run<ENV, R, P, SL, true, STORE_LAZY>)
+#define RLB_CALL(R, P, SL, T) if constexpr (T) return cudaFuncGetAttributes(attr, RunKernel<HP, ENV, R, P, SL, true, STORE_LAZY>::ptr())
         RLB_VARIANT_SWITCH(v, RLB_CALL)
 #undef RLB_CALL
         return cudaErrorInvalidValue;
     }
-#define RLB_CALL(R, P, SL, T) return cudaFuncGetAttributes(attr, k_run<ENV, R, P, SL, T, STORE_GLOBAL>)
+#define RLB_CALL(R, P, SL, T) return cudaFuncGetAttributes(attr, RunKernel<HP, ENV, R, P, SL, T, STORE_GLOBAL>::ptr())
     RLB_VARIANT_SWITCH(v, RLB_CALL)
 #undef RLB_CALL
     return cudaSuccess;
 }
 
-template <int ENV>
+// the step-level kernels that read hyper-parameters come in a plain and an _hp form (rlb_step_agent_kernels.inc); the
+// _hp form takes the sets as its last parameter
+#define RLB_STEP_LAUNCH(name, R, P, S, T, SMEM, ...)                                                               \
+    do {                                                                                                           \
+        if constexpr (HP) name##_hp<ENV, R, P, S, T><<<grid, kBlock, SMEM, stream>>>(__VA_ARGS__, a.sets);         \
+        else name<ENV, R, P, S, T><<<grid, kBlock, SMEM, stream>>>(__VA_ARGS__);                                   \
+    } while (0)
+
+template <int ENV, bool HP>
 cudaError_t launch_step(StepOp op, const Variant& v, const DevParams& p, const StepArgs& a, cudaStream_t stream) {
     const unsigned grid = grid_for(p.n_agents);
     const size_t smem = EnvTab<ENV>::smem_bytes(p.S);
@@ -187,14 +207,14 @@ cudaError_t launch_step(StepOp op, const Variant& v, const DevParams& p, const S
             k_env_step<ENV><<<grid, kBlock, smem, stream>>>(p, a.action, a.u32_out, a.reward_out, a.term_out, a.not_ready_out, a.any_not_ready);
             break;
         case OP_GET_ACTION: {
-#define RLB_CALL(R, P, S, T) k_get_action<ENV, R, P, S, T><<<grid, kBlock, 0, stream>>>(p, a.obs, a.u32_out, a.any_not_ready)
+#define RLB_CALL(R, P, S, T) RLB_STEP_LAUNCH(k_get_action, R, P, S, T, 0, p, a.obs, a.u32_out, a.any_not_ready)
             RLB_VARIANT_SWITCH(v, RLB_CALL)
 #undef RLB_CALL
             break;
         }
         case OP_UPDATE: {
 #define RLB_CALL(R, P, S, T) \
-    k_update<ENV, R, P, S, T><<<grid, kBlock, 0, stream>>>(p, a.obs, a.action, a.reward, a.term, a.obs2, a.action2, (R*)a.real_out, a.any_not_ready)
+    RLB_STEP_LAUNCH(k_update, R, P, S, T, 0, p, a.obs, a.action, a.reward, a.term, a.obs2, a.action2, (R*)a.real_out, a.any_not_ready)
             RLB_VARIANT_SWITCH(v, RLB_CALL)
 #undef RLB_CALL
             break;
@@ -206,26 +226,26 @@ cudaError_t launch_step(StepOp op, const Variant& v, const DevParams& p, const S
             break;
         }
         case OP_POLICY_UPDATE: {
-#define RLB_CALL(R, P, S, T) k_policy_update<ENV, R, P, S, T><<<grid, kBlock, 0, stream>>>(p, a.obs, a.action, (const R*)a.td_in, a.any_not_ready)
+#define RLB_CALL(R, P, S, T) RLB_STEP_LAUNCH(k_policy_update, R, P, S, T, 0, p, a.obs, a.action, (const R*)a.td_in, a.any_not_ready)
             RLB_VARIANT_SWITCH(v, RLB_CALL)
 #undef RLB_CALL
             break;
         }
         case OP_SELECTOR_GET_ACTION: {
-#define RLB_CALL(R, P, S, T) k_selector_get_action<ENV, R, P, S, T><<<grid, kBlock, 0, stream>>>(p, a.obs, (const R*)a.values, a.u32_out, a.any_not_ready)
+#define RLB_CALL(R, P, S, T) RLB_STEP_LAUNCH(k_selector_get_action, R, P, S, T, 0, p, a.obs, (const R*)a.values, a.u32_out, a.any_not_ready)
             RLB_VARIANT_SWITCH(v, RLB_CALL)
 #undef RLB_CALL
             break;
         }
         case OP_SELECTOR_PROBS: {
-#define RLB_CALL(R, P, S, T) k_selector_probs<ENV, R, P, S, T><<<grid, kBlock, 0, stream>>>(p, a.obs, (const R*)a.values, (R*)a.real_out, a.any_not_ready)
+#define RLB_CALL(R, P, S, T) RLB_STEP_LAUNCH(k_selector_probs, R, P, S, T, 0, p, a.obs, (const R*)a.values, (R*)a.real_out, a.any_not_ready)
             RLB_VARIANT_SWITCH(v, RLB_CALL)
 #undef RLB_CALL
             break;
         }
         case OP_AGENT_STEP: {
 #define RLB_CALL(R, P, S, T) \
-    k_agent_step<ENV, R, P, S, T><<<grid, kBlock, smem, stream>>>(p, a.kind_out, a.u32_out, a.u32_out2, a.reward_out, a.term_out, (R*)a.real_out)
+    RLB_STEP_LAUNCH(k_agent_step, R, P, S, T, smem, p, a.kind_out, a.u32_out, a.u32_out2, a.reward_out, a.term_out, (R*)a.real_out)
             RLB_VARIANT_SWITCH(v, RLB_CALL)
 #undef RLB_CALL
             break;
@@ -235,10 +255,16 @@ cudaError_t launch_step(StepOp op, const Variant& v, const DevParams& p, const S
 }
 
 #define RLB_INSTANTIATE_ENV(ENV)                                                                         \
-    template cudaError_t launch_run<ENV>(const Variant&, const DevParams&, int, cudaStream_t);           \
+    template cudaError_t launch_run<ENV, false>(const Variant&, const DevParams&, int, cudaStream_t, const HpParams&); \
     template size_t smem_store_bytes<ENV>(const Variant&, int, uint32_t, uint32_t, uint32_t);                           \
-    template cudaError_t launch_step<ENV>(StepOp, const Variant&, const DevParams&, const StepArgs&, cudaStream_t); \
-    template cudaError_t run_kernel_attributes<ENV>(const Variant&, int, cudaFuncAttributes*);
+    template cudaError_t launch_step<ENV, false>(StepOp, const Variant&, const DevParams&, const StepArgs&, cudaStream_t); \
+    template cudaError_t run_kernel_attributes<ENV, false>(const Variant&, int, cudaFuncAttributes*);
+
+// the same entry points with per-agent hyper-parameter sets (k_run_hp and the _hp step kernels); rlb_inst_<env>_hp.cu
+#define RLB_INSTANTIATE_ENV_HP(ENV)                                                                      \
+    template cudaError_t launch_run<ENV, true>(const Variant&, const DevParams&, int, cudaStream_t, const HpParams&);  \
+    template cudaError_t launch_step<ENV, true>(StepOp, const Variant&, const DevParams&, const StepArgs&, cudaStream_t); \
+    template cudaError_t run_kernel_attributes<ENV, true>(const Variant&, int, cudaFuncAttributes*);
 
 #define RLB_INSTANTIATE_ENV_MODEL(ENV) template cudaError_t launch_run_model<ENV>(const Variant&, const DevParams&, cudaStream_t);
 

@@ -95,112 +95,6 @@ __global__ void __launch_bounds__(128) k_env_step(const DevParams p, const uint3
     term_out[i] = term ? 1 : 0;
 }
 
-// Agent::get_action = selector.get_action(obs, policy.predict(obs))
-template <int ENV, typename Real, int POLICY, int SEL, bool TRACE>
-__global__ void __launch_bounds__(128) k_get_action(const DevParams p, const uint32_t* obs, uint32_t* action_out, uint32_t* flags) {
-    using Core = AgentCore<ENV, Real, POLICY, SEL, TRACE>;
-    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= p.n_agents) return;
-    if (obs[i] >= p.S) { atomicOr(flags, FLAG_BAD_ARG); return; }
-    Core core;
-    core.load(p, i);
-    Real pred[Core::A], vals[Core::A];
-    core.rows(obs[i], pred, vals);
-    action_out[i] = core.select(obs[i], pred, p);
-    core.save(p, i);
-}
-
-// Agent::update
-template <int ENV, typename Real, int POLICY, int SEL, bool TRACE>
-__global__ void __launch_bounds__(128) k_update(const DevParams p, const uint32_t* s, const uint32_t* a, const double* reward,
-                                                 const uint8_t* term, const uint32_t* s2, const uint32_t* a2, Real* td_out, uint32_t* flags) {
-    using Core = AgentCore<ENV, Real, POLICY, SEL, TRACE>;
-    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= p.n_agents) return;
-    if (s[i] >= p.S || s2[i] >= p.S || a[i] >= (uint32_t)Core::A || a2[i] >= (uint32_t)Core::A) { atomicOr(flags, FLAG_BAD_ARG); return; }
-    Core core;
-    core.load(p, i);
-    if constexpr (TRACE) {
-        // The engine sizes the trace for episodes of its own env (vmax rows); foreign transitions could ask for more.
-        // A terminal cell as curr_obs has no row in the on-chip stores of the fused kernel.
-        bool seen = false;
-        for (uint32_t j = 0; j < core.nvis; ++j) seen = seen || core.st.get_vis(j) == core.st.key(s[i]);
-        if (!seen && core.nvis >= p.vmax) { atomicOr(flags, FLAG_TRACE_FULL); return; }
-        if (p.S <= 64u && p.n_live < p.S && p.row_lut[s[i]] == 0xFFu) { atomicOr(flags, FLAG_DEAD_STATE); return; }
-    }
-    Real pred[Core::A], vals[Core::A];
-    core.rows(s2[i], pred, vals);
-    Real td = core.update(s[i], a[i], (Real)reward[i], term[i] != 0, s2[i], a2[i], vals, p);
-    if (p.planning_steps) {   // InternalModelAgent::update (internal_model_agent.rs:62-77)
-        RandomModelDev model;
-        model.load(p, i);
-        learn_and_plan(core, model, s[i], a[i], (Real)reward[i], s2[i], p);
-        model.save(p, i);
-    }
-    if (td_out) td_out[i] = td;
-    core.save(p, i);
-}
-
-// One iteration of the loop at agent.rs:83-106 per agent — k_run's per-lane state machine, one transition per launch:
-// an agent whose env is not ready (episode over or never begun) resets and picks its first action (agent.rs:83-84),
-// any other steps the env with the action it holds, picks the next action (also on a terminal observation, :89) and
-// updates (:90-97, with the Dyna replays when a model is attached).  curr_obs / curr_action live in DevParams::cur_*.
-template <int ENV, typename Real, int POLICY, int SEL, bool TRACE>
-__global__ void __launch_bounds__(128) k_agent_step(const DevParams p, uint8_t* kind_out, uint32_t* obs_out, uint32_t* action_out,
-                                                     double* reward_out, uint8_t* term_out, Real* td_out) {
-    using Core = AgentCore<ENV, Real, POLICY, SEL, TRACE>;
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    EnvTab<ENV> tab;
-    tab.load(p, smem_raw);
-    __syncthreads();
-    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= p.n_agents) return;
-    Core core;
-    core.load(p, i);
-    EnvState es = p.env[i];
-    EnvRegs<ENV> env;
-    env.from_state(es);
-    const bool fresh = !es.ready;
-    const uint32_t s = p.cur_obs[i], a = p.cur_action[i];
-    uint32_t o;
-    Real r = (Real)0;
-    bool term = false;
-    if (fresh) {
-        o = env.reset(core.rng, tab, p);
-        env.to_state(es, o);
-        es.pos = o;
-        es.ready = 1;
-    } else {
-        env.template step<Real>(es.pos, a, core.rng, tab, p, o, r, term);
-        const bool truncated = (ENV != RLB_ENV_BLACKJACK) && es.curr_step >= p.max_steps;   // reports obs 0, does not move (taxi.rs:148-151)
-        env.to_state(es, truncated ? es.pos : o);
-        if (term) es.ready = 0;
-    }
-    Real pred[Core::A], vals[Core::A];
-    core.rows(o, pred, vals);
-    const uint32_t a2 = core.select(o, pred, p);
-    Real td = (Real)0;
-    if (!fresh) {
-        td = core.update(s, a, r, term, o, a2, vals, p);
-        if (p.planning_steps) {
-            RandomModelDev model;
-            model.load(p, i);
-            learn_and_plan(core, model, s, a, r, o, p);
-            model.save(p, i);
-        }
-    }
-    p.env[i] = es;
-    p.cur_obs[i] = o;
-    p.cur_action[i] = a2;
-    core.save(p, i);
-    if (kind_out) kind_out[i] = fresh ? 0 : 1;
-    if (obs_out) obs_out[i] = o;
-    if (action_out) action_out[i] = a2;
-    if (reward_out) reward_out[i] = (double)r;
-    if (term_out) term_out[i] = term ? 1 : 0;
-    if (td_out) td_out[i] = td;
-}
-
 // Policy::predict (which = 0) / Policy::get_values (which = 1)
 template <int ENV, typename Real, int POLICY, int SEL, bool TRACE>
 __global__ void __launch_bounds__(128) k_policy_rows(const DevParams p, const uint32_t* obs, Real* out, int which, uint32_t* flags) {
@@ -216,52 +110,12 @@ __global__ void __launch_bounds__(128) k_policy_rows(const DevParams p, const ui
     for (int k = 0; k < Core::A; ++k) out[i * Core::A + k] = which == 0 ? pred[k] : vals[k];
 }
 
-// Policy::update: (Basic: Q | Double: beta if flag else alpha)[obs][action] += lr * td
-template <int ENV, typename Real, int POLICY, int SEL, bool TRACE>
-__global__ void __launch_bounds__(128) k_policy_update(const DevParams p, const uint32_t* obs, const uint32_t* action, const Real* td, uint32_t* flags) {
-    using Core = AgentCore<ENV, Real, POLICY, SEL, TRACE>;
-    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= p.n_agents) return;
-    if (obs[i] >= p.S || action[i] >= (uint32_t)Core::A) { atomicOr(flags, FLAG_BAD_ARG); return; }
-    Core core;
-    core.load(p, i);
-    const int write_tbl = (POLICY == RLB_POLICY_DOUBLE && core.flag) ? 1 : 0;
-    Real old = core.st.get_q(obs[i], write_tbl, action[i]);
-    core.st.set_q(obs[i], write_tbl, action[i], old + core.lr * td[i]);
-}
-
-// ActionSelection::get_action on caller-supplied values
-template <int ENV, typename Real, int POLICY, int SEL, bool TRACE>
-__global__ void __launch_bounds__(128) k_selector_get_action(const DevParams p, const uint32_t* obs, const Real* values, uint32_t* action_out, uint32_t* flags) {
-    using Core = AgentCore<ENV, Real, POLICY, SEL, TRACE>;
-    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= p.n_agents) return;
-    if (obs[i] >= p.S) { atomicOr(flags, FLAG_BAD_ARG); return; }
-    Core core;
-    core.load(p, i);
-    Real v[Core::A];
-#pragma unroll
-    for (int k = 0; k < Core::A; ++k) v[k] = values[i * Core::A + k];
-    action_out[i] = core.select(obs[i], v, p);
-    core.save(p, i);
-}
-
-// ActionSelection::get_exploration_probs on caller-supplied values
-template <int ENV, typename Real, int POLICY, int SEL, bool TRACE>
-__global__ void __launch_bounds__(128) k_selector_probs(const DevParams p, const uint32_t* obs, const Real* values, Real* probs_out, uint32_t* flags) {
-    using Core = AgentCore<ENV, Real, POLICY, SEL, TRACE>;
-    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= p.n_agents) return;
-    if (obs[i] >= p.S) { atomicOr(flags, FLAG_BAD_ARG); return; }
-    Core core;
-    core.load(p, i);
-    Real v[Core::A], pr[Core::A];
-#pragma unroll
-    for (int k = 0; k < Core::A; ++k) v[k] = values[i * Core::A + k];
-    core.probs(obs[i], v, pr, p);
-#pragma unroll
-    for (int k = 0; k < Core::A; ++k) probs_out[i * Core::A + k] = pr[k];
-}
+#define RLB_STEP_HP 0
+#include "rlb_step_agent_kernels.inc"
+#undef RLB_STEP_HP
+#define RLB_STEP_HP 1
+#include "rlb_step_agent_kernels.inc"
+#undef RLB_STEP_HP
 
 // Model::add_info (random_model.rs:37-41)
 static __global__ void k_model_add_info(const DevParams p, uint32_t A, const uint32_t* s, const uint32_t* a, const double* reward, const uint32_t* s2, uint32_t* flags) {

@@ -310,3 +310,132 @@ def main(argv=None):
         from . import charts
         charts.plot_experiment(res, plots)
     return res
+
+
+# ---- hyper-parameter sweeps: the bins' flags as grids, every grid point a group of agents of ONE engine ------------------
+SWEEP_FLAGS = ("learning_rate", "discount_factor", "lambda_factor", "initial_epsilon", "exploration_time", "final_epsilon",
+               "confidence_level")   # the bin flags that are agent constructor arguments (bin/taxi.rs:22-68, :78)
+AGENT_NAMES = {"onestep": abi.AGENT_ONE_STEP, "traces": abi.AGENT_TRACES}
+SELECTOR_NAMES = {"eps": abi.SEL_EPS_GREEDY, "ucb": abi.SEL_UCB}
+TARGET_KINDS = {"sarsa": abi.TARGET_SARSA, "qlearning": abi.TARGET_QLEARNING, "expected_sarsa": abi.TARGET_EXPECTED_SARSA}
+
+
+def expand_grid(grid):
+    """{flag: [values]} -> the cartesian product as a list of {flag: value}, the first flag varying slowest."""
+    import itertools
+    for k in grid:
+        if k not in SWEEP_FLAGS:
+            raise ValueError("%r cannot be swept; the agent constructor flags are %s" % (k, ", ".join(SWEEP_FLAGS)))
+    keys = list(grid)
+    return [dict(zip(keys, vals)) for vals in itertools.product(*(grid[k] for k in keys))]
+
+
+def point_hparams(flags, n_episodes):
+    """One grid point's rlb_hparams, the decay derived as run_experiment derives it (bin/taxi.rs:78)."""
+    return dict(learning_rate=flags["learning_rate"], discount_factor=flags["discount_factor"], lambda_factor=flags["lambda_factor"],
+                initial_epsilon=flags["initial_epsilon"], epsilon_decay=flags["initial_epsilon"] / (flags["exploration_time"] * n_episodes),
+                final_epsilon=flags["final_epsilon"], confidence_level=flags["confidence_level"], default_value=0.0)
+
+
+def run_sweep(env_name, grid, *, agent="onestep", selector="eps", target="qlearning", policy="basic", agents_per_point=1024,
+              seed=0x5EED0001, real="f64", device=0, verbose=True, **flags):
+    """One run of the bin (`train(n, n/10)` -> `evaluate(n)`, bin/taxi.rs:165-188) for every point of the cartesian grid
+    of `grid` ({flag: [values]}, flags otherwise as in run_experiment), all points at once: ONE engine, the points'
+    agents in contiguous groups of `agents_per_point`, each group constructed with its point's values
+    (rlb_engine_set_hparams); the grouped per-episode sums give every point its own curves.  Returns the bins' moving
+    averages of return and episode length per point, the evaluate mean return, and the points ranked by it."""
+    f = dict(DEFAULTS)
+    f.update(flags)
+    n = int(f["n_episodes"])
+    window = max(1, n // int(f["moving_average_window"]))
+    points = expand_grid(grid)
+    sets = []
+    for pt in points:
+        pf = dict(f)
+        pf.update(pt)
+        sets.append(point_hparams(pf, n))
+    if len(sets) > abi.MAX_HPARAM_SETS:
+        raise ValueError("%d grid points; an engine holds at most %d sets" % (len(sets), abi.MAX_HPARAM_SETS))
+    env = make_env(env_name, **f)
+    n_agents = len(points) * int(agents_per_point)
+    eng = abi.Engine(env.kind, n_agents=n_agents, policy=abi.POLICY_BASIC if policy == "basic" else abi.POLICY_DOUBLE,
+                     selector=SELECTOR_NAMES[selector], target=TARGET_KINDS[target], agent=AGENT_NAMES[agent],
+                     real=abi.REAL_F32 if real == "f32" else abi.REAL_F64, decay_kind=abi.DECAY_SUB, seed=seed, device=device,
+                     **sets[0], **env._cfg())
+    try:
+        eng.set_hparams(sets, np.repeat(np.arange(len(points), dtype=np.uint32), int(agents_per_point)))
+        t0 = time.perf_counter()
+        res = eng.train(n, max(1, n // 10))                                                          # [n, G, 4]
+        ev = eng.evaluate(n, sums=True)["sums"]                                                      # [n, G, 4]
+        dt = time.perf_counter() - t0
+    finally:
+        eng.close()
+    per = float(agents_per_point)
+    out_points = []
+    for g, pt in enumerate(points):
+        s_, e_ = res["sums"][:, g], ev[:, g]
+        out_points.append(dict(params=pt, hparams=sets[g],
+                               train_rewards=moving_average(window, s_[:, 1] / per),
+                               train_episodes_length=moving_average(window, s_[:, 0] / per),
+                               test_rewards=moving_average(window, e_[:, 1] / per),
+                               test_episodes_length=moving_average(window, e_[:, 0] / per),
+                               eval_mean_return=float(e_[:, 1].sum()) / (per * n)))
+    ranking = sorted(range(len(points)), key=lambda g: -out_points[g]["eval_mean_return"])
+    if verbose:
+        print("%d points x %d agents, %d episodes: %.2fs (%.3g train steps/s)" % (len(points), agents_per_point, n, dt,
+                                                                                  res["train_steps"] / dt if dt > 0 else 0.0))
+        for g in ranking[:10]:
+            print("  %-60s evaluate mean return %.4f" % (points[g], out_points[g]["eval_mean_return"]))
+    return dict(env=env_name, agent=agent, selector=selector, target=target, policy=policy, real=real, n_episodes=n,
+                agents_per_point=int(agents_per_point), grid={k: list(v) for k, v in grid.items()}, points=out_points,
+                ranking=ranking, seconds=dt, train_steps=int(res["train_steps"]))
+
+
+def parse_list(text):
+    return [float(x) for x in text.split(",") if x.strip()]
+
+
+def main_sweep(argv=None):
+    import argparse
+    ap = argparse.ArgumentParser(description="Hyper-parameter sweep of one RL-Rust bin run over the B200 engine: every point "
+                                             "of the grid is a group of agents of one engine")
+    ap.add_argument("env", choices=["blackjack", "frozen_lake", "cliffwalking", "taxi"])
+    ap.add_argument("--grid", action="append", default=[], metavar="FLAG=V1,V2,...",
+                    help="a bin flag and its values (repeatable; one of %s)" % ", ".join(SWEEP_FLAGS))
+    for name in SWEEP_FLAGS:
+        ap.add_argument("--" + name, default=None, metavar="V1,V2,...", help="values of this flag (a comma list: a grid axis)")
+    ap.add_argument("--n_episodes", "-n", type=int, default=DEFAULTS["n_episodes"])
+    for name in ("max_steps", "moving_average_window"):
+        ap.add_argument("--" + name, type=int, default=DEFAULTS[name])
+    ap.add_argument("--stochastic_env", action="store_true")
+    ap.add_argument("--map", default="4x4")
+    ap.add_argument("--agent", choices=sorted(AGENT_NAMES), default="onestep")
+    ap.add_argument("--selector", choices=sorted(SELECTOR_NAMES), default="eps")
+    ap.add_argument("--target", choices=sorted(TARGET_KINDS), default="qlearning")
+    ap.add_argument("--policy", choices=["basic", "double"], default="basic")
+    ap.add_argument("--agents_per_point", type=int, default=1024)
+    ap.add_argument("--seed", type=lambda x: int(x, 0), default=0x5EED0001)
+    ap.add_argument("--real", choices=["f32", "f64"], default="f64")
+    ap.add_argument("--device", type=int, default=0)
+    ap.add_argument("--out", default=None, help="write the result as JSON here")
+    a = vars(ap.parse_args(argv))
+    grid = {}
+    for name in SWEEP_FLAGS:
+        v = a.pop(name)
+        if v is not None:
+            grid[name] = parse_list(v)
+    for item in a.pop("grid"):
+        if "=" not in item:
+            ap.error("--grid takes FLAG=V1,V2,...")
+        k, v = item.split("=", 1)
+        if k not in SWEEP_FLAGS:
+            ap.error("--grid %s: not a sweepable flag (%s)" % (k, ", ".join(SWEEP_FLAGS)))
+        grid[k] = parse_list(v)
+    if not grid:
+        ap.error("nothing to sweep: give at least one --grid FLAG=V1,V2,...")
+    env_name, outp = a.pop("env"), a.pop("out")
+    res = run_sweep(env_name, grid, **a)
+    if outp:
+        with open(outp, "w") as fh:
+            json.dump(res, fh)
+    return res

@@ -1,6 +1,8 @@
 """Snapshot / resume of an engine at an episode boundary ("next" row N3; the reference has no checkpointing at all).
 The complete state is: Q tables, UCB counts, and per agent the RNG word index, epsilon, UCB t and Double flag
-(rlb_download_tables / rlb_get_agent_states), plus the Dyna model when one is attached (rlb_download_model).  Stored as one .npz; the configuration is stored beside it and checked."""
+(rlb_download_tables / rlb_get_agent_states), plus the Dyna model when one is attached (rlb_download_model) and the
+per-agent hyper-parameter sets when they are installed (rlb_engine_set_hparams).  Stored as one .npz; the configuration
+is stored beside it and checked."""
 import ctypes as C
 
 import numpy as np
@@ -16,6 +18,8 @@ def save_snapshot(engine, path):
     extra = {}
     if planning:
         extra["model_len"], extra["model"] = engine.download_model()
+    if engine.hparams is not None:
+        extra["hp_sets"], extra["hp_group"] = engine.hparams
     q, counts = engine.download_tables()
     cfg = {k: int(getattr(engine.cfg, k)) for k in _CFG_FIELDS}
     np.savez_compressed(path, q=q, counts=counts, states=engine.states(), selector_kind=np.int64(engine.cfg.selector_kind),
@@ -30,6 +34,11 @@ def load_snapshot(engine, path):
             raise ValueError("snapshot was taken with %s = %d, engine has %d" % (k, int(z["cfg_" + k]), int(getattr(engine.cfg, k))))
     if int(z["selector_kind"]) != int(engine.cfg.selector_kind):
         engine.set_selector(int(z["selector_kind"]))
+    # the sets before the tables and states: installing them refills both with each agent's constructor values
+    if "hp_sets" in z.files:
+        engine.set_hparams(z["hp_sets"], z["hp_group"])
+    elif engine.G:
+        engine.set_hparams(None, None)
     has_counts = int(z["selector_kind"]) == 1
     engine.upload_tables(z["q"], z["counts"] if has_counts else None)
     engine.set_states(z["states"])

@@ -255,6 +255,19 @@ typedef struct rlb_hparams {
  * (rlb_agent_set_model / rlb_config.planning_steps) together with sets, whichever comes second. */
 rlb_status rlb_engine_set_hparams(rlb_engine* e, const rlb_hparams* sets, uint32_t n_sets, const uint32_t* group);
 uint32_t rlb_engine_hparam_sets(const rlb_engine* e);    /* 0 while rlb_config's values apply */
+/* Replace the values of the installed hyper-parameter sets without reconstructing any agent (the explore step of
+ * population-based training; no reference equivalent).  sets [n_sets], host or device: sets[g] becomes the values of
+ * installed set g.  The groups, the grouped-reduction order and everything stored per agent (tables, epsilon, UCB state,
+ * flags, model, RNG position) stay as they are.  From the next call on every kernel uses the new learning_rate,
+ * discount_factor, lambda_factor, confidence_level, epsilon_decay and final_epsilon; initial_epsilon and default_value
+ * take effect at the next reset (rlb_agent_reset, rlb_selector_reset, rlb_policy_reset, rlb_agent_set_kind,
+ * rlb_agent_set_action_selector).
+ * Equivalence: from here on every call gives the bits of an engine B created with the same rlb_config, then
+ * rlb_engine_set_hparams(sets, n_sets, the same group), then given this engine's tables, agent states and model
+ * (rlb_upload_tables, rlb_set_agent_states, rlb_upload_model).
+ * RLB_ERR_INVALID_ARG, the engine untouched: sets == NULL, no sets installed, n_sets != rlb_engine_hparam_sets(e).
+ * Values are not checked. */
+rlb_status rlb_engine_retune_hparams(rlb_engine* e, const rlb_hparams* sets, uint32_t n_sets);
 
 /* ---- Env<T,COUNT> (env.rs:19-49), batched ------------------------------------------------ */
 /* Env::reset (blackjack.rs:105, frozen_lake.rs:106, cliff_walking.rs:67, taxi.rs:135).  obs_out [N] u32 */
@@ -367,6 +380,21 @@ rlb_status rlb_download_tables(rlb_engine* e, void* q_out, uint32_t* counts_out)
 rlb_status rlb_upload_tables(rlb_engine* e, const void* q, const uint32_t* counts);
 rlb_status rlb_get_agent_states(rlb_engine* e, rlb_agent_state* states_out /* [N] */);
 rlb_status rlb_set_agent_states(rlb_engine* e, const rlb_agent_state* states /* [N] */);
+/* Agent dst[j] takes the learned state of agent src[j], for j < n_pairs (the exploit step of population-based training;
+ * no reference equivalent), in one device launch: its Q table(s) (both for Double), its UCB counts when the selector is
+ * UCB, epsilon, ucb_t and policy_flag, and its Dyna model when one is attached (entries, membership bits, length).
+ * dst[j] keeps its RNG stream position rng_n (its Philox stream stays keyed by its own global id, so a clone does not
+ * replay the source's draws), its env state, its eligibility rows and lazy-sweep bookkeeping, its rlb_agent_step state
+ * and its hyper-parameter set.  src, dst [n_pairs] u32, host or device.
+ * Equivalence: the result is bit for bit what rlb_download_tables + rlb_get_agent_states (+ rlb_download_model), a copy
+ * of those fields from src[j] to dst[j] on the host, and the matching uploads give.  So, like rlb_agent_state, the call
+ * is complete AT AN EPISODE BOUNDARY, which is where rlb_agent_train / rlb_agent_evaluate leave every agent.
+ * A source may appear any number of times (one winner, many losers).  n_pairs == 0 does nothing.
+ * RLB_ERR_INVALID_ARG, the engine untouched: a NULL src or dst with n_pairs > 0, an id >= N, a dst that appears twice,
+ * an id that is both a source and a destination anywhere in the call (so no pair writes what another reads, and the
+ * result does not depend on the order of the pairs).  RLB_ERR_UNSUPPORTED: an eligibility-trace agent under a Dyna model
+ * (its rows survive episode boundaries there). */
+rlb_status rlb_agent_clone(rlb_engine* e, const uint32_t* src, const uint32_t* dst, uint64_t n_pairs);
 
 /* ---- multi-GPU: the path's one exchange (no reference equivalent: the crate is single-threaded) ----------------
  * Agents are independent, so a job shards by contiguous ranges of GLOBAL agent id (rlb_config.first_agent_id) with no

@@ -82,7 +82,7 @@ EXPORTS = [
     "rlb_agent_train_range_async", "rlb_agent_train_wait", "rlb_agent_step",
     "rlb_comm_unique_id", "rlb_comm_init_rank", "rlb_comm_init_all", "rlb_comm_destroy", "rlb_comm_rank", "rlb_comm_world_size",
     "rlb_comm_gather_episode_sums", "rlb_comm_allreduce_sum", "rlb_comm_group_begin", "rlb_comm_group_end",
-    "rlb_selftest_ucb_math", "rlb_engine_set_hparams", "rlb_engine_hparam_sets",
+    "rlb_selftest_ucb_math", "rlb_engine_set_hparams", "rlb_engine_hparam_sets", "rlb_engine_retune_hparams", "rlb_agent_clone",
 ]
 
 
@@ -119,6 +119,8 @@ def _load():
     L.rlb_engine_set_hparams.argtypes = [vp, vp, u32, vp]
     L.rlb_engine_hparam_sets.restype = u32
     L.rlb_engine_hparam_sets.argtypes = [vp]
+    L.rlb_engine_retune_hparams.argtypes = [vp, vp, u32]
+    L.rlb_agent_clone.argtypes = [vp, vp, vp, u64]
     L.rlb_env_reset.argtypes = [vp, vp]
     L.rlb_env_step.argtypes = [vp, vp, vp, vp, vp, vp]
     L.rlb_agent_get_action.argtypes = [vp, vp, vp]
@@ -310,6 +312,29 @@ class Engine:
     def hparam_sets(self):
         """rlb_engine_hparam_sets: the number of sets installed, 0 while the configured values apply."""
         return lib.rlb_engine_hparam_sets(self.h)
+
+    def retune_hparams(self, sets):
+        """rlb_engine_retune_hparams: sets[g] becomes the values of installed set g from the next call on, the learned
+        state left alone (initial_epsilon and default_value take effect at the next reset; see include/rlb.h).  `sets` as
+        for set_hparams, one per installed set.  `hparams` then holds the new values, so snapshots record them."""
+        arr = self.hparams_array(sets)
+        check(lib.rlb_engine_retune_hparams(self.h, ptr(arr) if len(arr) else None, len(arr)))
+        self.hparams = (arr.copy(), self.hparams[1])
+
+    # ---- population-based training: the exploit step
+    def clone_agents(self, src, dst):
+        """rlb_agent_clone: agent dst[j] takes the learned state (tables, counts, epsilon, UCB t, Double flag, model) of
+        agent src[j]; it keeps its RNG stream, env and hyper-parameter set.  Complete at an episode boundary.  No id may be
+        both a source and a destination, and no destination may appear twice."""
+        ids = []
+        for a in (src, dst):
+            a = np.asarray(a)
+            if a.ndim != 1 or (a.size and (a.min() < 0 or a.max() >= 2 ** 32)):
+                raise ValueError("agent ids must be a 1-d array of integers in [0, 2**32)")
+            ids.append(np.ascontiguousarray(a, np.uint32))
+        if len(ids[0]) != len(ids[1]):
+            raise ValueError("src and dst must have the same length")
+        check(lib.rlb_agent_clone(self.h, ptr(ids[0]), ptr(ids[1]), len(ids[0])))
 
     def _sums_shape(self, n):
         return (n, self.G, 4) if self.G else (n, 4)

@@ -853,6 +853,23 @@ rlb_status rlb_engine_dims(const rlb_engine* e, uint32_t* n_states, uint32_t* n_
 }
 uint32_t rlb_engine_store_kind(const rlb_engine* e) { return e ? (uint32_t)e->store : 0u; }
 
+// the installed sets' values (d_hp_sets) and, narrowed on the host exactly as the engine-wide fills narrow rlb_config's,
+// the fills' values (d_hp_q0, d_hp_eps0); synchronous, so `h_sets` may go when it returns
+static cudaError_t write_set_values(rlb_engine* e, const std::vector<rlb_hparams>& h_sets) {
+    const size_t n_sets = h_sets.size();
+    std::vector<double> eps0(n_sets), q0d(n_sets);
+    std::vector<float> q0f(n_sets);
+    for (size_t g = 0; g < n_sets; ++g) { eps0[g] = h_sets[g].initial_epsilon; q0d[g] = h_sets[g].default_value; q0f[g] = (float)h_sets[g].default_value; }
+    cudaError_t err = cudaMemcpyAsync(e->d_hp_sets, h_sets.data(), n_sets * sizeof(rlb_hparams), cudaMemcpyHostToDevice, e->stream);
+    if (err == cudaSuccess) {
+        if (e->cfg.real_kind == RLB_REAL_F32) err = cudaMemcpyAsync(e->d_hp_q0, q0f.data(), n_sets * 4, cudaMemcpyHostToDevice, e->stream);
+        else err = cudaMemcpyAsync(e->d_hp_q0, q0d.data(), n_sets * 8, cudaMemcpyHostToDevice, e->stream);
+    }
+    if (err == cudaSuccess) err = cudaMemcpyAsync(e->d_hp_eps0, eps0.data(), n_sets * sizeof(double), cudaMemcpyHostToDevice, e->stream);
+    if (err == cudaSuccess) err = cudaStreamSynchronize(e->stream);
+    return err;
+}
+
 rlb_status rlb_engine_set_hparams(rlb_engine* e, const rlb_hparams* sets, uint32_t n_sets, const uint32_t* group) {
     if (!e) { set_error("engine is NULL"); return RLB_ERR_INVALID_ARG; }
     if (n_sets == 0 && (sets || group)) { set_error("n_sets == 0 with a non-NULL sets or group"); return RLB_ERR_INVALID_ARG; }
@@ -884,23 +901,16 @@ rlb_status rlb_engine_set_hparams(rlb_engine* e, const rlb_hparams* sets, uint32
         for (uint32_t g = 0; g < n_sets; ++g) offsets[g + 1] += offsets[g];
         std::vector<uint32_t> next(offsets.begin(), offsets.end() - 1);
         for (uint64_t i = 0; i < N; ++i) order[next[h_group[i]]++] = (uint32_t)i;
-        // the fills' values, narrowed on the host exactly as the engine-wide fills narrow rlb_config's
-        std::vector<double> eps0(n_sets), q0d(n_sets);
-        std::vector<float> q0f(n_sets);
-        for (uint32_t g = 0; g < n_sets; ++g) { eps0[g] = h_sets[g].initial_epsilon; q0d[g] = h_sets[g].default_value; q0f[g] = (float)h_sets[g].default_value; }
         CK(cudaMalloc(&e->d_hp_sets, (size_t)n_sets * sizeof(rlb_hparams)));
         CK(cudaMalloc(&e->d_hp_group, N * sizeof(uint32_t)));
         CK(cudaMalloc(&e->d_hp_order, N * sizeof(uint32_t)));
         CK(cudaMalloc(&e->d_hp_offsets, (size_t)(n_sets + 1) * sizeof(uint32_t)));
         CK(cudaMalloc(&e->d_hp_q0, (size_t)n_sets * e->real_size));
         CK(cudaMalloc(&e->d_hp_eps0, (size_t)n_sets * sizeof(double)));
-        CK(cudaMemcpyAsync(e->d_hp_sets, h_sets.data(), (size_t)n_sets * sizeof(rlb_hparams), cudaMemcpyHostToDevice, e->stream));
         CK(cudaMemcpyAsync(e->d_hp_group, h_group.data(), N * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
         CK(cudaMemcpyAsync(e->d_hp_order, order.data(), N * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
         CK(cudaMemcpyAsync(e->d_hp_offsets, offsets.data(), (size_t)(n_sets + 1) * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
-        if (e->cfg.real_kind == RLB_REAL_F32) CK(cudaMemcpyAsync(e->d_hp_q0, q0f.data(), (size_t)n_sets * 4, cudaMemcpyHostToDevice, e->stream));
-        else CK(cudaMemcpyAsync(e->d_hp_q0, q0d.data(), (size_t)n_sets * 8, cudaMemcpyHostToDevice, e->stream));
-        CK(cudaMemcpyAsync(e->d_hp_eps0, eps0.data(), (size_t)n_sets * sizeof(double), cudaMemcpyHostToDevice, e->stream));
+        CK(write_set_values(e, h_sets));
         e->hp_n = n_sets;
     }
     // the constructors again, with each agent's own values: fresh tables, policy_flag = true, an empty trace, a fresh
@@ -914,6 +924,61 @@ rlb_status rlb_engine_set_hparams(rlb_engine* e, const rlb_hparams* sets, uint32
     return RLB_OK;
 }
 uint32_t rlb_engine_hparam_sets(const rlb_engine* e) { return e ? e->hp_n : 0u; }
+
+rlb_status rlb_engine_retune_hparams(rlb_engine* e, const rlb_hparams* sets, uint32_t n_sets) {
+    if (!e || !sets) { set_error("NULL argument"); return RLB_ERR_INVALID_ARG; }
+    if (!e->hp_n) { set_error("no hyper-parameter sets are installed (rlb_engine_set_hparams)"); return RLB_ERR_INVALID_ARG; }
+    if (n_sets != e->hp_n) { set_error("n_sets = %u, but %u sets are installed", n_sets, e->hp_n); return RLB_ERR_INVALID_ARG; }
+    ENTER(e);
+    std::vector<rlb_hparams> h_sets(n_sets);
+    CK(cudaMemcpy(h_sets.data(), sets, (size_t)n_sets * sizeof(rlb_hparams), is_device_ptr(sets) ? cudaMemcpyDeviceToHost : cudaMemcpyHostToHost));
+    CK(write_set_values(e, h_sets));
+    return RLB_OK;
+}
+
+rlb_status rlb_agent_clone(rlb_engine* e, const uint32_t* src, const uint32_t* dst, uint64_t n_pairs) {
+    if (!e) { set_error("engine is NULL"); return RLB_ERR_INVALID_ARG; }
+    if (!n_pairs) return RLB_OK;
+    if (!src || !dst) { set_error("NULL argument"); return RLB_ERR_INVALID_ARG; }
+    const uint64_t N = e->cfg.n_agents;
+    if (n_pairs > N) { set_error("n_pairs = %llu > n_agents: some destination appears twice", (unsigned long long)n_pairs); return RLB_ERR_INVALID_ARG; }
+    if (e->cfg.planning_steps && e->cfg.agent_kind == RLB_AGENT_TRACES) {
+        // planning updates run with terminated = false: the eligibility rows survive episode boundaries
+        set_error("cloning an eligibility-trace agent under a Dyna model is not supported");
+        return RLB_ERR_UNSUPPORTED;
+    }
+    ENTER(e);
+    std::vector<uint32_t> ids(2 * n_pairs);   // src then dst
+    CK(cudaMemcpy(ids.data(), src, n_pairs * 4, is_device_ptr(src) ? cudaMemcpyDeviceToHost : cudaMemcpyHostToHost));
+    CK(cudaMemcpy(ids.data() + n_pairs, dst, n_pairs * 4, is_device_ptr(dst) ? cudaMemcpyDeviceToHost : cudaMemcpyHostToHost));
+    for (uint64_t j = 0; j < 2 * n_pairs; ++j)
+        if (ids[j] >= N) { set_error("%s[%llu] = %u >= n_agents", j < n_pairs ? "src" : "dst", (unsigned long long)(j % n_pairs), ids[j]); return RLB_ERR_INVALID_ARG; }
+    // no destination twice, and no id both a source and a destination: then no pair writes what another reads
+    std::vector<uint8_t> is_dst(N, 0);
+    for (uint64_t j = 0; j < n_pairs; ++j) {
+        if (is_dst[ids[n_pairs + j]]) { set_error("dst[%llu] = %u appears twice", (unsigned long long)j, ids[n_pairs + j]); return RLB_ERR_INVALID_ARG; }
+        is_dst[ids[n_pairs + j]] = 1;
+    }
+    for (uint64_t j = 0; j < n_pairs; ++j)
+        if (is_dst[ids[j]]) { set_error("agent %u is both a source and a destination", ids[j]); return RLB_ERR_INVALID_ARG; }
+    const void* d_ids;
+    CK(stage_in(e, 0, ids.data(), 2 * n_pairs * 4, &d_ids));
+    CloneArgs a{};
+    // whole padded rows: the round trip moves only the A real columns, but padding exists only under -DRLB_TAXI_APAD=8,
+    // and load_row / store_row read and write the first A columns of a row alone, so what the padding holds is never used
+    a.seg[a.n_seg++] = CloneSegment{(uint8_t*)e->d_q, e->q_bytes / N};
+    if (e->cfg.selector_kind == RLB_SEL_UCB) a.seg[a.n_seg++] = CloneSegment{(uint8_t*)e->d_counts, e->counts_bytes / N};
+    if (e->cfg.planning_steps) {
+        a.seg[a.n_seg++] = CloneSegment{(uint8_t*)e->d_model_ent, (uint64_t)e->dp.mcap * sizeof(uint2)};
+        a.seg[a.n_seg++] = CloneSegment{(uint8_t*)e->d_model_bits, (uint64_t)e->dp.mwords * sizeof(uint32_t)};
+        a.model_len = e->d_model_len;
+    }
+    a.src = (const uint32_t*)d_ids; a.dst = a.src + n_pairs; a.n_pairs = n_pairs;
+    a.eps = e->d_eps; a.ucb_t = e->d_ucb_t; a.flag = e->d_flag;
+    CK(launch_clone_agents(a, e->stream));
+    CK(cudaStreamSynchronize(e->stream));
+    return RLB_OK;
+}
 
 // ------------------------------------------------------------------------------- Env
 rlb_status rlb_env_reset(rlb_engine* e, uint32_t* obs_out) {

@@ -62,4 +62,24 @@ cudaError_t launch_eps_decay_grouped(double* eps, uint64_t n_agents, int kind, c
 cudaError_t launch_episode_sums_grouped(int real_kind, const void* records, uint64_t n_agents, const uint32_t* order,
                                         const uint32_t* offsets, uint32_t n_sets, uint64_t n_ep, double* out, cudaStream_t stream);
 
+// ---- agent-to-agent copies of learned state (rlb_clone.cu, rlb_agent_clone) ----
+constexpr int CLONE_MAX_SEGMENTS = 4;   // Q, UCB counts, model entries, model bits
+struct CloneSegment {
+    uint8_t* base;     // agent i's block is [base + i * stride, base + (i + 1) * stride)
+    uint64_t stride;   // bytes, a multiple of 4
+};
+struct CloneArgs {
+    CloneSegment seg[CLONE_MAX_SEGMENTS];
+    uint32_t n_seg;
+    const uint32_t* src;   // [n_pairs] device: no id in src is also in dst, no id appears twice in dst
+    const uint32_t* dst;
+    uint64_t n_pairs;
+    double* eps;
+    uint64_t* ucb_t;
+    uint8_t* flag;
+    uint32_t* model_len;   // nullptr without a model
+};
+// every segment's block, eps, ucb_t, flag and model_len of agent dst[j] = those of agent src[j]: one launch of k_clone_agents
+cudaError_t launch_clone_agents(const CloneArgs& a, cudaStream_t stream);
+
 }   // namespace rlb

@@ -337,43 +337,43 @@ def point_hparams(flags, n_episodes):
                 final_epsilon=flags["final_epsilon"], confidence_level=flags["confidence_level"], default_value=0.0)
 
 
-def run_sweep(env_name, grid, *, agent="onestep", selector="eps", target="qlearning", policy="basic", agents_per_point=1024,
-              seed=0x5EED0001, real="f64", device=0, verbose=True, **flags):
-    """One run of the bin (`train(n, n/10)` -> `evaluate(n)`, bin/taxi.rs:165-188) for every point of the cartesian grid
-    of `grid` ({flag: [values]}, flags otherwise as in run_experiment), all points at once: ONE engine, the points'
-    agents in contiguous groups of `agents_per_point`, each group constructed with its point's values
-    (rlb_engine_set_hparams); the grouped per-episode sums give every point its own curves.  Returns the bins' moving
-    averages of return and episode length per point, the evaluate mean return, and the points ranked by it."""
+def grid_engine(env_name, grid, *, agent, selector, target, policy, agents_per_point, seed, real, device, **flags):
+    """The grid as one engine: every point of the cartesian grid of `grid` a set, its agents a contiguous group of
+    `agents_per_point` constructed with the point's values (rlb_engine_set_hparams).  Returns (engine, n_episodes,
+    moving-average window, points, every point's flags, every point's rlb_hparams)."""
     f = dict(DEFAULTS)
     f.update(flags)
     n = int(f["n_episodes"])
     window = max(1, n // int(f["moving_average_window"]))
     points = expand_grid(grid)
-    sets = []
+    point_flags = []
     for pt in points:
         pf = dict(f)
         pf.update(pt)
-        sets.append(point_hparams(pf, n))
+        point_flags.append(pf)
+    sets = [point_hparams(pf, n) for pf in point_flags]
     if len(sets) > abi.MAX_HPARAM_SETS:
         raise ValueError("%d grid points; an engine holds at most %d sets" % (len(sets), abi.MAX_HPARAM_SETS))
     env = make_env(env_name, **f)
-    n_agents = len(points) * int(agents_per_point)
-    eng = abi.Engine(env.kind, n_agents=n_agents, policy=abi.POLICY_BASIC if policy == "basic" else abi.POLICY_DOUBLE,
+    eng = abi.Engine(env.kind, n_agents=len(points) * int(agents_per_point), policy=abi.POLICY_BASIC if policy == "basic" else abi.POLICY_DOUBLE,
                      selector=SELECTOR_NAMES[selector], target=TARGET_KINDS[target], agent=AGENT_NAMES[agent],
                      real=abi.REAL_F32 if real == "f32" else abi.REAL_F64, decay_kind=abi.DECAY_SUB, seed=seed, device=device,
                      **sets[0], **env._cfg())
     try:
         eng.set_hparams(sets, np.repeat(np.arange(len(points), dtype=np.uint32), int(agents_per_point)))
-        t0 = time.perf_counter()
-        res = eng.train(n, max(1, n // 10))                                                          # [n, G, 4]
-        ev = eng.evaluate(n, sums=True)["sums"]                                                      # [n, G, 4]
-        dt = time.perf_counter() - t0
-    finally:
+    except BaseException:
         eng.close()
+        raise
+    return eng, n, window, points, point_flags, sets
+
+
+def point_results(points, sets, train_sums, eval_sums, agents_per_point, n, window):
+    """Per point: the bins' moving averages of return and episode length (train and evaluate) and the evaluate mean
+    return, from the grouped sums [n, G, 4]; and the points ranked by that return."""
     per = float(agents_per_point)
     out_points = []
     for g, pt in enumerate(points):
-        s_, e_ = res["sums"][:, g], ev[:, g]
+        s_, e_ = train_sums[:, g], eval_sums[:, g]
         out_points.append(dict(params=pt, hparams=sets[g],
                                train_rewards=moving_average(window, s_[:, 1] / per),
                                train_episodes_length=moving_average(window, s_[:, 0] / per),
@@ -381,6 +381,26 @@ def run_sweep(env_name, grid, *, agent="onestep", selector="eps", target="qlearn
                                test_episodes_length=moving_average(window, e_[:, 0] / per),
                                eval_mean_return=float(e_[:, 1].sum()) / (per * n)))
     ranking = sorted(range(len(points)), key=lambda g: -out_points[g]["eval_mean_return"])
+    return out_points, ranking
+
+
+def run_sweep(env_name, grid, *, agent="onestep", selector="eps", target="qlearning", policy="basic", agents_per_point=1024,
+              seed=0x5EED0001, real="f64", device=0, verbose=True, **flags):
+    """One run of the bin (`train(n, n/10)` -> `evaluate(n)`, bin/taxi.rs:165-188) for every point of the cartesian grid
+    of `grid` ({flag: [values]}, flags otherwise as in run_experiment), all points at once: ONE engine, the points'
+    agents in contiguous groups of `agents_per_point`, each group constructed with its point's values
+    (rlb_engine_set_hparams); the grouped per-episode sums give every point its own curves.  Returns the bins' moving
+    averages of return and episode length per point, the evaluate mean return, and the points ranked by it."""
+    eng, n, window, points, _, sets = grid_engine(env_name, grid, agent=agent, selector=selector, target=target, policy=policy,
+                                                  agents_per_point=agents_per_point, seed=seed, real=real, device=device, **flags)
+    try:
+        t0 = time.perf_counter()
+        res = eng.train(n, max(1, n // 10))                                                          # [n, G, 4]
+        ev = eng.evaluate(n, sums=True)["sums"]                                                      # [n, G, 4]
+        dt = time.perf_counter() - t0
+    finally:
+        eng.close()
+    out_points, ranking = point_results(points, sets, res["sums"], ev, agents_per_point, n, window)
     if verbose:
         print("%d points x %d agents, %d episodes: %.2fs (%.3g train steps/s)" % (len(points), agents_per_point, n, dt,
                                                                                   res["train_steps"] / dt if dt > 0 else 0.0))
@@ -395,10 +415,10 @@ def parse_list(text):
     return [float(x) for x in text.split(",") if x.strip()]
 
 
-def main_sweep(argv=None):
+def sweep_parser(description):
+    """The flags of tools/rl_sweep.py (and, with their own additions, tools/rl_pbt.py)."""
     import argparse
-    ap = argparse.ArgumentParser(description="Hyper-parameter sweep of one RL-Rust bin run over the B200 engine: every point "
-                                             "of the grid is a group of agents of one engine")
+    ap = argparse.ArgumentParser(description=description)
     ap.add_argument("env", choices=["blackjack", "frozen_lake", "cliffwalking", "taxi"])
     ap.add_argument("--grid", action="append", default=[], metavar="FLAG=V1,V2,...",
                     help="a bin flag and its values (repeatable; one of %s)" % ", ".join(SWEEP_FLAGS))
@@ -418,6 +438,11 @@ def main_sweep(argv=None):
     ap.add_argument("--real", choices=["f32", "f64"], default="f64")
     ap.add_argument("--device", type=int, default=0)
     ap.add_argument("--out", default=None, help="write the result as JSON here")
+    return ap
+
+
+def parse_sweep_args(ap, argv):
+    """(env name, grid, output path, the other flags as keyword arguments)"""
     a = vars(ap.parse_args(argv))
     grid = {}
     for name in SWEEP_FLAGS:
@@ -433,9 +458,115 @@ def main_sweep(argv=None):
         grid[k] = parse_list(v)
     if not grid:
         ap.error("nothing to sweep: give at least one --grid FLAG=V1,V2,...")
-    env_name, outp = a.pop("env"), a.pop("out")
-    res = run_sweep(env_name, grid, **a)
-    if outp:
-        with open(outp, "w") as fh:
+    return a.pop("env"), grid, a.pop("out"), a
+
+
+def write_json(res, path):
+    if path:
+        with open(path, "w") as fh:
             json.dump(res, fh)
+
+
+def main_sweep(argv=None):
+    ap = sweep_parser("Hyper-parameter sweep of one RL-Rust bin run over the B200 engine: every point of the grid is a "
+                      "group of agents of one engine")
+    env_name, grid, outp, kw = parse_sweep_args(ap, argv)
+    res = run_sweep(env_name, grid, **kw)
+    write_json(res, outp)
+    return res
+
+
+# ---- population-based training (Jaderberg et al., 2017): the sweep's grid as the initial population ----------------------
+PBT_FACTORS = (0.8, 1.2)
+_TINY = float(np.nextafter(0.0, 1.0))
+PBT_BOUNDS = dict(learning_rate=(_TINY, 1.0), discount_factor=(0.0, 1.0), lambda_factor=(0.0, 1.0), initial_epsilon=(0.0, 1.0),
+                  final_epsilon=(0.0, 1.0), exploration_time=(_TINY, np.inf), confidence_level=(0.0, np.inf))   # (0, 1], [0, 1], > 0, >= 0
+
+
+def pbt_exploit(chunk_sums, fraction, rng):
+    """Ranks the sets by their mean training return over a chunk (chunk_sums [episodes, G, 4]; every set holds the same
+    number of agents) and pairs each of the bottom floor(fraction * G) sets with a set drawn uniformly from the top as many.
+    Returns [(loser, winner)], losers from the weakest up."""
+    n_sets = chunk_sums.shape[1]
+    mean_ret = chunk_sums[:, :, 1].sum(0)
+    order = sorted(range(n_sets), key=lambda g: (-mean_ret[g], g))   # best first; ties by set index
+    k = int(np.floor(fraction * n_sets))
+    top, bottom = order[:k], order[n_sets - k:][::-1]
+    return [(loser, top[int(rng.integers(k))]) for loser in bottom]
+
+
+def pbt_explore(flags, axes, rng):
+    """The winner's flags with every grid axis multiplied by 0.8 or 1.2 at random and clamped into its range."""
+    out = dict(flags)
+    for k in axes:
+        lo, hi = PBT_BOUNDS[k]
+        out[k] = float(min(max(flags[k] * PBT_FACTORS[int(rng.integers(2))], lo), hi))
+    return out
+
+
+def run_pbt(env_name, grid, *, interval, fraction=0.25, pbt_seed=0x9B7, agent="onestep", selector="eps", target="qlearning",
+            policy="basic", agents_per_point=1024, seed=0x5EED0001, real="f64", device=0, verbose=True, **flags):
+    """Population-based training over the grid of `grid`: the initial population is run_sweep's (one set per point,
+    contiguous groups of `agents_per_point`), and its one `train(n, n/10)` is driven in chunks of `interval` episodes.
+    After every chunk but the last the sets are ranked by their mean training return over the chunk; each of the bottom
+    floor(fraction * G) sets takes over the learned state of a set drawn from the top as many (agent j of the winner ->
+    agent j of the loser, one rlb_agent_clone) and continues with the winner's flags, every grid axis perturbed
+    (rlb_engine_retune_hparams).  `pbt_seed` seeds those draws.  Returns run_sweep's output plus every set's final flags
+    and the lineage: per chunk boundary, the list of (loser, winner, new flags)."""
+    if not 0.0 <= fraction <= 0.5:
+        raise ValueError("fraction must be in [0, 0.5]: the top and bottom sets may not overlap")
+    interval = int(interval)
+    if interval < 1:
+        raise ValueError("interval must be >= 1")
+    axes = list(grid)
+    per = int(agents_per_point)
+    eng, n, window, points, cur, sets = grid_engine(env_name, grid, agent=agent, selector=selector, target=target, policy=policy,
+                                                    agents_per_point=per, seed=seed, real=real, device=device, **flags)
+    rng = np.random.default_rng(pbt_seed)
+    lineage, parts, train_steps = [], [], 0          # cur: every set's flags in force
+    try:
+        t0 = time.perf_counter()
+        for begin in range(0, n, interval):
+            end = min(begin + interval, n)
+            res = eng.train(end, max(1, n // 10), ep_begin=begin)                                    # [end - begin, G, 4]
+            parts.append(res["sums"])
+            train_steps += int(res["train_steps"])
+            if end == n:
+                break
+            pairs = pbt_exploit(res["sums"], fraction, rng)
+            step = []
+            for loser, winner in pairs:
+                cur[loser] = pbt_explore(cur[winner], axes, rng)
+                sets[loser] = point_hparams(cur[loser], n)
+                step.append(dict(loser=loser, winner=winner, flags={k: cur[loser][k] for k in axes}))
+            if pairs:
+                j = np.arange(per, dtype=np.int64)
+                eng.clone_agents(np.concatenate([w * per + j for _, w in pairs]), np.concatenate([l * per + j for l, _ in pairs]))
+                eng.retune_hparams(sets)
+            lineage.append(dict(episode=end, pairs=step))
+        ev = eng.evaluate(n, sums=True)["sums"]                                                      # [n, G, 4]
+        dt = time.perf_counter() - t0
+    finally:
+        eng.close()
+    out_points, ranking = point_results(points, sets, np.concatenate(parts), ev, per, n, window)
+    for g, pt in enumerate(out_points):
+        pt["final_params"] = {k: cur[g][k] for k in axes}
+    if verbose:
+        print("PBT: %d sets x %d agents, %d episodes in chunks of %d, fraction %.3g: %.2fs" % (len(points), per, n, interval, fraction, dt))
+        for g in ranking[:10]:
+            print("  set %-4d %-60s evaluate mean return %.4f" % (g, out_points[g]["final_params"], out_points[g]["eval_mean_return"]))
+    return dict(env=env_name, agent=agent, selector=selector, target=target, policy=policy, real=real, n_episodes=n,
+                agents_per_point=per, grid={k: list(v) for k, v in grid.items()}, interval=interval, fraction=fraction,
+                pbt_seed=int(pbt_seed), points=out_points, ranking=ranking, lineage=lineage, seconds=dt, train_steps=train_steps)
+
+
+def main_pbt(argv=None):
+    ap = sweep_parser("Population-based training over one RL-Rust bin run on the B200 engine: the grid is the initial "
+                      "population, and between chunks the weakest sets take over the state of strong ones and perturb their flags")
+    ap.add_argument("--interval", type=int, required=True, help="episodes per chunk between exploit / explore steps")
+    ap.add_argument("--fraction", type=float, default=0.25, help="share of the sets replaced after each chunk (and drawn from)")
+    ap.add_argument("--pbt_seed", type=lambda x: int(x, 0), default=0x9B7, help="seed of the winner draws and perturbations")
+    env_name, grid, outp, kw = parse_sweep_args(ap, argv)
+    res = run_pbt(env_name, grid, **kw)
+    write_json(res, outp)
     return res

@@ -268,6 +268,25 @@ uint32_t rlb_engine_hparam_sets(const rlb_engine* e);    /* 0 while rlb_config's
  * RLB_ERR_INVALID_ARG, the engine untouched: sets == NULL, no sets installed, n_sets != rlb_engine_hparam_sets(e).
  * Values are not checked. */
 rlb_status rlb_engine_retune_hparams(rlb_engine* e, const rlb_hparams* sets, uint32_t n_sets);
+/* Pause and resume hyper-parameter sets (successive halving; no reference equivalent).  active [n_sets] u8, host or
+ * device: nonzero = set g takes part in later train / evaluate calls.  active = NULL, n_sets = 0: every set active (also
+ * the state after rlb_engine_set_hparams); an all-ones mask is the same.
+ * Which calls: rlb_agent_train, rlb_agent_train_range, rlb_agent_train_range_async and rlb_agent_evaluate run only the
+ * agents of active sets, in a launch sized to them.  Every other call (the step-level calls, rlb_agent_step, resets,
+ * rlb_agent_set_kind, rlb_agent_clone, snapshots, uploads and downloads) still acts on all N agents.
+ * Active agents get, bit for bit, what they would get with every set active: tables, counts, epsilon, UCB t, the Double
+ * flag, RNG position, env state, their episode records and their set's row of the per-episode sums.
+ * Inactive agents keep their whole state bit for bit (tables, counts, epsilon, t, flag, RNG position, env, eligibility
+ * rows, lazy-sweep bookkeeping, rlb_agent_step state).  Their records in a returned episodes buffer are zero, their
+ * td_count and traj_count 0, and their set's row of episode_sums / sums_out 0.0.  train_steps, eval_steps,
+ * eval_return_sum and eval_episodes count active agents only.  A set paused for some calls and then resumed continues
+ * from where it stopped: its agents equal those of an engine that made only the calls during which the set was active.
+ * Every set inactive is allowed: the compute calls then launch nothing and return zero sums and totals.
+ * rlb_engine_set_hparams makes every set active again (also when it uninstalls them); rlb_engine_retune_hparams keeps
+ * the mask.
+ * RLB_ERR_INVALID_ARG, the engine untouched: no sets installed, n_sets != rlb_engine_hparam_sets(e), or a NULL /
+ * non-NULL mismatch between active and n_sets. */
+rlb_status rlb_engine_set_active_sets(rlb_engine* e, const uint8_t* active, uint32_t n_sets);
 
 /* ---- Env<T,COUNT> (env.rs:19-49), batched ------------------------------------------------ */
 /* Env::reset (blackjack.rs:105, frozen_lake.rs:106, cliff_walking.rs:67, taxi.rs:135).  obs_out [N] u32 */

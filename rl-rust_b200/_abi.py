@@ -83,6 +83,7 @@ EXPORTS = [
     "rlb_comm_unique_id", "rlb_comm_init_rank", "rlb_comm_init_all", "rlb_comm_destroy", "rlb_comm_rank", "rlb_comm_world_size",
     "rlb_comm_gather_episode_sums", "rlb_comm_allreduce_sum", "rlb_comm_group_begin", "rlb_comm_group_end",
     "rlb_selftest_ucb_math", "rlb_engine_set_hparams", "rlb_engine_hparam_sets", "rlb_engine_retune_hparams", "rlb_agent_clone",
+    "rlb_engine_set_active_sets",
 ]
 
 
@@ -121,6 +122,7 @@ def _load():
     L.rlb_engine_hparam_sets.argtypes = [vp]
     L.rlb_engine_retune_hparams.argtypes = [vp, vp, u32]
     L.rlb_agent_clone.argtypes = [vp, vp, vp, u64]
+    L.rlb_engine_set_active_sets.argtypes = [vp, vp, u32]
     L.rlb_env_reset.argtypes = [vp, vp]
     L.rlb_env_step.argtypes = [vp, vp, vp, vp, vp, vp]
     L.rlb_agent_get_action.argtypes = [vp, vp, vp]
@@ -248,6 +250,7 @@ class Engine:
         self.episode_dtype = EPISODE_F32 if real == REAL_F32 else EPISODE_F64
         self.G = 0                  # hyper-parameter sets installed (set_hparams); per-episode sums are (E, G, 4) while G > 0
         self.hparams = None         # (sets, group) as installed
+        self.active_sets = None     # bool (G,) while some set is paused (set_active_sets), else None
 
     def close(self):
         if getattr(self, "h", None):
@@ -297,7 +300,7 @@ class Engine:
         While sets are installed, train() and evaluate() return per-episode sums shaped (E, G, 4)."""
         if sets is None and group is None:
             check(lib.rlb_engine_set_hparams(self.h, None, 0, None))
-            self.G, self.hparams = 0, None
+            self.G, self.hparams, self.active_sets = 0, None, None
             return
         arr = self.hparams_array(sets)
         grp = np.asarray(group)
@@ -307,7 +310,7 @@ class Engine:
             raise ValueError("group ids must be in [0, 2**32)")
         grp = np.ascontiguousarray(grp, np.uint32)
         check(lib.rlb_engine_set_hparams(self.h, ptr(arr) if len(arr) else None, len(arr), ptr(grp) if len(arr) else None))
-        self.G, self.hparams = len(arr), (arr.copy(), grp.copy())
+        self.G, self.hparams, self.active_sets = len(arr), (arr.copy(), grp.copy()), None
 
     def hparam_sets(self):
         """rlb_engine_hparam_sets: the number of sets installed, 0 while the configured values apply."""
@@ -320,6 +323,22 @@ class Engine:
         arr = self.hparams_array(sets)
         check(lib.rlb_engine_retune_hparams(self.h, ptr(arr) if len(arr) else None, len(arr)))
         self.hparams = (arr.copy(), self.hparams[1])
+
+    def set_active_sets(self, mask):
+        """rlb_engine_set_active_sets: only the sets whose entry of `mask` ((G,) bools) is true take part in later train()
+        and evaluate() calls; the other sets' agents are left exactly as they are, and their rows of the sums are 0.
+        mask=None makes every set active.  Every other call still acts on all agents (see include/rlb.h).
+        `active_sets` then holds the mask, or None while every set is active."""
+        if mask is None:
+            check(lib.rlb_engine_set_active_sets(self.h, None, 0))
+            self.active_sets = None
+            return
+        m = np.asarray(mask)
+        if m.shape != (self.G,):
+            raise ValueError("mask must have shape (%d,), got %r" % (self.G, m.shape))
+        m = np.ascontiguousarray(m != 0, np.uint8)
+        check(lib.rlb_engine_set_active_sets(self.h, ptr(m) if len(m) else None, len(m)))
+        self.active_sets = None if m.all() else m.astype(bool)
 
     # ---- population-based training: the exploit step
     def clone_agents(self, src, dst):

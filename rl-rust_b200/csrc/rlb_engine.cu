@@ -96,6 +96,12 @@ struct rlb_engine {
     uint32_t* d_hp_offsets = nullptr;  // [hp_n + 1] where each set starts in d_hp_order
     void* d_hp_q0 = nullptr;           // [hp_n] default_value narrowed to Real, for the table fills
     double* d_hp_eps0 = nullptr;       // [hp_n] initial_epsilon
+    std::vector<uint32_t> h_hp_order, h_hp_offsets;   // host copies of d_hp_order / d_hp_offsets
+    // active sets (rlb_engine_set_active_sets); hp_active is empty while every set is active
+    std::vector<uint8_t> hp_active;    // [hp_n] nonzero: the set takes part in train / evaluate calls
+    uint32_t* d_hp_run = nullptr;      // [hp_n_run] d_hp_order restricted to the active sets: k_run_hp's agent list and the reduction's order
+    uint32_t* d_hp_run_offsets = nullptr;   // [hp_n + 1] where each set starts in d_hp_run (an inactive set has length 0)
+    uint64_t hp_n_run = 0;
     // Calls whose work is enqueued but not yet waited for (rlb_agent_train_range_async): at most two, so that the
     // kernels of call i + 1 are in the queue before the host blocks on the copies of call i.
     struct Pending {
@@ -204,7 +210,8 @@ cudaError_t dispatch_run(rlb_engine* e, const DevParams& p) {
         }
     }
     if (e->hp_n) {   // every agent with its own hyper-parameter set (never with a model: rlb_engine_set_hparams)
-        const HpParams sets{e->d_hp_sets, e->d_hp_group};
+        const bool masked = !e->hp_active.empty();   // only the active sets' agents run: a launch sized to them
+        const HpParams sets{e->d_hp_sets, e->d_hp_group, masked ? e->d_hp_run : nullptr, masked ? e->hp_n_run : e->cfg.n_agents};
         switch (e->cfg.env_kind) {
             case RLB_ENV_BLACKJACK: return launch_run<RLB_ENV_BLACKJACK, true>(e->variant, p, e->store, e->stream, sets);
             case RLB_ENV_FROZEN_LAKE: return launch_run<RLB_ENV_FROZEN_LAKE, true>(e->variant, p, e->store, e->stream, sets);
@@ -429,8 +436,10 @@ uint64_t chunk_episodes(const rlb_engine* e, uint64_t want) {
 // sums_out [n_ep][4], or [n_ep][hp_n][4] with hyper-parameter sets
 rlb_status reduce_episodes(rlb_engine* e, uint64_t n_ep, const void* records, double* sums_out) {
     if (!n_ep) return RLB_OK;
-    if (e->hp_n) {
-        CK(launch_episode_sums_grouped(e->cfg.real_kind, records, e->cfg.n_agents, e->d_hp_order, e->d_hp_offsets, e->hp_n, n_ep, sums_out, e->stream));
+    if (e->hp_n) {   // with inactive sets: only the active sets' agents are read, an inactive set's row is 0.0
+        const bool masked = !e->hp_active.empty();
+        CK(launch_episode_sums_grouped(e->cfg.real_kind, records, e->cfg.n_agents, masked ? e->d_hp_run : e->d_hp_order,
+                                       masked ? e->d_hp_run_offsets : e->d_hp_offsets, e->hp_n, n_ep, sums_out, e->stream));
         return RLB_OK;
     }
     if (e->cfg.real_kind == RLB_REAL_F32) k_episode_sums<float><<<(unsigned)n_ep, 256, 0, e->stream>>>(records, e->cfg.n_agents, sums_out);
@@ -625,6 +634,8 @@ rlb_status enqueue_range(rlb_engine* e, int mode, uint64_t begin, uint64_t end, 
         char* const scratch = (char*)e->d_episodes + (pipelined ? (size_t)half * chunk * N * rec : 0);
         // this half's previous records — of this call or of the one before it — must have left
         if (pipelined) CK(cudaStreamWaitEvent(e->stream, e->ev_drained[half], 0));
+        // inactive sets' agents write no records: the caller gets zeros for them
+        if (rec_dst && !e->hp_active.empty()) CK(cudaMemsetAsync(scratch, 0, (c1 - c0) * N * rec, e->stream));
         DevParams p = e->dp;
         p.mode = mode;
         p.eval_at = eval_at;
@@ -815,7 +826,7 @@ void rlb_engine_destroy(rlb_engine* e) {
     void* bufs[] = {e->d_q, e->d_counts, e->d_etr, e->d_etr_il, e->d_vis, e->d_nvis, e->d_rng_n, e->d_eps, e->d_ucb_t, e->d_flag, e->d_env,
                     e->d_trans, e->d_thr, e->d_thr_state, e->d_totals, e->d_flagword, e->d_episodes, e->d_sums,
                     e->d_model_ent, e->d_model_bits, e->d_model_len, e->d_hp_sets, e->d_hp_group, e->d_hp_order, e->d_hp_offsets,
-                    e->d_hp_q0, e->d_hp_eps0};
+                    e->d_hp_q0, e->d_hp_eps0, e->d_hp_run, e->d_hp_run_offsets};
     for (void* b : bufs) if (b) cudaFree(b);
     for (void* b : e->d_stage) if (b) cudaFree(b);
     if (e->ev0) cudaEventDestroy(e->ev0);
@@ -889,10 +900,13 @@ rlb_status rlb_engine_set_hparams(rlb_engine* e, const rlb_hparams* sets, uint32
     // release the old sets (the kernels that read them have completed: ENTER waited for pending calls, and the stream
     // is drained before the buffers go)
     CK(cudaStreamSynchronize(e->stream));
-    void* old[] = {e->d_hp_sets, e->d_hp_group, e->d_hp_order, e->d_hp_offsets, e->d_hp_q0, e->d_hp_eps0};
+    void* old[] = {e->d_hp_sets, e->d_hp_group, e->d_hp_order, e->d_hp_offsets, e->d_hp_q0, e->d_hp_eps0, e->d_hp_run, e->d_hp_run_offsets};
     for (void* b : old) if (b) cudaFree(b);
     e->d_hp_sets = nullptr; e->d_hp_group = nullptr; e->d_hp_order = nullptr; e->d_hp_offsets = nullptr;
     e->d_hp_q0 = nullptr; e->d_hp_eps0 = nullptr;
+    e->d_hp_run = nullptr; e->d_hp_run_offsets = nullptr; e->hp_n_run = 0;
+    e->hp_active.clear();   // every set active again
+    e->h_hp_order.clear(); e->h_hp_offsets.clear();
     e->hp_n = 0;
     if (n_sets) {
         // the grouped reduction's read order: agents by set, ascending local index within a set (a stable counting sort)
@@ -911,6 +925,7 @@ rlb_status rlb_engine_set_hparams(rlb_engine* e, const rlb_hparams* sets, uint32
         CK(cudaMemcpyAsync(e->d_hp_order, order.data(), N * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
         CK(cudaMemcpyAsync(e->d_hp_offsets, offsets.data(), (size_t)(n_sets + 1) * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
         CK(write_set_values(e, h_sets));
+        e->h_hp_order = std::move(order); e->h_hp_offsets = std::move(offsets);
         e->hp_n = n_sets;
     }
     // the constructors again, with each agent's own values: fresh tables, policy_flag = true, an empty trace, a fresh
@@ -933,6 +948,39 @@ rlb_status rlb_engine_retune_hparams(rlb_engine* e, const rlb_hparams* sets, uin
     std::vector<rlb_hparams> h_sets(n_sets);
     CK(cudaMemcpy(h_sets.data(), sets, (size_t)n_sets * sizeof(rlb_hparams), is_device_ptr(sets) ? cudaMemcpyDeviceToHost : cudaMemcpyHostToHost));
     CK(write_set_values(e, h_sets));
+    return RLB_OK;
+}
+
+rlb_status rlb_engine_set_active_sets(rlb_engine* e, const uint8_t* active, uint32_t n_sets) {
+    if (!e) { set_error("engine is NULL"); return RLB_ERR_INVALID_ARG; }
+    if (!e->hp_n) { set_error("no hyper-parameter sets are installed (rlb_engine_set_hparams)"); return RLB_ERR_INVALID_ARG; }
+    if ((n_sets == 0) != (active == nullptr)) { set_error("active and n_sets: NULL with 0, or a mask of rlb_engine_hparam_sets() entries"); return RLB_ERR_INVALID_ARG; }
+    if (active && n_sets != e->hp_n) { set_error("n_sets = %u, but %u sets are installed", n_sets, e->hp_n); return RLB_ERR_INVALID_ARG; }
+    ENTER(e);
+    std::vector<uint8_t> mask(e->hp_n, 1);
+    if (active) CK(cudaMemcpy(mask.data(), active, n_sets, is_device_ptr(active) ? cudaMemcpyDeviceToHost : cudaMemcpyHostToHost));
+    bool all = true;
+    for (uint8_t& m : mask) { m = m ? 1 : 0; all = all && m; }
+    // the kernels that read the old list have completed (ENTER); drain the stream before it goes
+    CK(cudaStreamSynchronize(e->stream));
+    if (e->d_hp_run) cudaFree(e->d_hp_run);
+    if (e->d_hp_run_offsets) cudaFree(e->d_hp_run_offsets);
+    e->d_hp_run = nullptr; e->d_hp_run_offsets = nullptr; e->hp_n_run = 0;
+    e->hp_active.clear();
+    if (all) return RLB_OK;   // an all-ones mask is NULL: the identity launch
+    // d_hp_order restricted to the active sets, in the same order: contiguous groups stay ascending id ranges
+    std::vector<uint32_t> run, offsets(e->hp_n + 1, 0);
+    for (uint32_t g = 0; g < e->hp_n; ++g) {
+        if (mask[g]) run.insert(run.end(), e->h_hp_order.begin() + e->h_hp_offsets[g], e->h_hp_order.begin() + e->h_hp_offsets[g + 1]);
+        offsets[g + 1] = (uint32_t)run.size();
+    }
+    CK(cudaMalloc(&e->d_hp_run, std::max<size_t>(run.size(), 1) * sizeof(uint32_t)));
+    CK(cudaMalloc(&e->d_hp_run_offsets, offsets.size() * sizeof(uint32_t)));
+    if (!run.empty()) CK(cudaMemcpyAsync(e->d_hp_run, run.data(), run.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
+    CK(cudaMemcpyAsync(e->d_hp_run_offsets, offsets.data(), offsets.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
+    CK(cudaStreamSynchronize(e->stream));
+    e->hp_n_run = run.size();
+    e->hp_active = std::move(mask);
     return RLB_OK;
 }
 

@@ -84,9 +84,12 @@ struct RunKernel {
 
 template <int ENV, bool HP>
 cudaError_t launch_run(const Variant& v, const DevParams& p, int store, cudaStream_t stream, const HpParams& h) {
+    // threads the grid covers: every agent, or with per-agent sets the launch positions of h (the active sets' agents)
+    const uint64_t n = HP ? h.n_launch : p.n_agents;
+    if (n == 0) return cudaSuccess;   // every set inactive: nothing to run, and a grid of zero CTAs is an error
     if (store == STORE_HYBRID) {
         if constexpr (SmemCapable<ENV>::value) {
-            const unsigned grid = (unsigned)((p.n_agents + 31) / 32);   // one warp per CTA: 32 agents, one per lane
+            const unsigned grid = (unsigned)((n + 31) / 32);   // one warp per CTA: 32 agents, one per lane
             const size_t smem = smem_store_bytes<ENV>(v, store, p.n_live, p.S, p.vmax);
 #define RLB_CALL(R, P, SL, T)                                                                                          \
     {                                                                                                                  \
@@ -104,7 +107,7 @@ cudaError_t launch_run(const Variant& v, const DevParams& p, int store, cudaStre
     }
     if (store == STORE_SMEM) {
         if constexpr (SmemCapable<ENV>::value) {
-            const unsigned grid = (unsigned)((p.n_agents + 7) / 8);   // one warp per CTA: 8 agents x 4 lanes
+            const unsigned grid = (unsigned)((n + 7) / 8);   // one warp per CTA: 8 agents x 4 lanes
             const size_t smem = smem_store_bytes<ENV>(v, store, p.S, p.S, p.vmax);
 #define RLB_CALL(R, P, SL, T)                                                                                          \
     {                                                                                                                  \
@@ -120,12 +123,12 @@ cudaError_t launch_run(const Variant& v, const DevParams& p, int store, cudaStre
             return cudaErrorInvalidValue;
         }
     }
-    const unsigned grid = grid_for(p.n_agents);
+    const unsigned grid = grid_for(n);
     const size_t smem = EnvTab<ENV>::smem_bytes(p.S);
     if (store == STORE_LAZY) {   // trace agents, HBM tables, sweeps applied lazily: + the TD history in shared memory
         if (!v.trace) return cudaErrorInvalidValue;
         constexpr int kLazyBlock = RLB_LZ_BLOCK;
-        const unsigned lz_grid = (unsigned)((p.n_agents + kLazyBlock - 1) / kLazyBlock);
+        const unsigned lz_grid = (unsigned)((n + kLazyBlock - 1) / kLazyBlock);
         const size_t hist = ((smem + 15) & ~(size_t)15) + (size_t)p.lz_cap * kLazyBlock * (v.real == RLB_REAL_F32 ? 4 : 8);
 #define RLB_CALL(R, P, SL, T)                                                                                          \
     if constexpr (T) {                                                                                                 \

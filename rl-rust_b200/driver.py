@@ -570,3 +570,97 @@ def main_pbt(argv=None):
     res = run_pbt(env_name, grid, **kw)
     write_json(res, outp)
     return res
+
+
+# ---- successive halving (Jamieson & Talwalkar, 2016): train the grid on growing budgets, keep the best 1/eta each time ----
+def halving_rungs(n, min_episodes, eta):
+    """The rung budgets b_k = min(n, min_episodes * eta**k), k = 0, 1, ... up to the first that reaches n."""
+    if int(min_episodes) < 1 or int(eta) < 2:
+        raise ValueError("min_episodes must be >= 1 and eta >= 2")
+    out, b = [], int(min_episodes)
+    while True:
+        out.append(min(int(n), b))
+        if out[-1] >= n:
+            return out
+        b *= int(eta)
+
+
+def halving_select(rung_sums, active, eta):
+    """Ranks the active sets by their mean training return over a rung (rung_sums [episodes, G, 4]; every set holds the
+    same number of agents), ties by set index, and keeps the best max(1, floor(len(active) / eta)).  Returns (kept,
+    dropped): kept in ascending set index, dropped from the strongest down."""
+    ret = rung_sums[:, :, 1].sum(0)
+    order = sorted(active, key=lambda g: (-ret[g], g))
+    keep = max(1, len(active) // int(eta))
+    return sorted(order[:keep]), order[keep:]
+
+
+def run_halving(env_name, grid, *, min_episodes, eta=3, agent="onestep", selector="eps", target="qlearning", policy="basic",
+                agents_per_point=1024, seed=0x5EED0001, real="f64", device=0, verbose=True, **flags):
+    """Successive halving over the grid of `grid`: run_sweep's engine (one set per point, contiguous groups of
+    `agents_per_point`) and its one `train(n, n/10)`, driven in rungs that end at the budgets min(n, min_episodes * eta**k).
+    After every rung but the last the active sets are ranked by their mean training return over that rung, and all but
+    the best max(1, floor(active / eta)) are paused (rlb_engine_set_active_sets): they train no further, and the engine's
+    launches cover only the sets still running.  `evaluate(n)` then runs over the survivors.  A survivor's curves and
+    evaluate return are exactly run_sweep's for its point.  Returns run_sweep's output, where a dropped set's training
+    curves cover the episodes it trained and its test curves and evaluate return are None, plus per set
+    `episodes_trained`, `rung` (the rung it stopped at) and `last_rung_mean_return`, and `rungs`: each rung's budget and
+    its active and dropped sets.  The ranking lists the survivors by evaluate return, then the dropped sets by episodes
+    trained and by their last rung's return."""
+    per = int(agents_per_point)
+    eng, n, window, points, _, sets = grid_engine(env_name, grid, agent=agent, selector=selector, target=target, policy=policy,
+                                                  agents_per_point=per, seed=seed, real=real, device=device, **flags)
+    n_sets = len(points)
+    try:
+        budgets = halving_rungs(n, min_episodes, eta)
+        train_sums = np.zeros((n, n_sets, 4))
+        trained, stopped, last_ret = [0] * n_sets, [0] * n_sets, [0.0] * n_sets
+        active, rungs, train_steps, begin = list(range(n_sets)), [], 0, 0
+        t0 = time.perf_counter()
+        for k, end in enumerate(budgets):
+            res = eng.train(end, max(1, n // 10), ep_begin=begin)                                    # [end - begin, G, 4]
+            train_sums[begin:end] = res["sums"]                                                      # paused sets' rows: 0.0
+            train_steps += int(res["train_steps"])
+            rung_ret = res["sums"][:, :, 1].sum(0)
+            for g in active:
+                trained[g], stopped[g], last_ret[g] = end, k, float(rung_ret[g]) / (per * (end - begin))
+            kept, dropped = (halving_select(res["sums"], active, eta) if end < n else (active, []))
+            rungs.append(dict(rung=k, budget=end, episodes=[begin, end], active=list(active), dropped=sorted(dropped)))
+            if dropped:
+                mask = np.zeros(n_sets, bool)
+                mask[kept] = True
+                eng.set_active_sets(mask)
+            active, begin = kept, end
+        ev = eng.evaluate(n, sums=True)["sums"]                                                      # [n, G, 4]; dropped sets 0.0
+        dt = time.perf_counter() - t0
+    finally:
+        eng.close()
+    out_points, _ = point_results(points, sets, train_sums, ev, per, n, window)
+    survivors = set(active)
+    for g, pt in enumerate(out_points):
+        pt.update(episodes_trained=trained[g], rung=stopped[g], last_rung_mean_return=last_ret[g])
+        if g not in survivors:
+            s_ = train_sums[:trained[g], g]
+            pt.update(train_rewards=moving_average(window, s_[:, 1] / per), train_episodes_length=moving_average(window, s_[:, 0] / per),
+                      test_rewards=None, test_episodes_length=None, eval_mean_return=None)
+    ranking = sorted(survivors, key=lambda g: (-out_points[g]["eval_mean_return"], g))
+    ranking += sorted(set(range(n_sets)) - survivors, key=lambda g: (-trained[g], -last_ret[g], g))
+    if verbose:
+        print("successive halving: %d sets x %d agents, %d episodes, rungs %s (eta %d): %.2fs, %d train steps"
+              % (n_sets, per, n, budgets, int(eta), dt, train_steps))
+        for g in ranking[:min(10, len(survivors))]:
+            print("  set %-4d %-60s evaluate mean return %.4f" % (g, points[g], out_points[g]["eval_mean_return"]))
+    return dict(env=env_name, agent=agent, selector=selector, target=target, policy=policy, real=real, n_episodes=n,
+                agents_per_point=per, grid={k: list(v) for k, v in grid.items()}, min_episodes=int(min_episodes), eta=int(eta),
+                points=out_points, ranking=ranking, rungs=rungs, seconds=dt, train_steps=train_steps)
+
+
+def main_halving(argv=None):
+    ap = sweep_parser("Successive halving over one RL-Rust bin run on the B200 engine: every grid point trains for "
+                      "min_episodes, the best 1/eta go on for eta times as many, and so on up to n_episodes")
+    ap.add_argument("--min_episodes", type=int, required=True, help="the first rung's budget in episodes")
+    ap.add_argument("--eta", type=int, default=3, help="keep the best 1/eta of the sets after each rung; budgets grow eta-fold")
+    env_name, grid, outp, kw = parse_sweep_args(ap, argv)
+    res = run_halving(env_name, grid, **kw)
+    write_json(res, outp)
+    return res

@@ -1,7 +1,8 @@
 """Snapshot / resume of an engine at an episode boundary ("next" row N3; the reference has no checkpointing at all).
 The complete state is: Q tables, UCB counts, and per agent the RNG word index, epsilon, UCB t and Double flag
 (rlb_download_tables / rlb_get_agent_states), plus the Dyna model when one is attached (rlb_download_model) and the
-per-agent hyper-parameter sets when they are installed (rlb_engine_set_hparams).  Stored as one .npz; the configuration
+per-agent hyper-parameter sets when they are installed (rlb_engine_set_hparams), with the active-set mask while some
+set is paused (rlb_engine_set_active_sets).  Stored as one .npz; the configuration
 is stored beside it and checked."""
 import ctypes as C
 
@@ -20,6 +21,8 @@ def save_snapshot(engine, path):
         extra["model_len"], extra["model"] = engine.download_model()
     if engine.hparams is not None:
         extra["hp_sets"], extra["hp_group"] = engine.hparams
+        if engine.active_sets is not None:
+            extra["hp_active"] = np.asarray(engine.active_sets, np.uint8)
     q, counts = engine.download_tables()
     cfg = {k: int(getattr(engine.cfg, k)) for k in _CFG_FIELDS}
     np.savez_compressed(path, q=q, counts=counts, states=engine.states(), selector_kind=np.int64(engine.cfg.selector_kind),
@@ -37,6 +40,8 @@ def load_snapshot(engine, path):
     # the sets before the tables and states: installing them refills both with each agent's constructor values
     if "hp_sets" in z.files:
         engine.set_hparams(z["hp_sets"], z["hp_group"])
+        if "hp_active" in z.files:
+            engine.set_active_sets(z["hp_active"])
     elif engine.G:
         engine.set_hparams(None, None)
     has_counts = int(z["selector_kind"]) == 1

@@ -252,7 +252,8 @@ typedef struct rlb_hparams {
  * rlb_comm_gather_episode_sums(.., n_episodes * n_sets, ..).
  * RLB_ERR_INVALID_ARG, the engine untouched: n_sets == 0 with a non-NULL pointer, n_sets > 0 with a NULL one,
  * n_sets > RLB_MAX_HPARAM_SETS, any group[i] >= n_sets.  Values are not checked.  RLB_ERR_UNSUPPORTED: a Dyna model
- * (rlb_agent_set_model / rlb_config.planning_steps) together with sets, whichever comes second. */
+ * (rlb_agent_set_model / rlb_config.planning_steps) together with sets, whichever comes second (per-set planning counts
+ * attach one: rlb_engine_set_planning_steps), and uninstalling the sets while such counts are in force. */
 rlb_status rlb_engine_set_hparams(rlb_engine* e, const rlb_hparams* sets, uint32_t n_sets, const uint32_t* group);
 uint32_t rlb_engine_hparam_sets(const rlb_engine* e);    /* 0 while rlb_config's values apply */
 /* Replace the values of the installed hyper-parameter sets without reconstructing any agent (the explore step of
@@ -287,6 +288,27 @@ rlb_status rlb_engine_retune_hparams(rlb_engine* e, const rlb_hparams* sets, uin
  * RLB_ERR_INVALID_ARG, the engine untouched: no sets installed, n_sets != rlb_engine_hparam_sets(e), or a NULL /
  * non-NULL mismatch between active and n_sets. */
 rlb_status rlb_engine_set_active_sets(rlb_engine* e, const uint8_t* active, uint32_t n_sets);
+/* Dyna-Q under hyper-parameter sets: a planning count per set (no reference equivalent; rlb_hparams' layout is ABI, so
+ * the count is kept beside it).  steps [n_sets] u32, host or device: the agents of set g are
+ * InternalModelAgent::new(agent, RandomModel::default(), steps[g]) (agent/internal_model_agent.rs:17-29), i.e. they make
+ * steps[g] planning replays per real update.  The sets-aware way to attach a model: rlb_agent_set_model(k > 0) after
+ * rlb_engine_set_hparams, and rlb_engine_set_hparams(n_sets > 0) with a model attached, still return RLB_ERR_UNSUPPORTED.
+ * The first call on an engine without a model wraps every agent as it is (tables, epsilon, counts, flag and RNG stay; the
+ * model starts empty), as rlb_agent_set_model does; it needs the HBM store and re-picks the store.  A later call changes
+ * only the counts, models, tables and states left as they are: every later call then gives the bits of an engine B with
+ * the same rlb_config and rlb_engine_set_hparams, given this engine's tables, agent states and model (rlb_upload_tables,
+ * rlb_set_agent_states, rlb_upload_model) and then the same counts.  A count of 0 is allowed: those agents train as
+ * the plain agent does (tables, states, records and sums), while their model still records every first-seen
+ * transition.  rlb_model_capacity stays nonzero while the model is attached, every count 0 included.
+ * steps = NULL, n_sets = 0: drop the model and the counts (as rlb_agent_set_model(e, 0), which does the same).
+ * The counts are kept by rlb_agent_set_kind (which re-wraps around an empty model), rlb_agent_reset (which empties the
+ * model), rlb_engine_retune_hparams and rlb_agent_clone (the destination keeps its set, so its count); the active-set
+ * mask applies to the model launches as to every train launch.  Uninstalling the sets (rlb_engine_set_hparams(e, NULL,
+ * 0, NULL)) while counts are in force returns RLB_ERR_UNSUPPORTED.
+ * RLB_ERR_INVALID_ARG, the engine untouched: no sets installed, n_sets != rlb_engine_hparam_sets(e), or a NULL /
+ * non-NULL mismatch between steps and n_sets.  RLB_ERR_UNSUPPORTED: store_kind names a store other than HBM.  Values
+ * are not checked. */
+rlb_status rlb_engine_set_planning_steps(rlb_engine* e, const uint32_t* steps, uint32_t n_sets);
 
 /* ---- Env<T,COUNT> (env.rs:19-49), batched ------------------------------------------------ */
 /* Env::reset (blackjack.rs:105, frozen_lake.rs:106, cliff_walking.rs:67, taxi.rs:135).  obs_out [N] u32 */

@@ -83,7 +83,7 @@ EXPORTS = [
     "rlb_comm_unique_id", "rlb_comm_init_rank", "rlb_comm_init_all", "rlb_comm_destroy", "rlb_comm_rank", "rlb_comm_world_size",
     "rlb_comm_gather_episode_sums", "rlb_comm_allreduce_sum", "rlb_comm_group_begin", "rlb_comm_group_end",
     "rlb_selftest_ucb_math", "rlb_engine_set_hparams", "rlb_engine_hparam_sets", "rlb_engine_retune_hparams", "rlb_agent_clone",
-    "rlb_engine_set_active_sets",
+    "rlb_engine_set_active_sets", "rlb_engine_set_planning_steps",
 ]
 
 
@@ -123,6 +123,7 @@ def _load():
     L.rlb_engine_retune_hparams.argtypes = [vp, vp, u32]
     L.rlb_agent_clone.argtypes = [vp, vp, vp, u64]
     L.rlb_engine_set_active_sets.argtypes = [vp, vp, u32]
+    L.rlb_engine_set_planning_steps.argtypes = [vp, vp, u32]
     L.rlb_env_reset.argtypes = [vp, vp]
     L.rlb_env_step.argtypes = [vp, vp, vp, vp, vp, vp]
     L.rlb_agent_get_action.argtypes = [vp, vp, vp]
@@ -251,6 +252,7 @@ class Engine:
         self.G = 0                  # hyper-parameter sets installed (set_hparams); per-episode sums are (E, G, 4) while G > 0
         self.hparams = None         # (sets, group) as installed
         self.active_sets = None     # bool (G,) while some set is paused (set_active_sets), else None
+        self.planning = None        # uint32 (G,) per-set Dyna planning counts (set_planning_steps), else None
 
     def close(self):
         if getattr(self, "h", None):
@@ -300,7 +302,7 @@ class Engine:
         While sets are installed, train() and evaluate() return per-episode sums shaped (E, G, 4)."""
         if sets is None and group is None:
             check(lib.rlb_engine_set_hparams(self.h, None, 0, None))
-            self.G, self.hparams, self.active_sets = 0, None, None
+            self.G, self.hparams, self.active_sets, self.planning = 0, None, None, None
             return
         arr = self.hparams_array(sets)
         grp = np.asarray(group)
@@ -310,7 +312,7 @@ class Engine:
             raise ValueError("group ids must be in [0, 2**32)")
         grp = np.ascontiguousarray(grp, np.uint32)
         check(lib.rlb_engine_set_hparams(self.h, ptr(arr) if len(arr) else None, len(arr), ptr(grp) if len(arr) else None))
-        self.G, self.hparams, self.active_sets = len(arr), (arr.copy(), grp.copy()), None
+        self.G, self.hparams, self.active_sets, self.planning = len(arr), (arr.copy(), grp.copy()), None, None
 
     def hparam_sets(self):
         """rlb_engine_hparam_sets: the number of sets installed, 0 while the configured values apply."""
@@ -339,6 +341,24 @@ class Engine:
         m = np.ascontiguousarray(m != 0, np.uint8)
         check(lib.rlb_engine_set_active_sets(self.h, ptr(m) if len(m) else None, len(m)))
         self.active_sets = None if m.all() else m.astype(bool)
+
+    def set_planning_steps(self, steps):
+        """rlb_engine_set_planning_steps: the agents of set g become Dyna-Q agents making steps[g] planning replays per real
+        update ((G,) non-negative integers; 0 allowed).  The first call wraps every agent as it is around an empty model; a
+        later one changes only the counts.  steps=None drops the model (as set_model(0)).  `planning` then holds the
+        counts, or None (see include/rlb.h)."""
+        if steps is None:
+            check(lib.rlb_engine_set_planning_steps(self.h, None, 0))
+            self.cfg.planning_steps, self.planning = 0, None
+            return
+        k = np.asarray(steps)
+        if k.shape != (self.G,):
+            raise ValueError("steps must have shape (%d,), got %r" % (self.G, k.shape))
+        if k.size and (k.dtype.kind not in "iu" or k.min() < 0 or k.max() >= 2 ** 32):
+            raise ValueError("planning steps must be integers in [0, 2**32)")
+        k = np.ascontiguousarray(k, np.uint32)
+        check(lib.rlb_engine_set_planning_steps(self.h, ptr(k) if len(k) else None, len(k)))
+        self.cfg.planning_steps, self.planning = max(1, int(k.max())), k.copy()
 
     # ---- population-based training: the exploit step
     def clone_agents(self, src, dst):
@@ -455,6 +475,8 @@ class Engine:
     def set_model(self, planning_steps):
         check(lib.rlb_agent_set_model(self.h, planning_steps))
         self.cfg.planning_steps = planning_steps
+        if not planning_steps:
+            self.planning = None
 
     def model_add_info(self, obs, action, reward, next_obs):
         obs, action, next_obs = (np.ascontiguousarray(x, np.uint32) for x in (obs, action, next_obs))

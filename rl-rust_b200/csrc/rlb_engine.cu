@@ -5,6 +5,7 @@
 // index, epsilon, UCB t, Double flag, env state) as SoA arrays, the env transition tables,
 // and a scratch ring for the per-episode record stream that k_run writes and
 // k_episode_sums reduces.  There is no CPU path: every compute entry point needs a device.
+#include <algorithm>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -102,6 +103,9 @@ struct rlb_engine {
     uint32_t* d_hp_run = nullptr;      // [hp_n_run] d_hp_order restricted to the active sets: k_run_hp's agent list and the reduction's order
     uint32_t* d_hp_run_offsets = nullptr;   // [hp_n + 1] where each set starts in d_hp_run (an inactive set has length 0)
     uint64_t hp_n_run = 0;
+    // per-set Dyna planning counts (rlb_engine_set_planning_steps); empty while no per-set model is attached
+    std::vector<uint32_t> h_hp_planning;   // [hp_n]
+    uint32_t* d_hp_planning = nullptr;     // [hp_n] device copy: HpParams::planning
     // Calls whose work is enqueued but not yet waited for (rlb_agent_train_range_async): at most two, so that the
     // kernels of call i + 1 are in the queue before the host blocks on the copies of call i.
     struct Pending {
@@ -201,6 +205,16 @@ cudaError_t fill_eps_initial(rlb_engine* e) {
 }
 
 cudaError_t dispatch_run(rlb_engine* e, const DevParams& p) {
+    const bool masked = !e->hp_active.empty();   // only the active sets' agents run: a launch sized to them
+    const HpParams sets{e->d_hp_sets, e->d_hp_group, masked ? e->d_hp_run : nullptr, masked ? e->hp_n_run : e->cfg.n_agents, e->d_hp_planning};
+    if (p.planning_steps && p.mode == 0 && e->hp_n) {   // the model under sets: each set's own planning count
+        switch (e->cfg.env_kind) {
+            case RLB_ENV_BLACKJACK: return launch_run_model<RLB_ENV_BLACKJACK, true>(e->variant, p, e->stream, sets);
+            case RLB_ENV_FROZEN_LAKE: return launch_run_model<RLB_ENV_FROZEN_LAKE, true>(e->variant, p, e->stream, sets);
+            case RLB_ENV_CLIFF_WALKING: return launch_run_model<RLB_ENV_CLIFF_WALKING, true>(e->variant, p, e->stream, sets);
+            default: return launch_run_model<RLB_ENV_TAXI, true>(e->variant, p, e->stream, sets);
+        }
+    }
     if (p.planning_steps && p.mode == 0) {   // InternalModelAgent::update on the training path; evaluate never touches the model
         switch (e->cfg.env_kind) {
             case RLB_ENV_BLACKJACK: return launch_run_model<RLB_ENV_BLACKJACK>(e->variant, p, e->stream);
@@ -209,9 +223,7 @@ cudaError_t dispatch_run(rlb_engine* e, const DevParams& p) {
             default: return launch_run_model<RLB_ENV_TAXI>(e->variant, p, e->stream);
         }
     }
-    if (e->hp_n) {   // every agent with its own hyper-parameter set (never with a model: rlb_engine_set_hparams)
-        const bool masked = !e->hp_active.empty();   // only the active sets' agents run: a launch sized to them
-        const HpParams sets{e->d_hp_sets, e->d_hp_group, masked ? e->d_hp_run : nullptr, masked ? e->hp_n_run : e->cfg.n_agents};
+    if (e->hp_n) {   // every agent with its own hyper-parameter set (with a model: evaluate, which never touches it)
         switch (e->cfg.env_kind) {
             case RLB_ENV_BLACKJACK: return launch_run<RLB_ENV_BLACKJACK, true>(e->variant, p, e->store, e->stream, sets);
             case RLB_ENV_FROZEN_LAKE: return launch_run<RLB_ENV_FROZEN_LAKE, true>(e->variant, p, e->store, e->stream, sets);
@@ -305,7 +317,7 @@ rlb_status pick_store(rlb_engine* e) {
 cudaError_t dispatch_step(rlb_engine* e, StepOp op, const StepArgs& a) {
     if (e->hp_n) {
         StepArgs with_sets = a;
-        with_sets.sets = HpParams{e->d_hp_sets, e->d_hp_group};
+        with_sets.sets = HpParams{e->d_hp_sets, e->d_hp_group, nullptr, 0, e->d_hp_planning};
         switch (e->cfg.env_kind) {
             case RLB_ENV_BLACKJACK: return launch_step<RLB_ENV_BLACKJACK, true>(op, e->variant, e->dp, with_sets, e->stream);
             case RLB_ENV_FROZEN_LAKE: return launch_step<RLB_ENV_FROZEN_LAKE, true>(op, e->variant, e->dp, with_sets, e->stream);
@@ -353,15 +365,18 @@ rlb_status ensure_trace_buffers(rlb_engine* e) {
     return RLB_OK;
 }
 
-// InternalModelAgent::new(agent, RandomModel::default(), planning_steps) / unwrap when planning_steps == 0
+// InternalModelAgent::new(agent, RandomModel::default(), planning_steps) / unwrap when planning_steps == 0 (which also
+// drops the per-set planning counts)
 rlb_status attach_model(rlb_engine* e, uint32_t planning_steps) {
     const uint64_t N = e->cfg.n_agents;
     e->cfg.planning_steps = planning_steps;
     e->dp.planning_steps = planning_steps;
     if (!planning_steps) {
-        void* bufs[] = {e->d_model_ent, e->d_model_bits, e->d_model_len};
+        void* bufs[] = {e->d_model_ent, e->d_model_bits, e->d_model_len, e->d_hp_planning};
         CK(cudaStreamSynchronize(e->stream));
         for (void* b : bufs) if (b) cudaFree(b);
+        e->d_hp_planning = nullptr;
+        e->h_hp_planning.clear();
         e->d_model_ent = nullptr; e->d_model_bits = nullptr; e->d_model_len = nullptr;
         e->dp.model_ent = nullptr; e->dp.model_bits = nullptr; e->dp.model_len = nullptr; e->dp.mcap = 0; e->dp.mwords = 0;
         return RLB_OK;
@@ -826,7 +841,7 @@ void rlb_engine_destroy(rlb_engine* e) {
     void* bufs[] = {e->d_q, e->d_counts, e->d_etr, e->d_etr_il, e->d_vis, e->d_nvis, e->d_rng_n, e->d_eps, e->d_ucb_t, e->d_flag, e->d_env,
                     e->d_trans, e->d_thr, e->d_thr_state, e->d_totals, e->d_flagword, e->d_episodes, e->d_sums,
                     e->d_model_ent, e->d_model_bits, e->d_model_len, e->d_hp_sets, e->d_hp_group, e->d_hp_order, e->d_hp_offsets,
-                    e->d_hp_q0, e->d_hp_eps0, e->d_hp_run, e->d_hp_run_offsets};
+                    e->d_hp_q0, e->d_hp_eps0, e->d_hp_run, e->d_hp_run_offsets, e->d_hp_planning};
     for (void* b : bufs) if (b) cudaFree(b);
     for (void* b : e->d_stage) if (b) cudaFree(b);
     if (e->ev0) cudaEventDestroy(e->ev0);
@@ -896,6 +911,9 @@ rlb_status rlb_engine_set_hparams(rlb_engine* e, const rlb_hparams* sets, uint32
         for (uint64_t i = 0; i < N; ++i)
             if (h_group[i] >= n_sets) { set_error("group[%llu] = %u >= n_sets = %u", (unsigned long long)i, h_group[i], n_sets); return RLB_ERR_INVALID_ARG; }
         if (e->cfg.planning_steps) { set_error("per-agent hyper-parameter sets together with a Dyna model are not supported"); return RLB_ERR_UNSUPPORTED; }
+    } else if (!e->h_hp_planning.empty()) {
+        set_error("the per-set planning counts need the sets: drop the model first (rlb_engine_set_planning_steps(e, NULL, 0))");
+        return RLB_ERR_UNSUPPORTED;
     }
     // release the old sets (the kernels that read them have completed: ENTER waited for pending calls, and the stream
     // is drained before the buffers go)
@@ -982,6 +1000,42 @@ rlb_status rlb_engine_set_active_sets(rlb_engine* e, const uint8_t* active, uint
     e->hp_n_run = run.size();
     e->hp_active = std::move(mask);
     return RLB_OK;
+}
+
+rlb_status rlb_engine_set_planning_steps(rlb_engine* e, const uint32_t* steps, uint32_t n_sets) {
+    if (!e) { set_error("engine is NULL"); return RLB_ERR_INVALID_ARG; }
+    if (!e->hp_n) { set_error("no hyper-parameter sets are installed (rlb_engine_set_hparams)"); return RLB_ERR_INVALID_ARG; }
+    if ((n_sets == 0) != (steps == nullptr)) { set_error("steps and n_sets: NULL with 0, or rlb_engine_hparam_sets() counts"); return RLB_ERR_INVALID_ARG; }
+    if (steps && n_sets != e->hp_n) { set_error("n_sets = %u, but %u sets are installed", n_sets, e->hp_n); return RLB_ERR_INVALID_ARG; }
+    if (steps && e->cfg.store_kind != 0 && e->cfg.store_kind != STORE_GLOBAL) {
+        set_error("a Dyna model (planning_steps > 0) needs the HBM store");
+        return RLB_ERR_UNSUPPORTED;
+    }
+    ENTER(e);
+    if (!steps) {   // unwrap: rlb_agent_set_model(e, 0)
+        rlb_status st = attach_model(e, 0);
+        if (st != RLB_OK) return st;
+        return pick_store(e);
+    }
+    std::vector<uint32_t> h(n_sets);
+    CK(cudaMemcpy(h.data(), steps, (size_t)n_sets * sizeof(uint32_t), is_device_ptr(steps) ? cudaMemcpyDeviceToHost : cudaMemcpyHostToHost));
+    // DevParams::planning_steps stays nonzero while the model is attached, every count 0 included: it is what tells the
+    // dispatch and the step kernels that a model is there, and what rlb_agent_set_kind wraps the new agent with
+    const uint32_t wrap = std::max<uint32_t>(1u, *std::max_element(h.begin(), h.end()));
+    const bool first = !e->cfg.planning_steps;
+    if (first) {   // every agent wrapped as it is, around an empty model
+        rlb_status st = attach_model(e, wrap);
+        if (st != RLB_OK) return st;
+    } else {       // a model is attached: only the counts change
+        e->cfg.planning_steps = wrap;
+        e->dp.planning_steps = wrap;
+    }
+    if (!e->d_hp_planning) CK(cudaMalloc(&e->d_hp_planning, (size_t)n_sets * sizeof(uint32_t)));
+    // the kernels that read the old counts have completed (ENTER): the new ones go over them in stream order
+    CK(cudaMemcpyAsync(e->d_hp_planning, h.data(), (size_t)n_sets * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
+    CK(cudaStreamSynchronize(e->stream));
+    e->h_hp_planning = std::move(h);
+    return first ? pick_store(e) : RLB_OK;
 }
 
 rlb_status rlb_agent_clone(rlb_engine* e, const uint32_t* src, const uint32_t* dst, uint64_t n_pairs) {
@@ -1222,7 +1276,7 @@ rlb_status rlb_agent_set_model(rlb_engine* e, uint32_t planning_steps) {
         return RLB_ERR_UNSUPPORTED;
     }
     if (planning_steps && e->hp_n) {
-        set_error("a Dyna model together with per-agent hyper-parameter sets is not supported");
+        set_error("a Dyna model together with per-agent hyper-parameter sets: use rlb_engine_set_planning_steps");
         return RLB_ERR_UNSUPPORTED;
     }
     rlb_status st = attach_model(e, planning_steps);

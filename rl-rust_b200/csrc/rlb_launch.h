@@ -44,8 +44,10 @@ enum StepOp {
 // HP = true: the agents run with their own hyper-parameter sets `h` (k_run_hp); instantiated in rlb_inst_<env>_hp.cu
 template <int ENV, bool HP = false> cudaError_t launch_run(const Variant& v, const DevParams& p, int store, cudaStream_t stream,
                                                           const HpParams& h = HpParams{});
-// the same with the Dyna model attached (InternalModelAgent): HBM store only; instantiated in rlb_inst_<env>_model.cu
-template <int ENV> cudaError_t launch_run_model(const Variant& v, const DevParams& p, cudaStream_t stream);
+// the same with the Dyna model attached (InternalModelAgent): HBM store only; instantiated in rlb_inst_<env>_model.cu, and
+// with HP = true (k_run_hp, per-set planning counts h.planning) in rlb_inst_<env>_model_hp.cu
+template <int ENV, bool HP = false> cudaError_t launch_run_model(const Variant& v, const DevParams& p, cudaStream_t stream,
+                                                                const HpParams& h = HpParams{});
 // bytes of dynamic shared memory one 1-warp CTA of the shared-memory / hybrid store needs (0: env not compiled for it)
 template <int ENV> size_t smem_store_bytes(const Variant& v, int store, uint32_t rows, uint32_t S, uint32_t vmax);   // rows: table rows kept on chip
 template <int ENV, bool HP = false> cudaError_t launch_step(StepOp op, const Variant& v, const DevParams& p, const StepArgs& a, cudaStream_t stream);

@@ -151,11 +151,18 @@ cudaError_t launch_run(const Variant& v, const DevParams& p, int store, cudaStre
     return cudaGetLastError();
 }
 
-template <int ENV>
-cudaError_t launch_run_model(const Variant& v, const DevParams& p, cudaStream_t stream) {
-    const unsigned grid = grid_for(p.n_agents);
+template <int ENV, bool HP>
+cudaError_t launch_run_model(const Variant& v, const DevParams& p, cudaStream_t stream, const HpParams& h) {
+    // as launch_run: with per-agent sets the grid covers the launch positions of h (the active sets' agents)
+    const uint64_t n = HP ? h.n_launch : p.n_agents;
+    if (n == 0) return cudaSuccess;
+    const unsigned grid = grid_for(n);
     const size_t smem = EnvTab<ENV>::smem_bytes(p.S);
-#define RLB_CALL(R, P, SL, T) k_run<ENV, R, P, SL, T, STORE_GLOBAL, true><<<grid, kBlock, smem, stream>>>(p)
+#define RLB_CALL(R, P, SL, T)                                                                                          \
+    {                                                                                                                  \
+        if constexpr (HP) k_run_hp<ENV, R, P, SL, T, STORE_GLOBAL, true><<<grid, kBlock, smem, stream>>>(p, h);        \
+        else k_run<ENV, R, P, SL, T, STORE_GLOBAL, true><<<grid, kBlock, smem, stream>>>(p);                           \
+    }
     RLB_VARIANT_SWITCH(v, RLB_CALL)
 #undef RLB_CALL
     return cudaGetLastError();
@@ -269,6 +276,8 @@ cudaError_t launch_step(StepOp op, const Variant& v, const DevParams& p, const S
     template cudaError_t launch_step<ENV, true>(StepOp, const Variant&, const DevParams&, const StepArgs&, cudaStream_t); \
     template cudaError_t run_kernel_attributes<ENV, true>(const Variant&, int, cudaFuncAttributes*);
 
-#define RLB_INSTANTIATE_ENV_MODEL(ENV) template cudaError_t launch_run_model<ENV>(const Variant&, const DevParams&, cudaStream_t);
+#define RLB_INSTANTIATE_ENV_MODEL(ENV) template cudaError_t launch_run_model<ENV, false>(const Variant&, const DevParams&, cudaStream_t, const HpParams&);
+// the same with per-agent hyper-parameter sets and per-set planning counts (k_run_hp with the model); rlb_inst_<env>_model_hp.cu
+#define RLB_INSTANTIATE_ENV_MODEL_HP(ENV) template cudaError_t launch_run_model<ENV, true>(const Variant&, const DevParams&, cudaStream_t, const HpParams&);
 
 }   // namespace rlb

@@ -318,14 +318,27 @@ SWEEP_FLAGS = ("learning_rate", "discount_factor", "lambda_factor", "initial_eps
 AGENT_NAMES = {"onestep": abi.AGENT_ONE_STEP, "traces": abi.AGENT_TRACES}
 SELECTOR_NAMES = {"eps": abi.SEL_EPS_GREEDY, "ucb": abi.SEL_UCB}
 TARGET_KINDS = {"sarsa": abi.TARGET_SARSA, "qlearning": abi.TARGET_QLEARNING, "expected_sarsa": abi.TARGET_EXPECTED_SARSA}
+# Dyna-Q's planning replays per real update (InternalModelAgent::new's third argument, bin/cliffwalking_model.rs): an
+# integer axis of its own, kept beside rlb_hparams (rlb_engine_set_planning_steps); 0 is the plain agent
+PLANNING_AXIS = "planning_steps"
+
+
+def planning_value(v):
+    """A planning-steps grid value as an int; anything but a non-negative integer is a ValueError."""
+    if isinstance(v, (bool, np.bool_)) or not isinstance(v, (int, np.integer)) or v < 0:
+        raise ValueError("planning_steps values must be non-negative integers, got %r" % (v,))
+    return int(v)
 
 
 def expand_grid(grid):
     """{flag: [values]} -> the cartesian product as a list of {flag: value}, the first flag varying slowest."""
     import itertools
+    grid = dict(grid)
     for k in grid:
-        if k not in SWEEP_FLAGS:
-            raise ValueError("%r cannot be swept; the agent constructor flags are %s" % (k, ", ".join(SWEEP_FLAGS)))
+        if k == PLANNING_AXIS:
+            grid[k] = [planning_value(v) for v in grid[k]]
+        elif k not in SWEEP_FLAGS:
+            raise ValueError("%r cannot be swept; the agent constructor flags are %s, and %s" % (k, ", ".join(SWEEP_FLAGS), PLANNING_AXIS))
     keys = list(grid)
     return [dict(zip(keys, vals)) for vals in itertools.product(*(grid[k] for k in keys))]
 
@@ -340,7 +353,8 @@ def point_hparams(flags, n_episodes):
 def grid_engine(env_name, grid, *, agent, selector, target, policy, agents_per_point, seed, real, device, **flags):
     """The grid as one engine: every point of the cartesian grid of `grid` a set, its agents a contiguous group of
     `agents_per_point` constructed with the point's values (rlb_engine_set_hparams).  Returns (engine, n_episodes,
-    moving-average window, points, every point's flags, every point's rlb_hparams)."""
+    moving-average window, points, every point's flags, every point's rlb_hparams).  With a planning_steps axis every set
+    is also a Dyna-Q agent with its point's planning count (rlb_engine_set_planning_steps)."""
     f = dict(DEFAULTS)
     f.update(flags)
     n = int(f["n_episodes"])
@@ -361,6 +375,8 @@ def grid_engine(env_name, grid, *, agent, selector, target, policy, agents_per_p
                      **sets[0], **env._cfg())
     try:
         eng.set_hparams(sets, np.repeat(np.arange(len(points), dtype=np.uint32), int(agents_per_point)))
+        if PLANNING_AXIS in grid:
+            eng.set_planning_steps(np.array([pf[PLANNING_AXIS] for pf in point_flags], np.uint32))
     except BaseException:
         eng.close()
         raise
@@ -421,9 +437,11 @@ def sweep_parser(description):
     ap = argparse.ArgumentParser(description=description)
     ap.add_argument("env", choices=["blackjack", "frozen_lake", "cliffwalking", "taxi"])
     ap.add_argument("--grid", action="append", default=[], metavar="FLAG=V1,V2,...",
-                    help="a bin flag and its values (repeatable; one of %s)" % ", ".join(SWEEP_FLAGS))
+                    help="a bin flag and its values (repeatable; one of %s, %s)" % (", ".join(SWEEP_FLAGS), PLANNING_AXIS))
     for name in SWEEP_FLAGS:
         ap.add_argument("--" + name, default=None, metavar="V1,V2,...", help="values of this flag (a comma list: a grid axis)")
+    ap.add_argument("--" + PLANNING_AXIS, default=None, metavar="K1,K2,...",
+                    help="Dyna-Q planning replays per update (non-negative integers: a grid axis; 0 is the plain agent)")
     ap.add_argument("--n_episodes", "-n", type=int, default=DEFAULTS["n_episodes"])
     for name in ("max_steps", "moving_average_window"):
         ap.add_argument("--" + name, type=int, default=DEFAULTS[name])
@@ -444,17 +462,30 @@ def sweep_parser(description):
 def parse_sweep_args(ap, argv):
     """(env name, grid, output path, the other flags as keyword arguments)"""
     a = vars(ap.parse_args(argv))
+
+    def planning_list(text):
+        try:
+            return [planning_value(int(x)) for x in text.split(",") if x.strip()]
+        except ValueError:
+            ap.error("--%s takes non-negative integers, got %r" % (PLANNING_AXIS, text))
+
     grid = {}
     for name in SWEEP_FLAGS:
         v = a.pop(name)
         if v is not None:
             grid[name] = parse_list(v)
+    v = a.pop(PLANNING_AXIS)
+    if v is not None:
+        grid[PLANNING_AXIS] = planning_list(v)
     for item in a.pop("grid"):
         if "=" not in item:
             ap.error("--grid takes FLAG=V1,V2,...")
         k, v = item.split("=", 1)
+        if k == PLANNING_AXIS:
+            grid[k] = planning_list(v)
+            continue
         if k not in SWEEP_FLAGS:
-            ap.error("--grid %s: not a sweepable flag (%s)" % (k, ", ".join(SWEEP_FLAGS)))
+            ap.error("--grid %s: not a sweepable flag (%s, %s)" % (k, ", ".join(SWEEP_FLAGS), PLANNING_AXIS))
         grid[k] = parse_list(v)
     if not grid:
         ap.error("nothing to sweep: give at least one --grid FLAG=V1,V2,...")
@@ -495,12 +526,26 @@ def pbt_exploit(chunk_sums, fraction, rng):
     return [(loser, top[int(rng.integers(k))]) for loser in bottom]
 
 
+def pbt_perturb_planning(k, f):
+    """A planning count perturbed by the factor f (0.8 or 1.2) as an integer in [0, inf): round(k * f), and where that
+    leaves k as it is, k + 1 for f > 1 and max(0, k - 1) for f < 1."""
+    out = int(round(k * f))
+    if out == k:
+        out = k + 1 if f > 1.0 else max(0, k - 1)
+    return out
+
+
 def pbt_explore(flags, axes, rng):
-    """The winner's flags with every grid axis multiplied by 0.8 or 1.2 at random and clamped into its range."""
+    """The winner's flags with every grid axis multiplied by 0.8 or 1.2 at random and clamped into its range (the
+    planning count as an integer: pbt_perturb_planning)."""
     out = dict(flags)
     for k in axes:
+        f = PBT_FACTORS[int(rng.integers(2))]
+        if k == PLANNING_AXIS:
+            out[k] = pbt_perturb_planning(int(flags[k]), f)
+            continue
         lo, hi = PBT_BOUNDS[k]
-        out[k] = float(min(max(flags[k] * PBT_FACTORS[int(rng.integers(2))], lo), hi))
+        out[k] = float(min(max(flags[k] * f, lo), hi))
     return out
 
 
@@ -518,6 +563,8 @@ def run_pbt(env_name, grid, *, interval, fraction=0.25, pbt_seed=0x9B7, agent="o
     interval = int(interval)
     if interval < 1:
         raise ValueError("interval must be >= 1")
+    if PLANNING_AXIS in grid and agent == "traces":
+        raise ValueError("PBT with a planning_steps axis clones Dyna agents, and cloning a trace agent under a model is not supported")
     axes = list(grid)
     per = int(agents_per_point)
     eng, n, window, points, cur, sets = grid_engine(env_name, grid, agent=agent, selector=selector, target=target, policy=policy,
@@ -543,6 +590,8 @@ def run_pbt(env_name, grid, *, interval, fraction=0.25, pbt_seed=0x9B7, agent="o
                 j = np.arange(per, dtype=np.int64)
                 eng.clone_agents(np.concatenate([w * per + j for _, w in pairs]), np.concatenate([l * per + j for l, _ in pairs]))
                 eng.retune_hparams(sets)
+                if PLANNING_AXIS in axes:
+                    eng.set_planning_steps(np.array([c[PLANNING_AXIS] for c in cur], np.uint32))
             lineage.append(dict(episode=end, pairs=step))
         ev = eng.evaluate(n, sums=True)["sums"]                                                      # [n, G, 4]
         dt = time.perf_counter() - t0

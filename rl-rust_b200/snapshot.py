@@ -2,7 +2,8 @@
 The complete state is: Q tables, UCB counts, and per agent the RNG word index, epsilon, UCB t and Double flag
 (rlb_download_tables / rlb_get_agent_states), plus the Dyna model when one is attached (rlb_download_model) and the
 per-agent hyper-parameter sets when they are installed (rlb_engine_set_hparams), with the active-set mask while some
-set is paused (rlb_engine_set_active_sets).  Stored as one .npz; the configuration
+set is paused (rlb_engine_set_active_sets) and the per-set planning counts while they are in force
+(rlb_engine_set_planning_steps).  Stored as one .npz; the configuration
 is stored beside it and checked."""
 import ctypes as C
 
@@ -19,6 +20,8 @@ def save_snapshot(engine, path):
     extra = {}
     if planning:
         extra["model_len"], extra["model"] = engine.download_model()
+        if engine.planning is not None:
+            extra["hp_planning"] = np.asarray(engine.planning, np.uint32)
     if engine.hparams is not None:
         extra["hp_sets"], extra["hp_group"] = engine.hparams
         if engine.active_sets is not None:
@@ -39,16 +42,20 @@ def load_snapshot(engine, path):
         engine.set_selector(int(z["selector_kind"]))
     # the sets before the tables and states: installing them refills both with each agent's constructor values
     if "hp_sets" in z.files:
+        if "hp_planning" in z.files and int(engine.cfg.planning_steps):
+            engine.set_model(0)   # sets are installed without a model; the counts attach it again below
         engine.set_hparams(z["hp_sets"], z["hp_group"])
-        if "hp_active" in z.files:
-            engine.set_active_sets(z["hp_active"])
     elif engine.G:
         engine.set_hparams(None, None)
     has_counts = int(z["selector_kind"]) == 1
     engine.upload_tables(z["q"], z["counts"] if has_counts else None)
     engine.set_states(z["states"])
     planning = int(z["planning_steps"]) if "planning_steps" in z.files else 0
-    if planning != int(engine.cfg.planning_steps):
+    if "hp_planning" in z.files:
+        engine.set_planning_steps(z["hp_planning"])
+    elif planning != int(engine.cfg.planning_steps):
         engine.set_model(planning)
     if planning:
         engine.upload_model(z["model_len"], z["model"])
+    if "hp_active" in z.files:
+        engine.set_active_sets(z["hp_active"])

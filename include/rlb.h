@@ -243,8 +243,8 @@ typedef struct rlb_hparams {
  * the call acts as the constructor of the agents: their tables are refilled with their own default_value, epsilon set to
  * their initial_epsilon, UCB counts and t reset, policy_flag set (as rlb_agent_set_kind does; the env and the RNG
  * stream carry on).  Every later reset (rlb_selector_reset, rlb_policy_reset, rlb_agent_reset, rlb_agent_set_kind,
- * rlb_agent_set_action_selector) and compute call uses each agent's own set; decay_kind, target, agent kind, selector,
- * policy, real type and env stay engine-wide.
+ * rlb_agent_set_action_selector) and compute call uses each agent's own set; decay_kind, agent kind, selector,
+ * policy, real type and env stay engine-wide, and the target too unless rlb_engine_set_targets gives each set its own.
  * While sets are installed every per-episode sums output is [n_episodes][n_sets][4] (rlb_train_out.episode_sums,
  * rlb_agent_evaluate's sums_out): entry (e, g) is the rlb_train_out reduction, in the same order, over the agents of
  * set g in ascending local index — one set of all agents gives the [n_episodes][4] of an engine without sets, and a set
@@ -309,6 +309,23 @@ rlb_status rlb_engine_set_active_sets(rlb_engine* e, const uint8_t* active, uint
  * non-NULL mismatch between steps and n_sets.  RLB_ERR_UNSUPPORTED: store_kind names a store other than HBM.  Values
  * are not checked. */
 rlb_status rlb_engine_set_planning_steps(rlb_engine* e, const uint32_t* steps, uint32_t n_sets);
+/* The bootstrap target per hyper-parameter set (rlb_hparams' layout is ABI, so the target is kept beside it, as the
+ * planning counts are).  targets [n_sets] i32 RLB_TARGET_*, host or device: the agents of set g use targets[g] as
+ * Agent::set_future_q_value_func(targets[g]) would (agent.rs:19-48), in every update: the fused train calls, the
+ * step-level rlb_agent_update and rlb_agent_step, and the Dyna planning replays under rlb_engine_set_planning_steps; for
+ * one-step and eligibility-trace agents in every store.
+ * Equivalence: from this call on every call gives agent i the bits of agent 0 of an engine created with target_kind =
+ * targets[group[i]] and the rest as rlb_engine_set_hparams states it.  Nothing stored per agent changes (tables, epsilon,
+ * UCB state, flag, model, RNG position): a call between chunks equals an engine B given this engine's tables, agent
+ * states and model (rlb_upload_tables, rlb_set_agent_states, rlb_upload_model) and then the same targets.
+ * rlb_engine_set_hparams (installing or uninstalling) sets every set's target to rlb_config.target_kind, and
+ * rlb_agent_set_future_q_value_func(k) keeps its meaning, every agent now uses k: it sets every set's target to k.
+ * rlb_engine_retune_hparams, rlb_engine_set_active_sets, rlb_agent_set_kind, the resets and
+ * rlb_engine_set_planning_steps keep the targets; rlb_agent_clone's destination keeps its set, so its set's target.
+ * RLB_ERR_INVALID_ARG, the engine untouched: no sets installed, n_sets != rlb_engine_hparam_sets(e), targets NULL, or a
+ * value outside RLB_TARGET_SARSA .. RLB_TARGET_EXPECTED_SARSA.  Unlike rlb_hparams the values are checked: an
+ * unknown target would otherwise run as Expected Sarsa. */
+rlb_status rlb_engine_set_targets(rlb_engine* e, const int32_t* targets, uint32_t n_sets);
 
 /* ---- Env<T,COUNT> (env.rs:19-49), batched ------------------------------------------------ */
 /* Env::reset (blackjack.rs:105, frozen_lake.rs:106, cliff_walking.rs:67, taxi.rs:135).  obs_out [N] u32 */

@@ -83,7 +83,7 @@ EXPORTS = [
     "rlb_comm_unique_id", "rlb_comm_init_rank", "rlb_comm_init_all", "rlb_comm_destroy", "rlb_comm_rank", "rlb_comm_world_size",
     "rlb_comm_gather_episode_sums", "rlb_comm_allreduce_sum", "rlb_comm_group_begin", "rlb_comm_group_end",
     "rlb_selftest_ucb_math", "rlb_engine_set_hparams", "rlb_engine_hparam_sets", "rlb_engine_retune_hparams", "rlb_agent_clone",
-    "rlb_engine_set_active_sets", "rlb_engine_set_planning_steps",
+    "rlb_engine_set_active_sets", "rlb_engine_set_planning_steps", "rlb_engine_set_targets",
 ]
 
 
@@ -124,6 +124,7 @@ def _load():
     L.rlb_agent_clone.argtypes = [vp, vp, vp, u64]
     L.rlb_engine_set_active_sets.argtypes = [vp, vp, u32]
     L.rlb_engine_set_planning_steps.argtypes = [vp, vp, u32]
+    L.rlb_engine_set_targets.argtypes = [vp, vp, u32]
     L.rlb_env_reset.argtypes = [vp, vp]
     L.rlb_env_step.argtypes = [vp, vp, vp, vp, vp, vp]
     L.rlb_agent_get_action.argtypes = [vp, vp, vp]
@@ -253,6 +254,7 @@ class Engine:
         self.hparams = None         # (sets, group) as installed
         self.active_sets = None     # bool (G,) while some set is paused (set_active_sets), else None
         self.planning = None        # uint32 (G,) per-set Dyna planning counts (set_planning_steps), else None
+        self.targets = None         # int32 (G,) per-set targets while they differ from cfg.target_kind (set_targets), else None
 
     def close(self):
         if getattr(self, "h", None):
@@ -302,7 +304,7 @@ class Engine:
         While sets are installed, train() and evaluate() return per-episode sums shaped (E, G, 4)."""
         if sets is None and group is None:
             check(lib.rlb_engine_set_hparams(self.h, None, 0, None))
-            self.G, self.hparams, self.active_sets, self.planning = 0, None, None, None
+            self.G, self.hparams, self.active_sets, self.planning, self.targets = 0, None, None, None, None
             return
         arr = self.hparams_array(sets)
         grp = np.asarray(group)
@@ -312,7 +314,7 @@ class Engine:
             raise ValueError("group ids must be in [0, 2**32)")
         grp = np.ascontiguousarray(grp, np.uint32)
         check(lib.rlb_engine_set_hparams(self.h, ptr(arr) if len(arr) else None, len(arr), ptr(grp) if len(arr) else None))
-        self.G, self.hparams, self.active_sets, self.planning = len(arr), (arr.copy(), grp.copy()), None, None
+        self.G, self.hparams, self.active_sets, self.planning, self.targets = len(arr), (arr.copy(), grp.copy()), None, None, None
 
     def hparam_sets(self):
         """rlb_engine_hparam_sets: the number of sets installed, 0 while the configured values apply."""
@@ -359,6 +361,19 @@ class Engine:
         k = np.ascontiguousarray(k, np.uint32)
         check(lib.rlb_engine_set_planning_steps(self.h, ptr(k) if len(k) else None, len(k)))
         self.cfg.planning_steps, self.planning = max(1, int(k.max())), k.copy()
+
+    def set_targets(self, kinds):
+        """rlb_engine_set_targets: the agents of set g bootstrap with target kinds[g] ((G,) TARGET_* integers) in every
+        later update; tables and agent states stay as they are.  `targets` then holds the targets, or None while every
+        set has cfg.target_kind (see include/rlb.h).  set_hparams and set_target put every set back on the engine's."""
+        k = np.asarray(kinds)
+        if k.shape != (self.G,):
+            raise ValueError("targets must have shape (%d,), got %r" % (self.G, k.shape))
+        if k.size and (k.dtype.kind not in "iu" or k.min() < TARGET_SARSA or k.max() > TARGET_EXPECTED_SARSA):
+            raise ValueError("targets must be integers in [%d, %d]" % (TARGET_SARSA, TARGET_EXPECTED_SARSA))
+        k = np.ascontiguousarray(k, np.int32)
+        check(lib.rlb_engine_set_targets(self.h, ptr(k) if len(k) else None, len(k)))
+        self.targets = None if (k == self.cfg.target_kind).all() else k.copy()
 
     # ---- population-based training: the exploit step
     def clone_agents(self, src, dst):
@@ -459,6 +474,7 @@ class Engine:
     def set_target(self, kind):
         check(lib.rlb_agent_set_future_q_value_func(self.h, kind))
         self.cfg.target_kind = kind
+        self.targets = None
 
     def set_selector(self, kind):
         check(lib.rlb_agent_set_action_selector(self.h, kind))

@@ -106,6 +106,9 @@ struct rlb_engine {
     // per-set Dyna planning counts (rlb_engine_set_planning_steps); empty while no per-set model is attached
     std::vector<uint32_t> h_hp_planning;   // [hp_n]
     uint32_t* d_hp_planning = nullptr;     // [hp_n] device copy: HpParams::planning
+    // per-set bootstrap targets (rlb_engine_set_targets); every entry cfg.target_kind until that call
+    std::vector<int32_t> h_hp_targets;     // [hp_n]
+    int32_t* d_hp_targets = nullptr;       // [hp_n] device copy: HpParams::targets
     // Calls whose work is enqueued but not yet waited for (rlb_agent_train_range_async): at most two, so that the
     // kernels of call i + 1 are in the queue before the host blocks on the copies of call i.
     struct Pending {
@@ -206,7 +209,8 @@ cudaError_t fill_eps_initial(rlb_engine* e) {
 
 cudaError_t dispatch_run(rlb_engine* e, const DevParams& p) {
     const bool masked = !e->hp_active.empty();   // only the active sets' agents run: a launch sized to them
-    const HpParams sets{e->d_hp_sets, e->d_hp_group, masked ? e->d_hp_run : nullptr, masked ? e->hp_n_run : e->cfg.n_agents, e->d_hp_planning};
+    const HpParams sets{e->d_hp_sets, e->d_hp_group, masked ? e->d_hp_run : nullptr, masked ? e->hp_n_run : e->cfg.n_agents, e->d_hp_planning,
+                        e->d_hp_targets};
     if (p.planning_steps && p.mode == 0 && e->hp_n) {   // the model under sets: each set's own planning count
         switch (e->cfg.env_kind) {
             case RLB_ENV_BLACKJACK: return launch_run_model<RLB_ENV_BLACKJACK, true>(e->variant, p, e->stream, sets);
@@ -317,7 +321,7 @@ rlb_status pick_store(rlb_engine* e) {
 cudaError_t dispatch_step(rlb_engine* e, StepOp op, const StepArgs& a) {
     if (e->hp_n) {
         StepArgs with_sets = a;
-        with_sets.sets = HpParams{e->d_hp_sets, e->d_hp_group, nullptr, 0, e->d_hp_planning};
+        with_sets.sets = HpParams{e->d_hp_sets, e->d_hp_group, nullptr, 0, e->d_hp_planning, e->d_hp_targets};
         switch (e->cfg.env_kind) {
             case RLB_ENV_BLACKJACK: return launch_step<RLB_ENV_BLACKJACK, true>(op, e->variant, e->dp, with_sets, e->stream);
             case RLB_ENV_FROZEN_LAKE: return launch_step<RLB_ENV_FROZEN_LAKE, true>(op, e->variant, e->dp, with_sets, e->stream);
@@ -841,7 +845,8 @@ void rlb_engine_destroy(rlb_engine* e) {
     void* bufs[] = {e->d_q, e->d_counts, e->d_etr, e->d_etr_il, e->d_vis, e->d_nvis, e->d_rng_n, e->d_eps, e->d_ucb_t, e->d_flag, e->d_env,
                     e->d_trans, e->d_thr, e->d_thr_state, e->d_totals, e->d_flagword, e->d_episodes, e->d_sums,
                     e->d_model_ent, e->d_model_bits, e->d_model_len, e->d_hp_sets, e->d_hp_group, e->d_hp_order, e->d_hp_offsets,
-                    e->d_hp_q0, e->d_hp_eps0, e->d_hp_run, e->d_hp_run_offsets, e->d_hp_planning};
+                    e->d_hp_q0, e->d_hp_eps0, e->d_hp_run, e->d_hp_run_offsets, e->d_hp_planning,
+                    e->d_hp_targets};
     for (void* b : bufs) if (b) cudaFree(b);
     for (void* b : e->d_stage) if (b) cudaFree(b);
     if (e->ev0) cudaEventDestroy(e->ev0);
@@ -918,10 +923,12 @@ rlb_status rlb_engine_set_hparams(rlb_engine* e, const rlb_hparams* sets, uint32
     // release the old sets (the kernels that read them have completed: ENTER waited for pending calls, and the stream
     // is drained before the buffers go)
     CK(cudaStreamSynchronize(e->stream));
-    void* old[] = {e->d_hp_sets, e->d_hp_group, e->d_hp_order, e->d_hp_offsets, e->d_hp_q0, e->d_hp_eps0, e->d_hp_run, e->d_hp_run_offsets};
+    void* old[] = {e->d_hp_sets, e->d_hp_group, e->d_hp_order, e->d_hp_offsets, e->d_hp_q0, e->d_hp_eps0, e->d_hp_run, e->d_hp_run_offsets,
+                   e->d_hp_targets};
     for (void* b : old) if (b) cudaFree(b);
     e->d_hp_sets = nullptr; e->d_hp_group = nullptr; e->d_hp_order = nullptr; e->d_hp_offsets = nullptr;
-    e->d_hp_q0 = nullptr; e->d_hp_eps0 = nullptr;
+    e->d_hp_q0 = nullptr; e->d_hp_eps0 = nullptr; e->d_hp_targets = nullptr;
+    e->h_hp_targets.clear();
     e->d_hp_run = nullptr; e->d_hp_run_offsets = nullptr; e->hp_n_run = 0;
     e->hp_active.clear();   // every set active again
     e->h_hp_order.clear(); e->h_hp_offsets.clear();
@@ -939,11 +946,16 @@ rlb_status rlb_engine_set_hparams(rlb_engine* e, const rlb_hparams* sets, uint32
         CK(cudaMalloc(&e->d_hp_offsets, (size_t)(n_sets + 1) * sizeof(uint32_t)));
         CK(cudaMalloc(&e->d_hp_q0, (size_t)n_sets * e->real_size));
         CK(cudaMalloc(&e->d_hp_eps0, (size_t)n_sets * sizeof(double)));
+        CK(cudaMalloc(&e->d_hp_targets, (size_t)n_sets * sizeof(int32_t)));
         CK(cudaMemcpyAsync(e->d_hp_group, h_group.data(), N * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
         CK(cudaMemcpyAsync(e->d_hp_order, order.data(), N * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
         CK(cudaMemcpyAsync(e->d_hp_offsets, offsets.data(), (size_t)(n_sets + 1) * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
-        CK(write_set_values(e, h_sets));
+        // every set starts with the engine-wide target (rlb_engine_set_targets changes them)
+        std::vector<int32_t> targets(n_sets, e->cfg.target_kind);
+        CK(cudaMemcpyAsync(e->d_hp_targets, targets.data(), (size_t)n_sets * sizeof(int32_t), cudaMemcpyHostToDevice, e->stream));
+        CK(write_set_values(e, h_sets));   // synchronous: `targets` may go
         e->h_hp_order = std::move(order); e->h_hp_offsets = std::move(offsets);
+        e->h_hp_targets = std::move(targets);
         e->hp_n = n_sets;
     }
     // the constructors again, with each agent's own values: fresh tables, policy_flag = true, an empty trace, a fresh
@@ -1036,6 +1048,27 @@ rlb_status rlb_engine_set_planning_steps(rlb_engine* e, const uint32_t* steps, u
     CK(cudaStreamSynchronize(e->stream));
     e->h_hp_planning = std::move(h);
     return first ? pick_store(e) : RLB_OK;
+}
+
+// the device copy of h_hp_targets, after the kernels that read the old one (ENTER waited for pending calls; the copy
+// follows the rest in stream order)
+static rlb_status write_targets(rlb_engine* e) {
+    CK(cudaMemcpyAsync(e->d_hp_targets, e->h_hp_targets.data(), e->h_hp_targets.size() * sizeof(int32_t), cudaMemcpyHostToDevice, e->stream));
+    CK(cudaStreamSynchronize(e->stream));
+    return RLB_OK;
+}
+
+rlb_status rlb_engine_set_targets(rlb_engine* e, const int32_t* targets, uint32_t n_sets) {
+    if (!e) { set_error("engine is NULL"); return RLB_ERR_INVALID_ARG; }
+    if (!e->hp_n) { set_error("no hyper-parameter sets are installed (rlb_engine_set_hparams)"); return RLB_ERR_INVALID_ARG; }
+    if (!targets || n_sets != e->hp_n) { set_error("targets: one RLB_TARGET_* per installed set (%u), got %u", e->hp_n, n_sets); return RLB_ERR_INVALID_ARG; }
+    ENTER(e);
+    std::vector<int32_t> h(n_sets);
+    CK(cudaMemcpy(h.data(), targets, (size_t)n_sets * sizeof(int32_t), is_device_ptr(targets) ? cudaMemcpyDeviceToHost : cudaMemcpyHostToHost));
+    for (uint32_t g = 0; g < n_sets; ++g)
+        if (h[g] < RLB_TARGET_SARSA || h[g] > RLB_TARGET_EXPECTED_SARSA) { set_error("targets[%u] = %d is not an RLB_TARGET_*", g, h[g]); return RLB_ERR_INVALID_ARG; }
+    e->h_hp_targets = std::move(h);
+    return write_targets(e);
 }
 
 rlb_status rlb_agent_clone(rlb_engine* e, const uint32_t* src, const uint32_t* dst, uint64_t n_pairs) {
@@ -1205,6 +1238,12 @@ rlb_status rlb_agent_step(rlb_engine* e, uint8_t* kind_out, uint32_t* obs_out, u
 
 rlb_status rlb_agent_set_future_q_value_func(rlb_engine* e, int32_t target_kind) {
     if (!e || target_kind < 0 || target_kind > 2) { set_error("bad target_kind"); return RLB_ERR_INVALID_ARG; }
+    if (e->hp_n) {   // every agent now uses target_kind: every set's target too
+        ENTER(e);
+        std::fill(e->h_hp_targets.begin(), e->h_hp_targets.end(), target_kind);
+        rlb_status st = write_targets(e);
+        if (st != RLB_OK) return st;
+    }
     e->cfg.target_kind = target_kind;
     e->dp.target = target_kind;
     return RLB_OK;

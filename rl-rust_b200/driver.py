@@ -321,6 +321,9 @@ TARGET_KINDS = {"sarsa": abi.TARGET_SARSA, "qlearning": abi.TARGET_QLEARNING, "e
 # Dyna-Q's planning replays per real update (InternalModelAgent::new's third argument, bin/cliffwalking_model.rs): an
 # integer axis of its own, kept beside rlb_hparams (rlb_engine_set_planning_steps); 0 is the plain agent
 PLANNING_AXIS = "planning_steps"
+# the bootstrap target (Agent::set_future_q_value_func, agent.rs:48) as a categorical axis: names of TARGET_KINDS, kept
+# beside rlb_hparams (rlb_engine_set_targets)
+TARGET_AXIS = "target"
 
 
 def planning_value(v):
@@ -337,8 +340,13 @@ def expand_grid(grid):
     for k in grid:
         if k == PLANNING_AXIS:
             grid[k] = [planning_value(v) for v in grid[k]]
+        elif k == TARGET_AXIS:
+            bad = [v for v in grid[k] if not isinstance(v, str) or v not in TARGET_KINDS]
+            if bad:
+                raise ValueError("target values must be among %s, got %r" % (", ".join(sorted(TARGET_KINDS)), bad))
         elif k not in SWEEP_FLAGS:
-            raise ValueError("%r cannot be swept; the agent constructor flags are %s, and %s" % (k, ", ".join(SWEEP_FLAGS), PLANNING_AXIS))
+            raise ValueError("%r cannot be swept; the agent constructor flags are %s, %s and %s"
+                             % (k, ", ".join(SWEEP_FLAGS), PLANNING_AXIS, TARGET_AXIS))
     keys = list(grid)
     return [dict(zip(keys, vals)) for vals in itertools.product(*(grid[k] for k in keys))]
 
@@ -354,7 +362,8 @@ def grid_engine(env_name, grid, *, agent, selector, target, policy, agents_per_p
     """The grid as one engine: every point of the cartesian grid of `grid` a set, its agents a contiguous group of
     `agents_per_point` constructed with the point's values (rlb_engine_set_hparams).  Returns (engine, n_episodes,
     moving-average window, points, every point's flags, every point's rlb_hparams).  With a planning_steps axis every set
-    is also a Dyna-Q agent with its point's planning count (rlb_engine_set_planning_steps)."""
+    is also a Dyna-Q agent with its point's planning count (rlb_engine_set_planning_steps), and with a target axis every
+    set bootstraps with its point's target (rlb_engine_set_targets); `target` is then only the engine's configured one."""
     f = dict(DEFAULTS)
     f.update(flags)
     n = int(f["n_episodes"])
@@ -377,10 +386,22 @@ def grid_engine(env_name, grid, *, agent, selector, target, policy, agents_per_p
         eng.set_hparams(sets, np.repeat(np.arange(len(points), dtype=np.uint32), int(agents_per_point)))
         if PLANNING_AXIS in grid:
             eng.set_planning_steps(np.array([pf[PLANNING_AXIS] for pf in point_flags], np.uint32))
+        if TARGET_AXIS in grid:
+            eng.set_targets(point_targets(point_flags))
     except BaseException:
         eng.close()
         raise
     return eng, n, window, points, point_flags, sets
+
+
+def point_targets(point_flags):
+    """Every point's target name as the RLB_TARGET_* array rlb_engine_set_targets takes."""
+    return np.array([TARGET_KINDS[pf[TARGET_AXIS]] for pf in point_flags], np.int32)
+
+
+def engine_target(grid, target):
+    """The `target` of a result: the engine-wide name, or None where a target axis gives each point its own."""
+    return None if TARGET_AXIS in grid else target
 
 
 def point_results(points, sets, train_sums, eval_sums, agents_per_point, n, window):
@@ -422,7 +443,7 @@ def run_sweep(env_name, grid, *, agent="onestep", selector="eps", target="qlearn
                                                                                   res["train_steps"] / dt if dt > 0 else 0.0))
         for g in ranking[:10]:
             print("  %-60s evaluate mean return %.4f" % (points[g], out_points[g]["eval_mean_return"]))
-    return dict(env=env_name, agent=agent, selector=selector, target=target, policy=policy, real=real, n_episodes=n,
+    return dict(env=env_name, agent=agent, selector=selector, target=engine_target(grid, target), policy=policy, real=real, n_episodes=n,
                 agents_per_point=int(agents_per_point), grid={k: list(v) for k, v in grid.items()}, points=out_points,
                 ranking=ranking, seconds=dt, train_steps=int(res["train_steps"]))
 
@@ -431,13 +452,17 @@ def parse_list(text):
     return [float(x) for x in text.split(",") if x.strip()]
 
 
+def parse_names(text):
+    return [x.strip() for x in text.split(",") if x.strip()]
+
+
 def sweep_parser(description):
     """The flags of tools/rl_sweep.py (and, with their own additions, tools/rl_pbt.py)."""
     import argparse
     ap = argparse.ArgumentParser(description=description)
     ap.add_argument("env", choices=["blackjack", "frozen_lake", "cliffwalking", "taxi"])
     ap.add_argument("--grid", action="append", default=[], metavar="FLAG=V1,V2,...",
-                    help="a bin flag and its values (repeatable; one of %s, %s)" % (", ".join(SWEEP_FLAGS), PLANNING_AXIS))
+                    help="a bin flag and its values (repeatable; one of %s, %s, %s)" % (", ".join(SWEEP_FLAGS), PLANNING_AXIS, TARGET_AXIS))
     for name in SWEEP_FLAGS:
         ap.add_argument("--" + name, default=None, metavar="V1,V2,...", help="values of this flag (a comma list: a grid axis)")
     ap.add_argument("--" + PLANNING_AXIS, default=None, metavar="K1,K2,...",
@@ -449,7 +474,8 @@ def sweep_parser(description):
     ap.add_argument("--map", default="4x4")
     ap.add_argument("--agent", choices=sorted(AGENT_NAMES), default="onestep")
     ap.add_argument("--selector", choices=sorted(SELECTOR_NAMES), default="eps")
-    ap.add_argument("--target", choices=sorted(TARGET_KINDS), default="qlearning")
+    ap.add_argument("--target", default="qlearning", metavar="NAME[,NAME...]",
+                    help="bootstrap target, one of %s: one name for every agent, or a comma list (a grid axis)" % ", ".join(sorted(TARGET_KINDS)))
     ap.add_argument("--policy", choices=["basic", "double"], default="basic")
     ap.add_argument("--agents_per_point", type=int, default=1024)
     ap.add_argument("--seed", type=lambda x: int(x, 0), default=0x5EED0001)
@@ -469,7 +495,17 @@ def parse_sweep_args(ap, argv):
         except ValueError:
             ap.error("--%s takes non-negative integers, got %r" % (PLANNING_AXIS, text))
 
+    def target_list(text):
+        names = parse_names(text)
+        if not names or any(x not in TARGET_KINDS for x in names):
+            ap.error("--%s takes names among %s, got %r" % (TARGET_AXIS, ", ".join(sorted(TARGET_KINDS)), text))
+        return names
+
     grid = {}
+    targets = target_list(a["target"])
+    if len(targets) > 1:   # a comma list is an axis; a single name stays engine-wide
+        grid[TARGET_AXIS] = targets
+        a["target"] = targets[0]
     for name in SWEEP_FLAGS:
         v = a.pop(name)
         if v is not None:
@@ -484,8 +520,12 @@ def parse_sweep_args(ap, argv):
         if k == PLANNING_AXIS:
             grid[k] = planning_list(v)
             continue
+        if k == TARGET_AXIS:
+            grid[k] = target_list(v)
+            a["target"] = grid[k][0]
+            continue
         if k not in SWEEP_FLAGS:
-            ap.error("--grid %s: not a sweepable flag (%s, %s)" % (k, ", ".join(SWEEP_FLAGS), PLANNING_AXIS))
+            ap.error("--grid %s: not a sweepable flag (%s, %s, %s)" % (k, ", ".join(SWEEP_FLAGS), PLANNING_AXIS, TARGET_AXIS))
         grid[k] = parse_list(v)
     if not grid:
         ap.error("nothing to sweep: give at least one --grid FLAG=V1,V2,...")
@@ -535,11 +575,19 @@ def pbt_perturb_planning(k, f):
     return out
 
 
-def pbt_explore(flags, axes, rng):
-    """The winner's flags with every grid axis multiplied by 0.8 or 1.2 at random and clamped into its range (the
-    planning count as an integer: pbt_perturb_planning)."""
+def pbt_explore(flags, axes, rng, targets=None, resample_probability=0.25):
+    """The winner's flags with every numeric grid axis multiplied by 0.8 or 1.2 at random and clamped into its range (the
+    planning count as an integer: pbt_perturb_planning).  A target axis is inherited, and with probability
+    `resample_probability` redrawn uniformly from `targets` (the axis values).  Without a target axis the draws are
+    those of the numeric axes alone."""
     out = dict(flags)
     for k in axes:
+        if k == TARGET_AXIS:
+            if targets is None:
+                raise ValueError("a target axis needs its values (targets=) to resample from")
+            if rng.random() < resample_probability:
+                out[k] = targets[int(rng.integers(len(targets)))]
+            continue
         f = PBT_FACTORS[int(rng.integers(2))]
         if k == PLANNING_AXIS:
             out[k] = pbt_perturb_planning(int(flags[k]), f)
@@ -549,20 +597,23 @@ def pbt_explore(flags, axes, rng):
     return out
 
 
-def run_pbt(env_name, grid, *, interval, fraction=0.25, pbt_seed=0x9B7, agent="onestep", selector="eps", target="qlearning",
-            policy="basic", agents_per_point=1024, seed=0x5EED0001, real="f64", device=0, verbose=True, **flags):
+def run_pbt(env_name, grid, *, interval, fraction=0.25, pbt_seed=0x9B7, resample_probability=0.25, agent="onestep", selector="eps",
+            target="qlearning", policy="basic", agents_per_point=1024, seed=0x5EED0001, real="f64", device=0, verbose=True, **flags):
     """Population-based training over the grid of `grid`: the initial population is run_sweep's (one set per point,
     contiguous groups of `agents_per_point`), and its one `train(n, n/10)` is driven in chunks of `interval` episodes.
     After every chunk but the last the sets are ranked by their mean training return over the chunk; each of the bottom
     floor(fraction * G) sets takes over the learned state of a set drawn from the top as many (agent j of the winner ->
-    agent j of the loser, one rlb_agent_clone) and continues with the winner's flags, every grid axis perturbed
-    (rlb_engine_retune_hparams).  `pbt_seed` seeds those draws.  Returns run_sweep's output plus every set's final flags
+    agent j of the loser, one rlb_agent_clone) and continues with the winner's flags, every numeric grid axis perturbed
+    (rlb_engine_retune_hparams) and a target axis inherited, or with probability `resample_probability` redrawn from the
+    axis values (rlb_engine_set_targets).  `pbt_seed` seeds those draws.  Returns run_sweep's output plus every set's final flags
     and the lineage: per chunk boundary, the list of (loser, winner, new flags)."""
     if not 0.0 <= fraction <= 0.5:
         raise ValueError("fraction must be in [0, 0.5]: the top and bottom sets may not overlap")
     interval = int(interval)
     if interval < 1:
         raise ValueError("interval must be >= 1")
+    if not 0.0 <= resample_probability <= 1.0:
+        raise ValueError("resample_probability must be in [0, 1]")
     if PLANNING_AXIS in grid and agent == "traces":
         raise ValueError("PBT with a planning_steps axis clones Dyna agents, and cloning a trace agent under a model is not supported")
     axes = list(grid)
@@ -583,7 +634,7 @@ def run_pbt(env_name, grid, *, interval, fraction=0.25, pbt_seed=0x9B7, agent="o
             pairs = pbt_exploit(res["sums"], fraction, rng)
             step = []
             for loser, winner in pairs:
-                cur[loser] = pbt_explore(cur[winner], axes, rng)
+                cur[loser] = pbt_explore(cur[winner], axes, rng, grid.get(TARGET_AXIS), resample_probability)
                 sets[loser] = point_hparams(cur[loser], n)
                 step.append(dict(loser=loser, winner=winner, flags={k: cur[loser][k] for k in axes}))
             if pairs:
@@ -592,6 +643,8 @@ def run_pbt(env_name, grid, *, interval, fraction=0.25, pbt_seed=0x9B7, agent="o
                 eng.retune_hparams(sets)
                 if PLANNING_AXIS in axes:
                     eng.set_planning_steps(np.array([c[PLANNING_AXIS] for c in cur], np.uint32))
+                if TARGET_AXIS in axes:
+                    eng.set_targets(point_targets(cur))
             lineage.append(dict(episode=end, pairs=step))
         ev = eng.evaluate(n, sums=True)["sums"]                                                      # [n, G, 4]
         dt = time.perf_counter() - t0
@@ -604,9 +657,9 @@ def run_pbt(env_name, grid, *, interval, fraction=0.25, pbt_seed=0x9B7, agent="o
         print("PBT: %d sets x %d agents, %d episodes in chunks of %d, fraction %.3g: %.2fs" % (len(points), per, n, interval, fraction, dt))
         for g in ranking[:10]:
             print("  set %-4d %-60s evaluate mean return %.4f" % (g, out_points[g]["final_params"], out_points[g]["eval_mean_return"]))
-    return dict(env=env_name, agent=agent, selector=selector, target=target, policy=policy, real=real, n_episodes=n,
+    return dict(env=env_name, agent=agent, selector=selector, target=engine_target(grid, target), policy=policy, real=real, n_episodes=n,
                 agents_per_point=per, grid={k: list(v) for k, v in grid.items()}, interval=interval, fraction=fraction,
-                pbt_seed=int(pbt_seed), points=out_points, ranking=ranking, lineage=lineage, seconds=dt, train_steps=train_steps)
+                pbt_seed=int(pbt_seed), **({"resample_probability": resample_probability} if TARGET_AXIS in grid else {}), points=out_points, ranking=ranking, lineage=lineage, seconds=dt, train_steps=train_steps)
 
 
 def main_pbt(argv=None):
@@ -615,6 +668,8 @@ def main_pbt(argv=None):
     ap.add_argument("--interval", type=int, required=True, help="episodes per chunk between exploit / explore steps")
     ap.add_argument("--fraction", type=float, default=0.25, help="share of the sets replaced after each chunk (and drawn from)")
     ap.add_argument("--pbt_seed", type=lambda x: int(x, 0), default=0x9B7, help="seed of the winner draws and perturbations")
+    ap.add_argument("--resample_probability", type=float, default=0.25,
+                    help="with a target axis: chance that a loser's inherited target is redrawn from the axis values")
     env_name, grid, outp, kw = parse_sweep_args(ap, argv)
     res = run_pbt(env_name, grid, **kw)
     write_json(res, outp)
@@ -699,7 +754,7 @@ def run_halving(env_name, grid, *, min_episodes, eta=3, agent="onestep", selecto
               % (n_sets, per, n, budgets, int(eta), dt, train_steps))
         for g in ranking[:min(10, len(survivors))]:
             print("  set %-4d %-60s evaluate mean return %.4f" % (g, points[g], out_points[g]["eval_mean_return"]))
-    return dict(env=env_name, agent=agent, selector=selector, target=target, policy=policy, real=real, n_episodes=n,
+    return dict(env=env_name, agent=agent, selector=selector, target=engine_target(grid, target), policy=policy, real=real, n_episodes=n,
                 agents_per_point=per, grid={k: list(v) for k, v in grid.items()}, min_episodes=int(min_episodes), eta=int(eta),
                 points=out_points, ranking=ranking, rungs=rungs, seconds=dt, train_steps=train_steps)
 

@@ -2,8 +2,8 @@
 The complete state is: Q tables, UCB counts, and per agent the RNG word index, epsilon, UCB t and Double flag
 (rlb_download_tables / rlb_get_agent_states), plus the Dyna model when one is attached (rlb_download_model) and the
 per-agent hyper-parameter sets when they are installed (rlb_engine_set_hparams), with the active-set mask while some
-set is paused (rlb_engine_set_active_sets) and the per-set planning counts while they are in force
-(rlb_engine_set_planning_steps).  Stored as one .npz; the configuration
+set is paused (rlb_engine_set_active_sets), the per-set planning counts while they are in force
+(rlb_engine_set_planning_steps) and the per-set targets while they are (rlb_engine_set_targets).  Stored as one .npz; the configuration
 is stored beside it and checked."""
 import ctypes as C
 
@@ -26,6 +26,8 @@ def save_snapshot(engine, path):
         extra["hp_sets"], extra["hp_group"] = engine.hparams
         if engine.active_sets is not None:
             extra["hp_active"] = np.asarray(engine.active_sets, np.uint8)
+        if engine.targets is not None:
+            extra["hp_target"] = np.asarray(engine.targets, np.int32)
     q, counts = engine.download_tables()
     cfg = {k: int(getattr(engine.cfg, k)) for k in _CFG_FIELDS}
     np.savez_compressed(path, q=q, counts=counts, states=engine.states(), selector_kind=np.int64(engine.cfg.selector_kind),
@@ -57,5 +59,7 @@ def load_snapshot(engine, path):
         engine.set_model(planning)
     if planning:
         engine.upload_model(z["model_len"], z["model"])
+    if "hp_target" in z.files:
+        engine.set_targets(z["hp_target"])
     if "hp_active" in z.files:
         engine.set_active_sets(z["hp_active"])

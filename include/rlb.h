@@ -326,6 +326,32 @@ rlb_status rlb_engine_set_planning_steps(rlb_engine* e, const uint32_t* steps, u
  * value outside RLB_TARGET_SARSA .. RLB_TARGET_EXPECTED_SARSA.  Unlike rlb_hparams the values are checked: an
  * unknown target would otherwise run as Expected Sarsa. */
 rlb_status rlb_engine_set_targets(rlb_engine* e, const int32_t* targets, uint32_t n_sets);
+/* The action selector per hyper-parameter set (kept beside rlb_hparams, as the targets are).  selectors [n_sets] i32
+ * RLB_SEL_*, host or device: the agents of set g select actions as rlb_agent_set_action_selector(selectors[g]) would
+ * make them, in every call: the fused train and evaluate calls, rlb_agent_get_action, rlb_agent_update, rlb_agent_step,
+ * rlb_selector_get_action, rlb_selector_get_exploration_probs, rlb_selector_update and the resets.
+ * Equivalence: from this call on every call gives agent i the bits of agent 0 of an engine created with selector_kind =
+ * selectors[group[i]], its set's values, target and planning count, n_agents = 1 and first_agent_id + i, given this
+ * engine's tables and this agent's state.
+ * A set whose selector changes gets a fresh selector of its new kind, as rlb_agent_set_action_selector gives every agent:
+ * epsilon = its set's initial_epsilon, UCB t = 1, its agents' counts rows zero.  This holds in both directions, so an
+ * eps-greedy agent's counts are always zero.  A set whose selector is unchanged keeps its selector state: a second call
+ * with the same array does nothing.
+ * rlb_engine_set_hparams (installing or uninstalling) and rlb_agent_set_action_selector(k) put every set on the
+ * engine-wide selector, with a fresh selector everywhere.  rlb_engine_retune_hparams, rlb_engine_set_active_sets,
+ * rlb_engine_set_planning_steps, rlb_engine_set_targets and rlb_agent_set_kind keep the per-set selectors
+ * (rlb_agent_set_kind gives each agent a fresh selector of its set's kind); rlb_agent_reset and rlb_selector_reset reset
+ * each agent's selector as its set's kind does, and rlb_selector_update decays epsilon only in eps-greedy sets.
+ * rlb_agent_clone's destination keeps its set, so its set's selector: the counts segment is copied to destinations of
+ * UCB sets and left zero in those of eps-greedy sets.  rlb_download_tables / rlb_upload_tables carry counts while any
+ * set uses UCB.  Record, sums and totals layouts do not change.
+ * The fused calls launch once per selector: the agents of the eps-greedy sets and those of the UCB sets (restricted to
+ * the active sets) run as two concurrent launches, one launch where only one of them has agents.
+ * RLB_ERR_INVALID_ARG, the engine untouched: no sets installed, n_sets != rlb_engine_hparam_sets(e), selectors NULL, or
+ * a value outside RLB_SEL_EPS_GREEDY .. RLB_SEL_UCB.  RLB_ERR_UNSUPPORTED, the engine untouched: the engine's table
+ * store cannot run a requested selector (the thread-group or hybrid store when that selector's on-chip bytes exceed
+ * the per-block limit); the store is not re-picked. */
+rlb_status rlb_engine_set_selectors(rlb_engine* e, const int32_t* selectors, uint32_t n_sets);
 
 /* ---- Env<T,COUNT> (env.rs:19-49), batched ------------------------------------------------ */
 /* Env::reset (blackjack.rs:105, frozen_lake.rs:106, cliff_walking.rs:67, taxi.rs:135).  obs_out [N] u32 */
@@ -440,7 +466,7 @@ rlb_status rlb_get_agent_states(rlb_engine* e, rlb_agent_state* states_out /* [N
 rlb_status rlb_set_agent_states(rlb_engine* e, const rlb_agent_state* states /* [N] */);
 /* Agent dst[j] takes the learned state of agent src[j], for j < n_pairs (the exploit step of population-based training;
  * no reference equivalent), in one device launch: its Q table(s) (both for Double), its UCB counts when the selector is
- * UCB, epsilon, ucb_t and policy_flag, and its Dyna model when one is attached (entries, membership bits, length).
+ * UCB (under rlb_engine_set_selectors: when dst[j]'s set is UCB), epsilon, ucb_t and policy_flag, and its Dyna model when one is attached (entries, membership bits, length).
  * dst[j] keeps its RNG stream position rng_n (its Philox stream stays keyed by its own global id, so a clone does not
  * replay the source's draws), its env state, its eligibility rows and lazy-sweep bookkeeping, its rlb_agent_step state
  * and its hyper-parameter set.  src, dst [n_pairs] u32, host or device.

@@ -83,7 +83,7 @@ EXPORTS = [
     "rlb_comm_unique_id", "rlb_comm_init_rank", "rlb_comm_init_all", "rlb_comm_destroy", "rlb_comm_rank", "rlb_comm_world_size",
     "rlb_comm_gather_episode_sums", "rlb_comm_allreduce_sum", "rlb_comm_group_begin", "rlb_comm_group_end",
     "rlb_selftest_ucb_math", "rlb_engine_set_hparams", "rlb_engine_hparam_sets", "rlb_engine_retune_hparams", "rlb_agent_clone",
-    "rlb_engine_set_active_sets", "rlb_engine_set_planning_steps", "rlb_engine_set_targets",
+    "rlb_engine_set_active_sets", "rlb_engine_set_planning_steps", "rlb_engine_set_targets", "rlb_engine_set_selectors",
 ]
 
 
@@ -125,6 +125,7 @@ def _load():
     L.rlb_engine_set_active_sets.argtypes = [vp, vp, u32]
     L.rlb_engine_set_planning_steps.argtypes = [vp, vp, u32]
     L.rlb_engine_set_targets.argtypes = [vp, vp, u32]
+    L.rlb_engine_set_selectors.argtypes = [vp, vp, u32]
     L.rlb_env_reset.argtypes = [vp, vp]
     L.rlb_env_step.argtypes = [vp, vp, vp, vp, vp, vp]
     L.rlb_agent_get_action.argtypes = [vp, vp, vp]
@@ -255,6 +256,7 @@ class Engine:
         self.active_sets = None     # bool (G,) while some set is paused (set_active_sets), else None
         self.planning = None        # uint32 (G,) per-set Dyna planning counts (set_planning_steps), else None
         self.targets = None         # int32 (G,) per-set targets while they differ from cfg.target_kind (set_targets), else None
+        self.selectors = None       # int32 (G,) per-set selectors as last given to set_selectors, else None
 
     def close(self):
         if getattr(self, "h", None):
@@ -304,7 +306,7 @@ class Engine:
         While sets are installed, train() and evaluate() return per-episode sums shaped (E, G, 4)."""
         if sets is None and group is None:
             check(lib.rlb_engine_set_hparams(self.h, None, 0, None))
-            self.G, self.hparams, self.active_sets, self.planning, self.targets = 0, None, None, None, None
+            self.G, self.hparams, self.active_sets, self.planning, self.targets, self.selectors = 0, None, None, None, None, None
             return
         arr = self.hparams_array(sets)
         grp = np.asarray(group)
@@ -314,7 +316,7 @@ class Engine:
             raise ValueError("group ids must be in [0, 2**32)")
         grp = np.ascontiguousarray(grp, np.uint32)
         check(lib.rlb_engine_set_hparams(self.h, ptr(arr) if len(arr) else None, len(arr), ptr(grp) if len(arr) else None))
-        self.G, self.hparams, self.active_sets, self.planning, self.targets = len(arr), (arr.copy(), grp.copy()), None, None, None
+        self.G, self.hparams, self.active_sets, self.planning, self.targets, self.selectors = len(arr), (arr.copy(), grp.copy()), None, None, None, None
 
     def hparam_sets(self):
         """rlb_engine_hparam_sets: the number of sets installed, 0 while the configured values apply."""
@@ -374,6 +376,20 @@ class Engine:
         k = np.ascontiguousarray(k, np.int32)
         check(lib.rlb_engine_set_targets(self.h, ptr(k) if len(k) else None, len(k)))
         self.targets = None if (k == self.cfg.target_kind).all() else k.copy()
+
+    def set_selectors(self, kinds):
+        """rlb_engine_set_selectors: the agents of set g select actions with selector kinds[g] ((G,) SEL_* integers) in
+        every later call.  A set whose selector changes gets a fresh selector of its new kind (epsilon = its
+        initial_epsilon, UCB t = 1, counts zero); the others keep theirs (see include/rlb.h).  `selectors` then holds the
+        kinds; set_hparams and set_selector put every set back on the engine's selector and `selectors` back to None."""
+        k = np.asarray(kinds)
+        if k.shape != (self.G,):
+            raise ValueError("selectors must have shape (%d,), got %r" % (self.G, k.shape))
+        if k.size and (k.dtype.kind not in "iu" or k.min() < SEL_EPS_GREEDY or k.max() > SEL_UCB):
+            raise ValueError("selectors must be integers in [%d, %d]" % (SEL_EPS_GREEDY, SEL_UCB))
+        k = np.ascontiguousarray(k, np.int32)
+        check(lib.rlb_engine_set_selectors(self.h, ptr(k) if len(k) else None, len(k)))
+        self.selectors = k.copy()
 
     # ---- population-based training: the exploit step
     def clone_agents(self, src, dst):
@@ -479,6 +495,7 @@ class Engine:
     def set_selector(self, kind):
         check(lib.rlb_agent_set_action_selector(self.h, kind))
         self.cfg.selector_kind = kind
+        self.selectors = None
 
     def set_agent_kind(self, kind):
         check(lib.rlb_agent_set_kind(self.h, kind))

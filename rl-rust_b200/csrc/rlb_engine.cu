@@ -109,6 +109,19 @@ struct rlb_engine {
     // per-set bootstrap targets (rlb_engine_set_targets); every entry cfg.target_kind until that call
     std::vector<int32_t> h_hp_targets;     // [hp_n]
     int32_t* d_hp_targets = nullptr;       // [hp_n] device copy: HpParams::targets
+    // per-set action selectors (rlb_engine_set_selectors); every entry cfg.selector_kind until that call
+    std::vector<int32_t> h_hp_sel;         // [hp_n]
+    int32_t* d_hp_sel = nullptr;           // [hp_n] device copy (the epsilon decay of the eps-greedy sets)
+    uint8_t* d_sel_mode = nullptr;         // [hp_n] per-set modes of launch_selector_fresh
+    // The agents of each selector, d_hp_order filtered by the set's selector: selector 0's list, then selector 1's.  All
+    // agents for the step-level calls (d_sel_all), the active sets' for train / evaluate (d_sel_run, only under a mask).
+    // The lists exist only while both selectors have agents; the counts are kept whenever sets are installed.
+    uint32_t* d_sel_all = nullptr;
+    uint32_t* d_sel_run = nullptr;
+    uint64_t n_sel_all[2] = {0, 0}, n_sel_run[2] = {0, 0};
+    // the second selector's launch runs on its own stream, forked from and joined back to `stream` inside dispatch_run
+    cudaStream_t aux_stream = nullptr;
+    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     // Calls whose work is enqueued but not yet waited for (rlb_agent_train_range_async): at most two, so that the
     // kernels of call i + 1 are in the queue before the host blocks on the copies of call i.
     struct Pending {
@@ -207,17 +220,70 @@ cudaError_t fill_eps_initial(rlb_engine* e) {
     return fill<double>(e, e->d_eps, e->cfg.n_agents, e->cfg.initial_epsilon);
 }
 
-cudaError_t dispatch_run(rlb_engine* e, const DevParams& p) {
-    const bool masked = !e->hp_active.empty();   // only the active sets' agents run: a launch sized to them
-    const HpParams sets{e->d_hp_sets, e->d_hp_group, masked ? e->d_hp_run : nullptr, masked ? e->hp_n_run : e->cfg.n_agents, e->d_hp_planning,
-                        e->d_hp_targets};
-    if (p.planning_steps && p.mode == 0 && e->hp_n) {   // the model under sets: each set's own planning count
+#ifndef RLB_SEL_CONCURRENT
+#define RLB_SEL_CONCURRENT 1   // the two selectors' launches on two streams (0: back to back on the engine's stream)
+#endif
+
+// k_run_hp (with the model: its Dyna twin) over the launch positions of h, with selector v.sel
+cudaError_t launch_run_hp(rlb_engine* e, const DevParams& p, const Variant& v, const HpParams& h, cudaStream_t stream) {
+    if (p.planning_steps && p.mode == 0) {   // the model under sets: each set's own planning count
         switch (e->cfg.env_kind) {
-            case RLB_ENV_BLACKJACK: return launch_run_model<RLB_ENV_BLACKJACK, true>(e->variant, p, e->stream, sets);
-            case RLB_ENV_FROZEN_LAKE: return launch_run_model<RLB_ENV_FROZEN_LAKE, true>(e->variant, p, e->stream, sets);
-            case RLB_ENV_CLIFF_WALKING: return launch_run_model<RLB_ENV_CLIFF_WALKING, true>(e->variant, p, e->stream, sets);
-            default: return launch_run_model<RLB_ENV_TAXI, true>(e->variant, p, e->stream, sets);
+            case RLB_ENV_BLACKJACK: return launch_run_model<RLB_ENV_BLACKJACK, true>(v, p, stream, h);
+            case RLB_ENV_FROZEN_LAKE: return launch_run_model<RLB_ENV_FROZEN_LAKE, true>(v, p, stream, h);
+            case RLB_ENV_CLIFF_WALKING: return launch_run_model<RLB_ENV_CLIFF_WALKING, true>(v, p, stream, h);
+            default: return launch_run_model<RLB_ENV_TAXI, true>(v, p, stream, h);
         }
+    }
+    switch (e->cfg.env_kind) {   // every agent with its own hyper-parameter set (with a model: evaluate, which never touches it)
+        case RLB_ENV_BLACKJACK: return launch_run<RLB_ENV_BLACKJACK, true>(v, p, e->store, stream, h);
+        case RLB_ENV_FROZEN_LAKE: return launch_run<RLB_ENV_FROZEN_LAKE, true>(v, p, e->store, stream, h);
+        case RLB_ENV_CLIFF_WALKING: return launch_run<RLB_ENV_CLIFF_WALKING, true>(v, p, e->store, stream, h);
+        default: return launch_run<RLB_ENV_TAXI, true>(v, p, e->store, stream, h);
+    }
+}
+
+// the variant of one selector's agents
+Variant with_selector(const rlb_engine* e, int sel) {
+    Variant v = e->variant;
+    v.sel = sel;
+    return v;
+}
+
+cudaError_t dispatch_run(rlb_engine* e, const DevParams& p) {
+    if (e->hp_n) {
+        const bool masked = !e->hp_active.empty();   // only the active sets' agents run: a launch sized to them
+        HpParams sets{e->d_hp_sets, e->d_hp_group, masked ? e->d_hp_run : nullptr, masked ? e->hp_n_run : e->cfg.n_agents, e->d_hp_planning,
+                      e->d_hp_targets, 0};
+        if (!e->n_sel_run[0] || !e->n_sel_run[1])   // one selector among the running agents: one launch, as without per-set selectors
+            return launch_run_hp(e, p, with_selector(e, e->n_sel_run[1] ? RLB_SEL_UCB : e->n_sel_run[0] ? RLB_SEL_EPS_GREEDY : e->variant.sel), sets, e->stream);
+        // one launch per selector over its agents' list; the second's positions start at a multiple of 32 past the
+        // first's, so that the hybrid store's scratch rows (addressed by position) of the two never meet
+        const uint32_t* lists = masked ? e->d_sel_run : e->d_sel_all;
+        HpParams second = sets;
+        sets.agents = lists; sets.n_launch = e->n_sel_run[0];
+        second.agents = lists + e->n_sel_run[0]; second.n_launch = e->n_sel_run[1];
+        second.pos_base = (e->n_sel_run[0] + 31) / 32 * 32;
+        cudaStream_t s2 = e->stream;
+#if RLB_SEL_CONCURRENT
+        if (!e->aux_stream) {
+            cudaError_t err = cudaStreamCreateWithFlags(&e->aux_stream, cudaStreamNonBlocking);
+            if (err == cudaSuccess) err = cudaEventCreateWithFlags(&e->ev_fork, cudaEventDisableTiming);
+            if (err == cudaSuccess) err = cudaEventCreateWithFlags(&e->ev_join, cudaEventDisableTiming);
+            if (err != cudaSuccess) return err;
+        }
+        cudaError_t err = cudaEventRecord(e->ev_fork, e->stream);
+        if (err == cudaSuccess) err = cudaStreamWaitEvent(e->aux_stream, e->ev_fork, 0);
+        if (err != cudaSuccess) return err;
+        s2 = e->aux_stream;
+#endif
+        cudaError_t err0 = launch_run_hp(e, p, with_selector(e, RLB_SEL_EPS_GREEDY), sets, e->stream);
+        cudaError_t err1 = launch_run_hp(e, p, with_selector(e, RLB_SEL_UCB), second, s2);
+#if RLB_SEL_CONCURRENT
+        cudaError_t err2 = cudaEventRecord(e->ev_join, e->aux_stream);   // everything after dispatch_run sees one stream
+        if (err2 == cudaSuccess) err2 = cudaStreamWaitEvent(e->stream, e->ev_join, 0);
+        if (err2 != cudaSuccess) return err2;
+#endif
+        return err0 != cudaSuccess ? err0 : err1;
     }
     if (p.planning_steps && p.mode == 0) {   // InternalModelAgent::update on the training path; evaluate never touches the model
         switch (e->cfg.env_kind) {
@@ -225,14 +291,6 @@ cudaError_t dispatch_run(rlb_engine* e, const DevParams& p) {
             case RLB_ENV_FROZEN_LAKE: return launch_run_model<RLB_ENV_FROZEN_LAKE>(e->variant, p, e->stream);
             case RLB_ENV_CLIFF_WALKING: return launch_run_model<RLB_ENV_CLIFF_WALKING>(e->variant, p, e->stream);
             default: return launch_run_model<RLB_ENV_TAXI>(e->variant, p, e->stream);
-        }
-    }
-    if (e->hp_n) {   // every agent with its own hyper-parameter set (with a model: evaluate, which never touches it)
-        switch (e->cfg.env_kind) {
-            case RLB_ENV_BLACKJACK: return launch_run<RLB_ENV_BLACKJACK, true>(e->variant, p, e->store, e->stream, sets);
-            case RLB_ENV_FROZEN_LAKE: return launch_run<RLB_ENV_FROZEN_LAKE, true>(e->variant, p, e->store, e->stream, sets);
-            case RLB_ENV_CLIFF_WALKING: return launch_run<RLB_ENV_CLIFF_WALKING, true>(e->variant, p, e->store, e->stream, sets);
-            default: return launch_run<RLB_ENV_TAXI, true>(e->variant, p, e->store, e->stream, sets);
         }
     }
     switch (e->cfg.env_kind) {
@@ -246,17 +304,20 @@ cudaError_t dispatch_run(rlb_engine* e, const DevParams& p) {
 // Where k_run keeps the per-agent tables.  The shared-memory (thread-group) store pays when every step sweeps many
 // rows, i.e. for the eligibility-trace agents of the 4-action envs; one-step updates touch two rows per step and run
 // faster from HBM at full occupancy (measured, DESIGN.md §7).
-size_t store_bytes(rlb_engine* e, int store) {
+size_t store_bytes(rlb_engine* e, int store, const Variant& v) {
     switch (e->cfg.env_kind) {
-        case RLB_ENV_BLACKJACK: return smem_store_bytes<RLB_ENV_BLACKJACK>(e->variant, store, e->S, e->S, e->dp.vmax);
-        case RLB_ENV_FROZEN_LAKE: return smem_store_bytes<RLB_ENV_FROZEN_LAKE>(e->variant, store, store == STORE_HYBRID ? e->dp.n_live : e->S, e->S, e->dp.vmax);
-        case RLB_ENV_CLIFF_WALKING: return smem_store_bytes<RLB_ENV_CLIFF_WALKING>(e->variant, store, store == STORE_HYBRID ? e->dp.n_live : e->S, e->S, e->dp.vmax);
-        default: return smem_store_bytes<RLB_ENV_TAXI>(e->variant, store, e->S, e->S, e->dp.vmax);
+        case RLB_ENV_BLACKJACK: return smem_store_bytes<RLB_ENV_BLACKJACK>(v, store, e->S, e->S, e->dp.vmax);
+        case RLB_ENV_FROZEN_LAKE: return smem_store_bytes<RLB_ENV_FROZEN_LAKE>(v, store, store == STORE_HYBRID ? e->dp.n_live : e->S, e->S, e->dp.vmax);
+        case RLB_ENV_CLIFF_WALKING: return smem_store_bytes<RLB_ENV_CLIFF_WALKING>(v, store, store == STORE_HYBRID ? e->dp.n_live : e->S, e->S, e->dp.vmax);
+        default: return smem_store_bytes<RLB_ENV_TAXI>(v, store, e->S, e->S, e->dp.vmax);
     }
 }
+size_t store_bytes(rlb_engine* e, int store) { return store_bytes(e, store, e->variant); }
+
+constexpr size_t kSmemPerBlockMax = 227 * 1024;   // dynamic shared memory one CTA may have
 
 rlb_status pick_store(rlb_engine* e) {
-    const size_t per_block_max = 227 * 1024, per_sm = 228 * 1024;
+    const size_t per_block_max = kSmemPerBlockMax, per_sm = 228 * 1024;
     const size_t b_group = store_bytes(e, STORE_SMEM), b_hybrid = store_bytes(e, STORE_HYBRID);
     const bool fits_group = b_group > 0 && b_group <= per_block_max && e->S <= 256;      // GroupStore keeps visited states in 8 bits
     const bool fits_hybrid = b_hybrid > 0 && b_hybrid <= per_block_max && e->S <= 64;   // DevParams::row_lut holds 64 states
@@ -311,23 +372,39 @@ rlb_status pick_store(rlb_engine* e) {
     e->store = want;
     e->smem_bytes = want == STORE_SMEM ? b_group : (want == STORE_HYBRID ? b_hybrid : 0);
     if (want == STORE_HYBRID && e->variant.trace && !e->d_etr_il) {
-        const uint64_t n32 = (e->cfg.n_agents + 31) / 32 * 32;
+        // + 32 positions: a second concurrent launch (one per selector) starts at a multiple of 32 past the first's
+        const uint64_t n32 = (e->cfg.n_agents + 31) / 32 * 32 + 32;
         CK(cudaMalloc(&e->d_etr_il, (size_t)n32 * e->dp.vmax * e->APAD * e->real_size));
         e->dp.etr_il = e->d_etr_il;
     }
     return RLB_OK;
 }
 
+cudaError_t launch_step_hp(rlb_engine* e, StepOp op, const Variant& v, const StepArgs& a) {
+    switch (e->cfg.env_kind) {
+        case RLB_ENV_BLACKJACK: return launch_step<RLB_ENV_BLACKJACK, true>(op, v, e->dp, a, e->stream);
+        case RLB_ENV_FROZEN_LAKE: return launch_step<RLB_ENV_FROZEN_LAKE, true>(op, v, e->dp, a, e->stream);
+        case RLB_ENV_CLIFF_WALKING: return launch_step<RLB_ENV_CLIFF_WALKING, true>(op, v, e->dp, a, e->stream);
+        default: return launch_step<RLB_ENV_TAXI, true>(op, v, e->dp, a, e->stream);
+    }
+}
+
 cudaError_t dispatch_step(rlb_engine* e, StepOp op, const StepArgs& a) {
     if (e->hp_n) {
         StepArgs with_sets = a;
-        with_sets.sets = HpParams{e->d_hp_sets, e->d_hp_group, nullptr, 0, e->d_hp_planning, e->d_hp_targets};
-        switch (e->cfg.env_kind) {
-            case RLB_ENV_BLACKJACK: return launch_step<RLB_ENV_BLACKJACK, true>(op, e->variant, e->dp, with_sets, e->stream);
-            case RLB_ENV_FROZEN_LAKE: return launch_step<RLB_ENV_FROZEN_LAKE, true>(op, e->variant, e->dp, with_sets, e->stream);
-            case RLB_ENV_CLIFF_WALKING: return launch_step<RLB_ENV_CLIFF_WALKING, true>(op, e->variant, e->dp, with_sets, e->stream);
-            default: return launch_step<RLB_ENV_TAXI, true>(op, e->variant, e->dp, with_sets, e->stream);
-        }
+        with_sets.sets = HpParams{e->d_hp_sets, e->d_hp_group, nullptr, e->cfg.n_agents, e->d_hp_planning, e->d_hp_targets, 0};
+        const bool by_selector = op == OP_GET_ACTION || op == OP_UPDATE || op == OP_SELECTOR_GET_ACTION || op == OP_SELECTOR_PROBS ||
+                                 op == OP_AGENT_STEP;
+        if (!by_selector) return launch_step_hp(e, op, e->variant, with_sets);
+        // every agent (the step calls ignore the active mask), one launch per selector that has agents
+        if (!e->n_sel_all[0] || !e->n_sel_all[1])
+            return launch_step_hp(e, op, with_selector(e, e->n_sel_all[1] ? RLB_SEL_UCB : RLB_SEL_EPS_GREEDY), with_sets);
+        StepArgs second = with_sets;
+        with_sets.sets.agents = e->d_sel_all; with_sets.sets.n_launch = e->n_sel_all[0];
+        second.sets.agents = e->d_sel_all + e->n_sel_all[0]; second.sets.n_launch = e->n_sel_all[1];
+        cudaError_t err = launch_step_hp(e, op, with_selector(e, RLB_SEL_EPS_GREEDY), with_sets);
+        if (err != cudaSuccess) return err;
+        return launch_step_hp(e, op, with_selector(e, RLB_SEL_UCB), second);
     }
     switch (e->cfg.env_kind) {
         case RLB_ENV_BLACKJACK: return launch_step<RLB_ENV_BLACKJACK>(op, e->variant, e->dp, a, e->stream);
@@ -398,6 +475,24 @@ rlb_status attach_model(rlb_engine* e, uint32_t planning_steps) {
     return ensure_trace_buffers(e);
 }
 
+// UCB's counts and ln table, allocated the first time any agent uses UCB; *fresh: the counts were just allocated (their
+// contents undefined)
+rlb_status ensure_ucb_buffers(rlb_engine* e, bool* fresh) {
+    if (fresh) *fresh = !e->d_counts;
+    if (!e->d_counts) {
+        e->counts_bytes = (size_t)e->cfg.n_agents * e->S * e->APAD * sizeof(uint32_t);
+        CK(cudaMalloc(&e->d_counts, e->counts_bytes));
+    }
+    if (!e->d_log_table) {   // ln(t) table of the UCB bonus
+        CK(cudaMalloc(&e->d_log_table, (size_t)RLB_LOG_TABLE_N * sizeof(double)));
+        k_fill_log_table<<<(RLB_LOG_TABLE_N + 255) / 256, 256, 0, e->stream>>>(e->d_log_table, RLB_LOG_TABLE_N);
+        CK(cudaGetLastError());
+        e->dp.log_table = e->d_log_table; e->dp.log_table_n = RLB_LOG_TABLE_N;
+    }
+    e->dp.counts = e->d_counts;
+    return RLB_OK;
+}
+
 // (re)build the selector state: UniformEpsilonGreed::new / UpperConfidenceBound::new
 rlb_status install_selector(rlb_engine* e, int kind) {
     const uint64_t N = e->cfg.n_agents;
@@ -406,19 +501,68 @@ rlb_status install_selector(rlb_engine* e, int kind) {
     CK(fill_eps_initial(e));
     CK(fill<uint64_t>(e, e->d_ucb_t, N, 1ull));
     if (kind == RLB_SEL_UCB) {
-        if (!e->d_counts) {
-            e->counts_bytes = (size_t)N * e->S * e->APAD * sizeof(uint32_t);
-            CK(cudaMalloc(&e->d_counts, e->counts_bytes));
-        }
+        rlb_status st = ensure_ucb_buffers(e, nullptr);
+        if (st != RLB_OK) return st;
         CK(cudaMemsetAsync(e->d_counts, 0, e->counts_bytes, e->stream));
-        if (!e->d_log_table) {   // ln(t) table of the UCB bonus
-            CK(cudaMalloc(&e->d_log_table, (size_t)RLB_LOG_TABLE_N * sizeof(double)));
-            k_fill_log_table<<<(RLB_LOG_TABLE_N + 255) / 256, 256, 0, e->stream>>>(e->d_log_table, RLB_LOG_TABLE_N);
-            CK(cudaGetLastError());
-            e->dp.log_table = e->d_log_table; e->dp.log_table_n = RLB_LOG_TABLE_N;
-        }
     }
     e->dp.counts = e->d_counts;
+    return RLB_OK;
+}
+
+// per-set selectors are in force: some set's selector differs from the engine-wide one
+bool sel_per_set(const rlb_engine* e) {
+    for (int32_t k : e->h_hp_sel) if (k != e->cfg.selector_kind) return true;
+    return false;
+}
+bool any_set_ucb(const rlb_engine* e) { return std::find(e->h_hp_sel.begin(), e->h_hp_sel.end(), RLB_SEL_UCB) != e->h_hp_sel.end(); }
+
+// The per-selector agent counts and, while both selectors have agents, their lists (d_hp_order filtered by the set's
+// selector, and by the active-set mask for d_sel_run).  After any change of the sets, their selectors or the mask.
+rlb_status rebuild_selector_lists(rlb_engine* e) {
+    CK(cudaStreamSynchronize(e->stream));   // the kernels that read the old lists have completed (ENTER): drain the stream
+    if (e->d_sel_all) cudaFree(e->d_sel_all);
+    if (e->d_sel_run) cudaFree(e->d_sel_run);
+    e->d_sel_all = nullptr; e->d_sel_run = nullptr;
+    for (int k = 0; k < 2; ++k) e->n_sel_all[k] = e->n_sel_run[k] = 0;
+    if (!e->hp_n) return RLB_OK;
+    const bool masked = !e->hp_active.empty();
+    for (uint32_t g = 0; g < e->hp_n; ++g) {
+        const uint64_t n = e->h_hp_offsets[g + 1] - e->h_hp_offsets[g];
+        e->n_sel_all[e->h_hp_sel[g]] += n;
+        if (!masked || e->hp_active[g]) e->n_sel_run[e->h_hp_sel[g]] += n;
+    }
+    if (!e->n_sel_all[0] || !e->n_sel_all[1]) return RLB_OK;   // one selector: the lists of every set and of the active ones serve
+    std::vector<uint32_t> all, run;
+    for (int k = 0; k < 2; ++k)
+        for (uint32_t g = 0; g < e->hp_n; ++g) {
+            if (e->h_hp_sel[g] != k) continue;
+            auto b = e->h_hp_order.begin() + e->h_hp_offsets[g], en = e->h_hp_order.begin() + e->h_hp_offsets[g + 1];
+            all.insert(all.end(), b, en);
+            if (masked && e->hp_active[g]) run.insert(run.end(), b, en);
+        }
+    CK(cudaMalloc(&e->d_sel_all, all.size() * sizeof(uint32_t)));
+    CK(cudaMemcpyAsync(e->d_sel_all, all.data(), all.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
+    if (masked) {
+        CK(cudaMalloc(&e->d_sel_run, std::max<size_t>(run.size(), 1) * sizeof(uint32_t)));
+        if (!run.empty()) CK(cudaMemcpyAsync(e->d_sel_run, run.data(), run.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
+    }
+    CK(cudaStreamSynchronize(e->stream));
+    return RLB_OK;
+}
+
+// every set on the engine-wide selector (rlb_engine_set_hparams, rlb_agent_set_action_selector)
+rlb_status reset_set_selectors(rlb_engine* e) {
+    e->h_hp_sel.assign(e->hp_n, e->cfg.selector_kind);
+    if (e->hp_n) CK(cudaMemcpyAsync(e->d_hp_sel, e->h_hp_sel.data(), e->hp_n * sizeof(int32_t), cudaMemcpyHostToDevice, e->stream));
+    return rebuild_selector_lists(e);   // synchronous: h_hp_sel is read before it returns
+}
+
+// launch_selector_fresh with per-set modes (bit 0: epsilon, bit 1: UCB t and counts)
+rlb_status selector_fresh(rlb_engine* e, const std::vector<uint8_t>& mode) {
+    CK(cudaMemcpyAsync(e->d_sel_mode, mode.data(), mode.size(), cudaMemcpyHostToDevice, e->stream));
+    CK(launch_selector_fresh(e->d_sel_mode, e->d_hp_group, e->cfg.n_agents, e->d_hp_eps0, e->d_eps, e->d_ucb_t, e->d_counts,
+                             (uint64_t)e->S * e->APAD, e->stream));
+    CK(cudaStreamSynchronize(e->stream));   // `mode` may go
     return RLB_OK;
 }
 
@@ -846,8 +990,11 @@ void rlb_engine_destroy(rlb_engine* e) {
                     e->d_trans, e->d_thr, e->d_thr_state, e->d_totals, e->d_flagword, e->d_episodes, e->d_sums,
                     e->d_model_ent, e->d_model_bits, e->d_model_len, e->d_hp_sets, e->d_hp_group, e->d_hp_order, e->d_hp_offsets,
                     e->d_hp_q0, e->d_hp_eps0, e->d_hp_run, e->d_hp_run_offsets, e->d_hp_planning,
-                    e->d_hp_targets};
+                    e->d_hp_targets, e->d_hp_sel, e->d_sel_mode, e->d_sel_all, e->d_sel_run};
     for (void* b : bufs) if (b) cudaFree(b);
+    if (e->aux_stream) { cudaStreamSynchronize(e->aux_stream); cudaStreamDestroy(e->aux_stream); }
+    if (e->ev_fork) cudaEventDestroy(e->ev_fork);
+    if (e->ev_join) cudaEventDestroy(e->ev_join);
     for (void* b : e->d_stage) if (b) cudaFree(b);
     if (e->ev0) cudaEventDestroy(e->ev0);
     if (e->ev1) cudaEventDestroy(e->ev1);
@@ -923,11 +1070,12 @@ rlb_status rlb_engine_set_hparams(rlb_engine* e, const rlb_hparams* sets, uint32
     // release the old sets (the kernels that read them have completed: ENTER waited for pending calls, and the stream
     // is drained before the buffers go)
     CK(cudaStreamSynchronize(e->stream));
+    const bool had_ucb_sets = any_set_ucb(e);
     void* old[] = {e->d_hp_sets, e->d_hp_group, e->d_hp_order, e->d_hp_offsets, e->d_hp_q0, e->d_hp_eps0, e->d_hp_run, e->d_hp_run_offsets,
-                   e->d_hp_targets};
+                   e->d_hp_targets, e->d_hp_sel, e->d_sel_mode};
     for (void* b : old) if (b) cudaFree(b);
     e->d_hp_sets = nullptr; e->d_hp_group = nullptr; e->d_hp_order = nullptr; e->d_hp_offsets = nullptr;
-    e->d_hp_q0 = nullptr; e->d_hp_eps0 = nullptr; e->d_hp_targets = nullptr;
+    e->d_hp_q0 = nullptr; e->d_hp_eps0 = nullptr; e->d_hp_targets = nullptr; e->d_hp_sel = nullptr; e->d_sel_mode = nullptr;
     e->h_hp_targets.clear();
     e->d_hp_run = nullptr; e->d_hp_run_offsets = nullptr; e->hp_n_run = 0;
     e->hp_active.clear();   // every set active again
@@ -947,6 +1095,8 @@ rlb_status rlb_engine_set_hparams(rlb_engine* e, const rlb_hparams* sets, uint32
         CK(cudaMalloc(&e->d_hp_q0, (size_t)n_sets * e->real_size));
         CK(cudaMalloc(&e->d_hp_eps0, (size_t)n_sets * sizeof(double)));
         CK(cudaMalloc(&e->d_hp_targets, (size_t)n_sets * sizeof(int32_t)));
+        CK(cudaMalloc(&e->d_hp_sel, (size_t)n_sets * sizeof(int32_t)));
+        CK(cudaMalloc(&e->d_sel_mode, n_sets));
         CK(cudaMemcpyAsync(e->d_hp_group, h_group.data(), N * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
         CK(cudaMemcpyAsync(e->d_hp_order, order.data(), N * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
         CK(cudaMemcpyAsync(e->d_hp_offsets, offsets.data(), (size_t)(n_sets + 1) * sizeof(uint32_t), cudaMemcpyHostToDevice, e->stream));
@@ -964,6 +1114,10 @@ rlb_status rlb_engine_set_hparams(rlb_engine* e, const rlb_hparams* sets, uint32
     CK(fill<uint8_t>(e, e->d_flag, N, (uint8_t)1));
     CK(cudaMemsetAsync(e->d_nvis, 0, N * sizeof(uint32_t), e->stream));
     rlb_status st = install_selector(e, e->cfg.selector_kind);
+    if (st != RLB_OK) return st;
+    // every set on the engine-wide selector; the rows of agents that were in UCB sets zero again under eps-greedy
+    if (had_ucb_sets && e->cfg.selector_kind == RLB_SEL_EPS_GREEDY) CK(cudaMemsetAsync(e->d_counts, 0, e->counts_bytes, e->stream));
+    st = reset_set_selectors(e);
     if (st != RLB_OK) return st;
     CK(cudaStreamSynchronize(e->stream));
     return RLB_OK;
@@ -997,7 +1151,7 @@ rlb_status rlb_engine_set_active_sets(rlb_engine* e, const uint8_t* active, uint
     if (e->d_hp_run_offsets) cudaFree(e->d_hp_run_offsets);
     e->d_hp_run = nullptr; e->d_hp_run_offsets = nullptr; e->hp_n_run = 0;
     e->hp_active.clear();
-    if (all) return RLB_OK;   // an all-ones mask is NULL: the identity launch
+    if (all) return rebuild_selector_lists(e);   // an all-ones mask is NULL: the identity launch
     // d_hp_order restricted to the active sets, in the same order: contiguous groups stay ascending id ranges
     std::vector<uint32_t> run, offsets(e->hp_n + 1, 0);
     for (uint32_t g = 0; g < e->hp_n; ++g) {
@@ -1011,7 +1165,7 @@ rlb_status rlb_engine_set_active_sets(rlb_engine* e, const uint8_t* active, uint
     CK(cudaStreamSynchronize(e->stream));
     e->hp_n_run = run.size();
     e->hp_active = std::move(mask);
-    return RLB_OK;
+    return rebuild_selector_lists(e);
 }
 
 rlb_status rlb_engine_set_planning_steps(rlb_engine* e, const uint32_t* steps, uint32_t n_sets) {
@@ -1071,6 +1225,46 @@ rlb_status rlb_engine_set_targets(rlb_engine* e, const int32_t* targets, uint32_
     return write_targets(e);
 }
 
+rlb_status rlb_engine_set_selectors(rlb_engine* e, const int32_t* selectors, uint32_t n_sets) {
+    if (!e) { set_error("engine is NULL"); return RLB_ERR_INVALID_ARG; }
+    if (!e->hp_n) { set_error("no hyper-parameter sets are installed (rlb_engine_set_hparams)"); return RLB_ERR_INVALID_ARG; }
+    if (!selectors || n_sets != e->hp_n) { set_error("selectors: one RLB_SEL_* per installed set (%u), got %u", e->hp_n, n_sets); return RLB_ERR_INVALID_ARG; }
+    ENTER(e);
+    std::vector<int32_t> h(n_sets);
+    CK(cudaMemcpy(h.data(), selectors, (size_t)n_sets * sizeof(int32_t), is_device_ptr(selectors) ? cudaMemcpyDeviceToHost : cudaMemcpyHostToHost));
+    bool uses[2] = {false, false};
+    for (uint32_t g = 0; g < n_sets; ++g) {
+        if (h[g] < RLB_SEL_EPS_GREEDY || h[g] > RLB_SEL_UCB) { set_error("selectors[%u] = %d is not an RLB_SEL_*", g, h[g]); return RLB_ERR_INVALID_ARG; }
+        uses[h[g]] = true;
+    }
+    // the on-chip stores are sized for the engine's selector when picked: each requested one must fit as it is
+    if (e->store == STORE_SMEM || e->store == STORE_HYBRID)
+        for (int k = 0; k < 2; ++k) {
+            const size_t b = uses[k] ? store_bytes(e, e->store, with_selector(e, k)) : 0;
+            if (uses[k] && (b == 0 || b > kSmemPerBlockMax)) {
+                set_error("the %s store cannot run the %s selector: %zu bytes per CTA (max %zu)", e->store == STORE_SMEM ? "thread-group" : "hybrid",
+                          k == RLB_SEL_UCB ? "UCB" : "eps-greedy", b, kSmemPerBlockMax);
+                return RLB_ERR_UNSUPPORTED;
+            }
+        }
+    std::vector<uint8_t> mode(n_sets, 0);
+    bool changed = false;
+    for (uint32_t g = 0; g < n_sets; ++g) if (h[g] != e->h_hp_sel[g]) { mode[g] = 3; changed = true; }
+    if (!changed) return RLB_OK;
+    if (uses[RLB_SEL_UCB]) {
+        bool fresh = false;
+        rlb_status st = ensure_ucb_buffers(e, &fresh);
+        if (st != RLB_OK) return st;
+        if (fresh) CK(cudaMemsetAsync(e->d_counts, 0, e->counts_bytes, e->stream));   // every eps-greedy agent's counts are zero
+    }
+    // a fresh selector of its new kind for every agent of a changed set: epsilon, t and counts as the constructors leave them
+    rlb_status st = selector_fresh(e, mode);
+    if (st != RLB_OK) return st;
+    e->h_hp_sel = std::move(h);
+    CK(cudaMemcpyAsync(e->d_hp_sel, e->h_hp_sel.data(), n_sets * sizeof(int32_t), cudaMemcpyHostToDevice, e->stream));
+    return rebuild_selector_lists(e);
+}
+
 rlb_status rlb_agent_clone(rlb_engine* e, const uint32_t* src, const uint32_t* dst, uint64_t n_pairs) {
     if (!e) { set_error("engine is NULL"); return RLB_ERR_INVALID_ARG; }
     if (!n_pairs) return RLB_OK;
@@ -1096,21 +1290,49 @@ rlb_status rlb_agent_clone(rlb_engine* e, const uint32_t* src, const uint32_t* d
     }
     for (uint64_t j = 0; j < n_pairs; ++j)
         if (is_dst[ids[j]]) { set_error("agent %u is both a source and a destination", ids[j]); return RLB_ERR_INVALID_ARG; }
+    // Per-set selectors: a destination keeps its set's selector, so the counts go only to destinations of UCB sets (an
+    // eps-greedy agent's counts stay zero).  Those pairs first, then the others, in two launches.
+    const bool by_dst = sel_per_set(e);
+    uint64_t n_counts = e->cfg.selector_kind == RLB_SEL_UCB ? n_pairs : 0;   // the first n_counts pairs copy the counts
+    if (by_dst) {
+        std::vector<uint8_t> ucb(N, 0);   // agent -> its set is UCB
+        for (uint32_t g = 0; g < e->hp_n; ++g)
+            if (e->h_hp_sel[g] == RLB_SEL_UCB)
+                for (uint32_t k = e->h_hp_offsets[g]; k < e->h_hp_offsets[g + 1]; ++k) ucb[e->h_hp_order[k]] = 1;
+        std::vector<uint32_t> sorted(2 * n_pairs);
+        n_counts = 0;
+        for (int pass = 0; pass < 2; ++pass) {
+            uint64_t k = pass ? n_counts : 0;
+            for (uint64_t j = 0; j < n_pairs; ++j) {
+                if ((ucb[ids[n_pairs + j]] != 0) != (pass == 0)) continue;
+                sorted[k] = ids[j]; sorted[n_pairs + k] = ids[n_pairs + j]; ++k;
+            }
+            if (pass == 0) n_counts = k;
+        }
+        ids.swap(sorted);
+    }
     const void* d_ids;
     CK(stage_in(e, 0, ids.data(), 2 * n_pairs * 4, &d_ids));
     CloneArgs a{};
     // whole padded rows: the round trip moves only the A real columns, but padding exists only under -DRLB_TAXI_APAD=8,
     // and load_row / store_row read and write the first A columns of a row alone, so what the padding holds is never used
     a.seg[a.n_seg++] = CloneSegment{(uint8_t*)e->d_q, e->q_bytes / N};
-    if (e->cfg.selector_kind == RLB_SEL_UCB) a.seg[a.n_seg++] = CloneSegment{(uint8_t*)e->d_counts, e->counts_bytes / N};
+    if (n_counts) a.seg[a.n_seg++] = CloneSegment{(uint8_t*)e->d_counts, e->counts_bytes / N};
     if (e->cfg.planning_steps) {
         a.seg[a.n_seg++] = CloneSegment{(uint8_t*)e->d_model_ent, (uint64_t)e->dp.mcap * sizeof(uint2)};
         a.seg[a.n_seg++] = CloneSegment{(uint8_t*)e->d_model_bits, (uint64_t)e->dp.mwords * sizeof(uint32_t)};
         a.model_len = e->d_model_len;
     }
-    a.src = (const uint32_t*)d_ids; a.dst = a.src + n_pairs; a.n_pairs = n_pairs;
+    a.src = (const uint32_t*)d_ids; a.dst = a.src + n_pairs; a.n_pairs = n_counts ? n_counts : n_pairs;
     a.eps = e->d_eps; a.ucb_t = e->d_ucb_t; a.flag = e->d_flag;
     CK(launch_clone_agents(a, e->stream));
+    if (n_counts && n_counts < n_pairs) {   // the pairs whose destination is eps-greedy: everything but the counts
+        CloneArgs b = a;
+        b.n_seg = 0;
+        for (uint32_t k = 0; k < a.n_seg; ++k) if (a.seg[k].base != (uint8_t*)e->d_counts) b.seg[b.n_seg++] = a.seg[k];
+        b.src = a.src + n_counts; b.dst = a.dst + n_counts; b.n_pairs = n_pairs - n_counts;
+        CK(launch_clone_agents(b, e->stream));
+    }
     CK(cudaStreamSynchronize(e->stream));
     return RLB_OK;
 }
@@ -1252,8 +1474,14 @@ rlb_status rlb_agent_set_future_q_value_func(rlb_engine* e, int32_t target_kind)
 rlb_status rlb_agent_set_action_selector(rlb_engine* e, int32_t selector_kind) {
     if (!e || selector_kind < 0 || selector_kind > 1) { set_error("bad selector_kind"); return RLB_ERR_INVALID_ARG; }
     ENTER(e);
+    const bool had_ucb_sets = any_set_ucb(e);
     rlb_status st = install_selector(e, selector_kind);
     if (st != RLB_OK) return st;
+    if (e->hp_n) {   // every set on selector_kind, with a fresh selector: eps-greedy agents' counts zero
+        if (had_ucb_sets && selector_kind == RLB_SEL_EPS_GREEDY) CK(cudaMemsetAsync(e->d_counts, 0, e->counts_bytes, e->stream));
+        st = reset_set_selectors(e);
+        if (st != RLB_OK) return st;
+    }
     return pick_store(e);
 }
 
@@ -1276,6 +1504,8 @@ rlb_status rlb_agent_set_kind(rlb_engine* e, int32_t agent_kind) {
     CK(cudaMemsetAsync(e->d_nvis, 0, N * sizeof(uint32_t), e->stream));
     rlb_status st = install_selector(e, e->cfg.selector_kind);
     if (st != RLB_OK) return st;
+    // per-set selectors: a fresh selector of each set's own kind (epsilon and t are filled above for every agent)
+    if (sel_per_set(e) && e->d_counts) CK(cudaMemsetAsync(e->d_counts, 0, e->counts_bytes, e->stream));
     return pick_store(e);
 }
 
@@ -1283,6 +1513,11 @@ rlb_status rlb_selector_reset(rlb_engine* e) {
     if (!e) { set_error("engine is NULL"); return RLB_ERR_INVALID_ARG; }
     ENTER(e);
     const uint64_t N = e->cfg.n_agents;
+    if (sel_per_set(e)) {   // each set's agents as its selector resets: epsilon, or t and counts
+        std::vector<uint8_t> mode(e->hp_n);
+        for (uint32_t g = 0; g < e->hp_n; ++g) mode[g] = e->h_hp_sel[g] == RLB_SEL_UCB ? 2 : 1;
+        return selector_fresh(e, mode);
+    }
     if (e->cfg.selector_kind == RLB_SEL_EPS_GREEDY) {
         CK(fill_eps_initial(e));                                                // uniform_epsilon_greed.rs:78-80
     } else {
@@ -1529,7 +1764,9 @@ rlb_status rlb_selector_get_exploration_probs(rlb_engine* e, const uint32_t* obs
 rlb_status rlb_selector_update(rlb_engine* e) {
     if (!e) { set_error("engine is NULL"); return RLB_ERR_INVALID_ARG; }
     ENTER(e);
-    if (e->cfg.selector_kind == RLB_SEL_EPS_GREEDY && e->hp_n) {   // each agent with its own k and floor
+    if (sel_per_set(e)) {   // the agents of eps-greedy sets, each with its own k and floor; UCB's update does nothing
+        CK(launch_eps_decay_selected(e->d_eps, e->cfg.n_agents, e->cfg.decay_kind, e->d_hp_sets, e->d_hp_group, e->d_hp_sel, e->stream));
+    } else if (e->cfg.selector_kind == RLB_SEL_EPS_GREEDY && e->hp_n) {   // each agent with its own k and floor
         CK(launch_eps_decay_grouped(e->d_eps, e->cfg.n_agents, e->cfg.decay_kind, e->d_hp_sets, e->d_hp_group, e->stream));
     } else if (e->cfg.selector_kind == RLB_SEL_EPS_GREEDY) {
         const uint64_t N = e->cfg.n_agents;

@@ -64,6 +64,15 @@ cudaError_t launch_eps_decay_grouped(double* eps, uint64_t n_agents, int kind, c
 cudaError_t launch_episode_sums_grouped(int real_kind, const void* records, uint64_t n_agents, const uint32_t* order,
                                         const uint32_t* offsets, uint32_t n_sets, uint64_t n_ep, double* out, cudaStream_t stream);
 
+// ---- per-set action selectors (rlb_selectors.cu, rlb_engine_set_selectors) ----
+// Per set g, by mode[g]: bit 0 epsilon = eps0[g]; bit 1 ucb_t = 1 and the agent's counts row (row_words u32, counts may
+// be nullptr) zero; 0 leaves the set's agents alone.  One launch over every agent.
+cudaError_t launch_selector_fresh(const uint8_t* mode, const uint32_t* group, uint64_t n_agents, const double* eps0, double* eps,
+                                  uint64_t* ucb_t, uint32_t* counts, uint64_t row_words, cudaStream_t stream);
+// ActionSelection::update of the agents whose set's selector (sel[group[i]]) is eps-greedy, with their set's decay
+cudaError_t launch_eps_decay_selected(double* eps, uint64_t n_agents, int kind, const rlb_hparams* sets, const uint32_t* group,
+                                      const int32_t* sel, cudaStream_t stream);
+
 // ---- agent-to-agent copies of learned state (rlb_clone.cu, rlb_agent_clone) ----
 constexpr int CLONE_MAX_SEGMENTS = 4;   // Q, UCB counts, model entries, model bits
 struct CloneSegment {

@@ -208,7 +208,8 @@ cudaError_t run_kernel_attributes(const Variant& v, int store, cudaFuncAttribute
 
 template <int ENV, bool HP>
 cudaError_t launch_step(StepOp op, const Variant& v, const DevParams& p, const StepArgs& a, cudaStream_t stream) {
-    const unsigned grid = grid_for(p.n_agents);
+    // with per-agent sets the grid covers the launch positions of a.sets (every agent, or one selector's agents)
+    const unsigned grid = grid_for(HP ? a.sets.n_launch : p.n_agents);
     const size_t smem = EnvTab<ENV>::smem_bytes(p.S);
     switch (op) {
         case OP_ENV_CONSTRUCT: k_env_construct<ENV><<<grid, kBlock, 0, stream>>>(p); break;

@@ -324,6 +324,10 @@ PLANNING_AXIS = "planning_steps"
 # the bootstrap target (Agent::set_future_q_value_func, agent.rs:48) as a categorical axis: names of TARGET_KINDS, kept
 # beside rlb_hparams (rlb_engine_set_targets)
 TARGET_AXIS = "target"
+# the action selector (Agent's ActionSelection, bin/taxi.rs:154-163) as a categorical axis: names of SELECTOR_NAMES, kept
+# beside rlb_hparams (rlb_engine_set_selectors)
+SELECTOR_AXIS = "selector"
+CATEGORICAL_AXES = {TARGET_AXIS: TARGET_KINDS, SELECTOR_AXIS: SELECTOR_NAMES}
 
 
 def planning_value(v):
@@ -340,13 +344,13 @@ def expand_grid(grid):
     for k in grid:
         if k == PLANNING_AXIS:
             grid[k] = [planning_value(v) for v in grid[k]]
-        elif k == TARGET_AXIS:
-            bad = [v for v in grid[k] if not isinstance(v, str) or v not in TARGET_KINDS]
+        elif k in CATEGORICAL_AXES:
+            bad = [v for v in grid[k] if not isinstance(v, str) or v not in CATEGORICAL_AXES[k]]
             if bad:
-                raise ValueError("target values must be among %s, got %r" % (", ".join(sorted(TARGET_KINDS)), bad))
+                raise ValueError("%s values must be among %s, got %r" % (k, ", ".join(sorted(CATEGORICAL_AXES[k])), bad))
         elif k not in SWEEP_FLAGS:
-            raise ValueError("%r cannot be swept; the agent constructor flags are %s, %s and %s"
-                             % (k, ", ".join(SWEEP_FLAGS), PLANNING_AXIS, TARGET_AXIS))
+            raise ValueError("%r cannot be swept; the agent constructor flags are %s, %s, %s and %s"
+                             % (k, ", ".join(SWEEP_FLAGS), PLANNING_AXIS, TARGET_AXIS, SELECTOR_AXIS))
     keys = list(grid)
     return [dict(zip(keys, vals)) for vals in itertools.product(*(grid[k] for k in keys))]
 
@@ -363,7 +367,9 @@ def grid_engine(env_name, grid, *, agent, selector, target, policy, agents_per_p
     `agents_per_point` constructed with the point's values (rlb_engine_set_hparams).  Returns (engine, n_episodes,
     moving-average window, points, every point's flags, every point's rlb_hparams).  With a planning_steps axis every set
     is also a Dyna-Q agent with its point's planning count (rlb_engine_set_planning_steps), and with a target axis every
-    set bootstraps with its point's target (rlb_engine_set_targets); `target` is then only the engine's configured one."""
+    set bootstraps with its point's target (rlb_engine_set_targets); `target` is then only the engine's configured one.
+    With a selector axis every set selects with its point's selector (rlb_engine_set_selectors); the engine is created
+    with UCB when the axis holds it, so that the store it picks runs both selectors."""
     f = dict(DEFAULTS)
     f.update(flags)
     n = int(f["n_episodes"])
@@ -378,6 +384,8 @@ def grid_engine(env_name, grid, *, agent, selector, target, policy, agents_per_p
     if len(sets) > abi.MAX_HPARAM_SETS:
         raise ValueError("%d grid points; an engine holds at most %d sets" % (len(sets), abi.MAX_HPARAM_SETS))
     env = make_env(env_name, **f)
+    if SELECTOR_AXIS in grid and "ucb" in grid[SELECTOR_AXIS]:
+        selector = "ucb"
     eng = abi.Engine(env.kind, n_agents=len(points) * int(agents_per_point), policy=abi.POLICY_BASIC if policy == "basic" else abi.POLICY_DOUBLE,
                      selector=SELECTOR_NAMES[selector], target=TARGET_KINDS[target], agent=AGENT_NAMES[agent],
                      real=abi.REAL_F32 if real == "f32" else abi.REAL_F64, decay_kind=abi.DECAY_SUB, seed=seed, device=device,
@@ -388,6 +396,8 @@ def grid_engine(env_name, grid, *, agent, selector, target, policy, agents_per_p
             eng.set_planning_steps(np.array([pf[PLANNING_AXIS] for pf in point_flags], np.uint32))
         if TARGET_AXIS in grid:
             eng.set_targets(point_targets(point_flags))
+        if SELECTOR_AXIS in grid:
+            eng.set_selectors(point_selectors(point_flags))
     except BaseException:
         eng.close()
         raise
@@ -402,6 +412,16 @@ def point_targets(point_flags):
 def engine_target(grid, target):
     """The `target` of a result: the engine-wide name, or None where a target axis gives each point its own."""
     return None if TARGET_AXIS in grid else target
+
+
+def point_selectors(point_flags):
+    """Every point's selector name as the RLB_SEL_* array rlb_engine_set_selectors takes."""
+    return np.array([SELECTOR_NAMES[pf[SELECTOR_AXIS]] for pf in point_flags], np.int32)
+
+
+def engine_selector(grid, selector):
+    """The `selector` of a result: the engine-wide name, or None where a selector axis gives each point its own."""
+    return None if SELECTOR_AXIS in grid else selector
 
 
 def point_results(points, sets, train_sums, eval_sums, agents_per_point, n, window):
@@ -443,7 +463,7 @@ def run_sweep(env_name, grid, *, agent="onestep", selector="eps", target="qlearn
                                                                                   res["train_steps"] / dt if dt > 0 else 0.0))
         for g in ranking[:10]:
             print("  %-60s evaluate mean return %.4f" % (points[g], out_points[g]["eval_mean_return"]))
-    return dict(env=env_name, agent=agent, selector=selector, target=engine_target(grid, target), policy=policy, real=real, n_episodes=n,
+    return dict(env=env_name, agent=agent, selector=engine_selector(grid, selector), target=engine_target(grid, target), policy=policy, real=real, n_episodes=n,
                 agents_per_point=int(agents_per_point), grid={k: list(v) for k, v in grid.items()}, points=out_points,
                 ranking=ranking, seconds=dt, train_steps=int(res["train_steps"]))
 
@@ -462,7 +482,8 @@ def sweep_parser(description):
     ap = argparse.ArgumentParser(description=description)
     ap.add_argument("env", choices=["blackjack", "frozen_lake", "cliffwalking", "taxi"])
     ap.add_argument("--grid", action="append", default=[], metavar="FLAG=V1,V2,...",
-                    help="a bin flag and its values (repeatable; one of %s, %s, %s)" % (", ".join(SWEEP_FLAGS), PLANNING_AXIS, TARGET_AXIS))
+                    help="a bin flag and its values (repeatable; one of %s, %s, %s, %s)" % (", ".join(SWEEP_FLAGS), PLANNING_AXIS, TARGET_AXIS,
+                                                                                             SELECTOR_AXIS))
     for name in SWEEP_FLAGS:
         ap.add_argument("--" + name, default=None, metavar="V1,V2,...", help="values of this flag (a comma list: a grid axis)")
     ap.add_argument("--" + PLANNING_AXIS, default=None, metavar="K1,K2,...",
@@ -473,7 +494,8 @@ def sweep_parser(description):
     ap.add_argument("--stochastic_env", action="store_true")
     ap.add_argument("--map", default="4x4")
     ap.add_argument("--agent", choices=sorted(AGENT_NAMES), default="onestep")
-    ap.add_argument("--selector", choices=sorted(SELECTOR_NAMES), default="eps")
+    ap.add_argument("--selector", default="eps", metavar="NAME[,NAME...]",
+                    help="action selector, one of %s: one name for every agent, or a comma list (a grid axis)" % ", ".join(sorted(SELECTOR_NAMES)))
     ap.add_argument("--target", default="qlearning", metavar="NAME[,NAME...]",
                     help="bootstrap target, one of %s: one name for every agent, or a comma list (a grid axis)" % ", ".join(sorted(TARGET_KINDS)))
     ap.add_argument("--policy", choices=["basic", "double"], default="basic")
@@ -495,17 +517,18 @@ def parse_sweep_args(ap, argv):
         except ValueError:
             ap.error("--%s takes non-negative integers, got %r" % (PLANNING_AXIS, text))
 
-    def target_list(text):
+    def name_list(axis, text):
         names = parse_names(text)
-        if not names or any(x not in TARGET_KINDS for x in names):
-            ap.error("--%s takes names among %s, got %r" % (TARGET_AXIS, ", ".join(sorted(TARGET_KINDS)), text))
+        if not names or any(x not in CATEGORICAL_AXES[axis] for x in names):
+            ap.error("--%s takes names among %s, got %r" % (axis, ", ".join(sorted(CATEGORICAL_AXES[axis])), text))
         return names
 
     grid = {}
-    targets = target_list(a["target"])
-    if len(targets) > 1:   # a comma list is an axis; a single name stays engine-wide
-        grid[TARGET_AXIS] = targets
-        a["target"] = targets[0]
+    for axis in (TARGET_AXIS, SELECTOR_AXIS):
+        names = name_list(axis, a[axis])
+        if len(names) > 1:   # a comma list is an axis; a single name stays engine-wide
+            grid[axis] = names
+        a[axis] = names[0]
     for name in SWEEP_FLAGS:
         v = a.pop(name)
         if v is not None:
@@ -520,12 +543,12 @@ def parse_sweep_args(ap, argv):
         if k == PLANNING_AXIS:
             grid[k] = planning_list(v)
             continue
-        if k == TARGET_AXIS:
-            grid[k] = target_list(v)
-            a["target"] = grid[k][0]
+        if k in CATEGORICAL_AXES:
+            grid[k] = name_list(k, v)
+            a[k] = grid[k][0]
             continue
         if k not in SWEEP_FLAGS:
-            ap.error("--grid %s: not a sweepable flag (%s, %s, %s)" % (k, ", ".join(SWEEP_FLAGS), PLANNING_AXIS, TARGET_AXIS))
+            ap.error("--grid %s: not a sweepable flag (%s, %s, %s, %s)" % (k, ", ".join(SWEEP_FLAGS), PLANNING_AXIS, TARGET_AXIS, SELECTOR_AXIS))
         grid[k] = parse_list(v)
     if not grid:
         ap.error("nothing to sweep: give at least one --grid FLAG=V1,V2,...")
@@ -575,18 +598,19 @@ def pbt_perturb_planning(k, f):
     return out
 
 
-def pbt_explore(flags, axes, rng, targets=None, resample_probability=0.25):
+def pbt_explore(flags, axes, rng, targets=None, resample_probability=0.25, selectors=None):
     """The winner's flags with every numeric grid axis multiplied by 0.8 or 1.2 at random and clamped into its range (the
-    planning count as an integer: pbt_perturb_planning).  A target axis is inherited, and with probability
-    `resample_probability` redrawn uniformly from `targets` (the axis values).  Without a target axis the draws are
-    those of the numeric axes alone."""
+    planning count as an integer: pbt_perturb_planning).  A target or selector axis is inherited, and with probability
+    `resample_probability` redrawn uniformly from `targets` / `selectors` (the axis values), in the axis' place among the
+    draws.  Without those axes the draws are those of the numeric axes alone."""
     out = dict(flags)
     for k in axes:
-        if k == TARGET_AXIS:
-            if targets is None:
-                raise ValueError("a target axis needs its values (targets=) to resample from")
+        if k in CATEGORICAL_AXES:
+            values = targets if k == TARGET_AXIS else selectors
+            if values is None:
+                raise ValueError("a %s axis needs its values (%ss=) to resample from" % (k, k))
             if rng.random() < resample_probability:
-                out[k] = targets[int(rng.integers(len(targets)))]
+                out[k] = values[int(rng.integers(len(values)))]
             continue
         f = PBT_FACTORS[int(rng.integers(2))]
         if k == PLANNING_AXIS:
@@ -604,8 +628,10 @@ def run_pbt(env_name, grid, *, interval, fraction=0.25, pbt_seed=0x9B7, resample
     After every chunk but the last the sets are ranked by their mean training return over the chunk; each of the bottom
     floor(fraction * G) sets takes over the learned state of a set drawn from the top as many (agent j of the winner ->
     agent j of the loser, one rlb_agent_clone) and continues with the winner's flags, every numeric grid axis perturbed
-    (rlb_engine_retune_hparams) and a target axis inherited, or with probability `resample_probability` redrawn from the
-    axis values (rlb_engine_set_targets).  `pbt_seed` seeds those draws.  Returns run_sweep's output plus every set's final flags
+    (rlb_engine_retune_hparams) and a target or selector axis inherited, or with probability `resample_probability`
+    redrawn from the axis values (rlb_engine_set_targets, rlb_engine_set_selectors).  An inherited selector is given to the
+    loser before the clone, so that the winner's selector state lands on the right kind; a redrawn one that differs
+    gives the loser a fresh selector after it.  `pbt_seed` seeds those draws.  Returns run_sweep's output plus every set's final flags
     and the lineage: per chunk boundary, the list of (loser, winner, new flags)."""
     if not 0.0 <= fraction <= 0.5:
         raise ValueError("fraction must be in [0, 0.5]: the top and bottom sets may not overlap")
@@ -633,18 +659,24 @@ def run_pbt(env_name, grid, *, interval, fraction=0.25, pbt_seed=0x9B7, resample
                 break
             pairs = pbt_exploit(res["sums"], fraction, rng)
             step = []
+            inherited = [c.get(SELECTOR_AXIS) for c in cur]
             for loser, winner in pairs:
-                cur[loser] = pbt_explore(cur[winner], axes, rng, grid.get(TARGET_AXIS), resample_probability)
+                inherited[loser] = cur[winner].get(SELECTOR_AXIS)
+                cur[loser] = pbt_explore(cur[winner], axes, rng, grid.get(TARGET_AXIS), resample_probability, grid.get(SELECTOR_AXIS))
                 sets[loser] = point_hparams(cur[loser], n)
                 step.append(dict(loser=loser, winner=winner, flags={k: cur[loser][k] for k in axes}))
             if pairs:
                 j = np.arange(per, dtype=np.int64)
+                if SELECTOR_AXIS in axes:   # the winners' selectors first: the clone then copies their state onto the same kind
+                    eng.set_selectors(point_selectors([{SELECTOR_AXIS: k} for k in inherited]))
                 eng.clone_agents(np.concatenate([w * per + j for _, w in pairs]), np.concatenate([l * per + j for l, _ in pairs]))
                 eng.retune_hparams(sets)
                 if PLANNING_AXIS in axes:
                     eng.set_planning_steps(np.array([c[PLANNING_AXIS] for c in cur], np.uint32))
                 if TARGET_AXIS in axes:
                     eng.set_targets(point_targets(cur))
+                if SELECTOR_AXIS in axes and [c[SELECTOR_AXIS] for c in cur] != inherited:   # redrawn: a fresh selector
+                    eng.set_selectors(point_selectors(cur))
             lineage.append(dict(episode=end, pairs=step))
         ev = eng.evaluate(n, sums=True)["sums"]                                                      # [n, G, 4]
         dt = time.perf_counter() - t0
@@ -657,9 +689,9 @@ def run_pbt(env_name, grid, *, interval, fraction=0.25, pbt_seed=0x9B7, resample
         print("PBT: %d sets x %d agents, %d episodes in chunks of %d, fraction %.3g: %.2fs" % (len(points), per, n, interval, fraction, dt))
         for g in ranking[:10]:
             print("  set %-4d %-60s evaluate mean return %.4f" % (g, out_points[g]["final_params"], out_points[g]["eval_mean_return"]))
-    return dict(env=env_name, agent=agent, selector=selector, target=engine_target(grid, target), policy=policy, real=real, n_episodes=n,
+    return dict(env=env_name, agent=agent, selector=engine_selector(grid, selector), target=engine_target(grid, target), policy=policy, real=real, n_episodes=n,
                 agents_per_point=per, grid={k: list(v) for k, v in grid.items()}, interval=interval, fraction=fraction,
-                pbt_seed=int(pbt_seed), **({"resample_probability": resample_probability} if TARGET_AXIS in grid else {}), points=out_points, ranking=ranking, lineage=lineage, seconds=dt, train_steps=train_steps)
+                pbt_seed=int(pbt_seed), **({"resample_probability": resample_probability} if TARGET_AXIS in grid or SELECTOR_AXIS in grid else {}), points=out_points, ranking=ranking, lineage=lineage, seconds=dt, train_steps=train_steps)
 
 
 def main_pbt(argv=None):
@@ -669,7 +701,7 @@ def main_pbt(argv=None):
     ap.add_argument("--fraction", type=float, default=0.25, help="share of the sets replaced after each chunk (and drawn from)")
     ap.add_argument("--pbt_seed", type=lambda x: int(x, 0), default=0x9B7, help="seed of the winner draws and perturbations")
     ap.add_argument("--resample_probability", type=float, default=0.25,
-                    help="with a target axis: chance that a loser's inherited target is redrawn from the axis values")
+                    help="with a target or selector axis: chance that a loser's inherited value is redrawn from the axis values")
     env_name, grid, outp, kw = parse_sweep_args(ap, argv)
     res = run_pbt(env_name, grid, **kw)
     write_json(res, outp)
@@ -754,7 +786,7 @@ def run_halving(env_name, grid, *, min_episodes, eta=3, agent="onestep", selecto
               % (n_sets, per, n, budgets, int(eta), dt, train_steps))
         for g in ranking[:min(10, len(survivors))]:
             print("  set %-4d %-60s evaluate mean return %.4f" % (g, points[g], out_points[g]["eval_mean_return"]))
-    return dict(env=env_name, agent=agent, selector=selector, target=engine_target(grid, target), policy=policy, real=real, n_episodes=n,
+    return dict(env=env_name, agent=agent, selector=engine_selector(grid, selector), target=engine_target(grid, target), policy=policy, real=real, n_episodes=n,
                 agents_per_point=per, grid={k: list(v) for k, v in grid.items()}, min_episodes=int(min_episodes), eta=int(eta),
                 points=out_points, ranking=ranking, rungs=rungs, seconds=dt, train_steps=train_steps)
 

@@ -3,8 +3,8 @@ The complete state is: Q tables, UCB counts, and per agent the RNG word index, e
 (rlb_download_tables / rlb_get_agent_states), plus the Dyna model when one is attached (rlb_download_model) and the
 per-agent hyper-parameter sets when they are installed (rlb_engine_set_hparams), with the active-set mask while some
 set is paused (rlb_engine_set_active_sets), the per-set planning counts while they are in force
-(rlb_engine_set_planning_steps) and the per-set targets while they are (rlb_engine_set_targets).  Stored as one .npz; the configuration
-is stored beside it and checked."""
+(rlb_engine_set_planning_steps), the per-set targets while they are (rlb_engine_set_targets) and the per-set selectors
+while they are (rlb_engine_set_selectors).  Stored as one .npz; the configuration is stored beside it and checked."""
 import ctypes as C
 
 import numpy as np
@@ -28,6 +28,8 @@ def save_snapshot(engine, path):
             extra["hp_active"] = np.asarray(engine.active_sets, np.uint8)
         if engine.targets is not None:
             extra["hp_target"] = np.asarray(engine.targets, np.int32)
+        if engine.selectors is not None:
+            extra["hp_selector"] = np.asarray(engine.selectors, np.int32)
     q, counts = engine.download_tables()
     cfg = {k: int(getattr(engine.cfg, k)) for k in _CFG_FIELDS}
     np.savez_compressed(path, q=q, counts=counts, states=engine.states(), selector_kind=np.int64(engine.cfg.selector_kind),
@@ -49,7 +51,10 @@ def load_snapshot(engine, path):
         engine.set_hparams(z["hp_sets"], z["hp_group"])
     elif engine.G:
         engine.set_hparams(None, None)
-    has_counts = int(z["selector_kind"]) == 1
+    # the selectors before the tables and states: a change gives the changed sets a fresh selector
+    if "hp_selector" in z.files:
+        engine.set_selectors(z["hp_selector"])
+    has_counts = int(z["selector_kind"]) == 1 or ("hp_selector" in z.files and bool((z["hp_selector"] == 1).any()))
     engine.upload_tables(z["q"], z["counts"] if has_counts else None)
     engine.set_states(z["states"])
     planning = int(z["planning_steps"]) if "planning_steps" in z.files else 0

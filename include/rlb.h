@@ -176,8 +176,11 @@ typedef struct rlb_train_out {
     uint64_t eval_steps;         /* out: steps executed inside the injected evaluate(100) calls */
     double eval_return_sum;      /* out: sum of returns of those evaluate episodes */
     uint64_t eval_episodes;      /* out */
-    float kernel_ms;             /* out: device time of the fused kernel launches (CUDA events) */
-    uint32_t kernel_launches;    /* out */
+    float kernel_ms;             /* out: device time of the kernel launches (CUDA events): k_run, and the k_eval launches
+                                    of the evaluate blocks of the thread-group and hybrid stores */
+    uint32_t kernel_launches;    /* out: kernel launches (with per-set selectors: launch pairs); an on-chip store's
+                                    engine of >= 2^17 agents makes one k_run launch per training segment and one k_eval
+                                    launch per evaluate block */
     uint64_t trace_rows;         /* out: eligibility rows swept (elegibility_traces_agent.rs:86), for the roofline */
     /* `training_error` (agent.rs:73,98,117): the temporal difference of EVERY training step, in step order, episodes
      * concatenated — [n_agents][td_capacity] Real; td_count [n_agents] u64 receives the number of training steps each

@@ -134,6 +134,7 @@ struct rlb_engine {
         unsigned long long* h_totals = nullptr;      // pinned [8]
         bool pipelined = false;
         bool host_records = false;                   // the call copies per-agent records to a host buffer
+        uint32_t launches = 0;                       // k_run / k_eval dispatches (one per selector partition pair)
         rlb_traj_record* d_traj = nullptr; uint64_t* d_traj_count = nullptr; bool own_traj = false, own_count = false;
         void* d_td = nullptr; uint64_t* d_td_count = nullptr; bool own_td = false, own_td_count = false;
     };
@@ -224,8 +225,15 @@ cudaError_t fill_eps_initial(rlb_engine* e) {
 #define RLB_SEL_CONCURRENT 1   // the two selectors' launches on two streams (0: back to back on the engine's stream)
 #endif
 
-// k_run_hp (with the model: its Dyna twin) over the launch positions of h, with selector v.sel
-cudaError_t launch_run_hp(rlb_engine* e, const DevParams& p, const Variant& v, const HpParams& h, cudaStream_t stream) {
+// k_run_hp (with the model: its Dyna twin; eval: k_eval's twin) over the launch positions of h, with selector v.sel
+cudaError_t launch_run_hp(rlb_engine* e, const DevParams& p, const Variant& v, const HpParams& h, cudaStream_t stream, bool eval) {
+    if (eval) {
+        switch (e->cfg.env_kind) {
+            case RLB_ENV_FROZEN_LAKE: return launch_eval<RLB_ENV_FROZEN_LAKE, true>(v, p, stream, h);
+            case RLB_ENV_CLIFF_WALKING: return launch_eval<RLB_ENV_CLIFF_WALKING, true>(v, p, stream, h);
+            default: return cudaErrorInvalidValue;
+        }
+    }
     if (p.planning_steps && p.mode == 0) {   // the model under sets: each set's own planning count
         switch (e->cfg.env_kind) {
             case RLB_ENV_BLACKJACK: return launch_run_model<RLB_ENV_BLACKJACK, true>(v, p, stream, h);
@@ -249,13 +257,14 @@ Variant with_selector(const rlb_engine* e, int sel) {
     return v;
 }
 
-cudaError_t dispatch_run(rlb_engine* e, const DevParams& p) {
+// eval: k_eval in place of k_run (the evaluate blocks of the on-chip stores, run_chunk)
+cudaError_t dispatch_run(rlb_engine* e, const DevParams& p, bool eval = false) {
     if (e->hp_n) {
         const bool masked = !e->hp_active.empty();   // only the active sets' agents run: a launch sized to them
         HpParams sets{e->d_hp_sets, e->d_hp_group, masked ? e->d_hp_run : nullptr, masked ? e->hp_n_run : e->cfg.n_agents, e->d_hp_planning,
                       e->d_hp_targets, 0};
         if (!e->n_sel_run[0] || !e->n_sel_run[1])   // one selector among the running agents: one launch, as without per-set selectors
-            return launch_run_hp(e, p, with_selector(e, e->n_sel_run[1] ? RLB_SEL_UCB : e->n_sel_run[0] ? RLB_SEL_EPS_GREEDY : e->variant.sel), sets, e->stream);
+            return launch_run_hp(e, p, with_selector(e, e->n_sel_run[1] ? RLB_SEL_UCB : e->n_sel_run[0] ? RLB_SEL_EPS_GREEDY : e->variant.sel), sets, e->stream, eval);
         // one launch per selector over its agents' list; the second's positions start at a multiple of 32 past the
         // first's, so that the hybrid store's scratch rows (addressed by position) of the two never meet
         const uint32_t* lists = masked ? e->d_sel_run : e->d_sel_all;
@@ -276,8 +285,8 @@ cudaError_t dispatch_run(rlb_engine* e, const DevParams& p) {
         if (err != cudaSuccess) return err;
         s2 = e->aux_stream;
 #endif
-        cudaError_t err0 = launch_run_hp(e, p, with_selector(e, RLB_SEL_EPS_GREEDY), sets, e->stream);
-        cudaError_t err1 = launch_run_hp(e, p, with_selector(e, RLB_SEL_UCB), second, s2);
+        cudaError_t err0 = launch_run_hp(e, p, with_selector(e, RLB_SEL_EPS_GREEDY), sets, e->stream, eval);
+        cudaError_t err1 = launch_run_hp(e, p, with_selector(e, RLB_SEL_UCB), second, s2, eval);
 #if RLB_SEL_CONCURRENT
         cudaError_t err2 = cudaEventRecord(e->ev_join, e->aux_stream);   // everything after dispatch_run sees one stream
         if (err2 == cudaSuccess) err2 = cudaStreamWaitEvent(e->stream, e->ev_join, 0);
@@ -293,12 +302,72 @@ cudaError_t dispatch_run(rlb_engine* e, const DevParams& p) {
             default: return launch_run_model<RLB_ENV_TAXI>(e->variant, p, e->stream);
         }
     }
+    if (eval) {
+        switch (e->cfg.env_kind) {
+            case RLB_ENV_FROZEN_LAKE: return launch_eval<RLB_ENV_FROZEN_LAKE>(e->variant, p, e->stream);
+            case RLB_ENV_CLIFF_WALKING: return launch_eval<RLB_ENV_CLIFF_WALKING>(e->variant, p, e->stream);
+            default: return cudaErrorInvalidValue;
+        }
+    }
     switch (e->cfg.env_kind) {
         case RLB_ENV_BLACKJACK: return launch_run<RLB_ENV_BLACKJACK>(e->variant, p, e->store, e->stream);
         case RLB_ENV_FROZEN_LAKE: return launch_run<RLB_ENV_FROZEN_LAKE>(e->variant, p, e->store, e->stream);
         case RLB_ENV_CLIFF_WALKING: return launch_run<RLB_ENV_CLIFF_WALKING>(e->variant, p, e->store, e->stream);
         default: return launch_run<RLB_ENV_TAXI>(e->variant, p, e->store, e->stream);
     }
+}
+
+#ifndef RLB_EVAL_SPLIT
+#define RLB_EVAL_SPLIT 1   // the on-chip stores' evaluate blocks in k_eval launches of their own (0: inside k_run, fused)
+#endif
+// Fewer agents: the fused kernel's evaluate block already has (nearly) every agent resident — one wave of the hybrid
+// k_run is 7 CTAs x 32 agents per SM, 33 152 agents on 148 SMs — and the two extra launches per block and k_eval's
+// 128-agent CTAs on few SMs cost more than the occupancy gains.  Split against fused, kernel time: +13 / +12 / +8 % at
+// 4 096 / 8 192 / 32 768 agents, -1 / -5 / -7 % at 65 536 / 131 072 / 262 144 (profiles/eval_split_cost.txt).
+#ifndef RLB_EVAL_SPLIT_MIN_AGENTS
+#define RLB_EVAL_SPLIT_MIN_AGENTS (1u << 17)
+#endif
+
+// One launch range of enqueue_range: train episodes [p.ep0, p.ep1) (mode 0) or evaluate p.n_eval episodes (mode 1).
+// The thread-group and hybrid stores hold ~1 KB of shared memory per agent, which caps k_run at a few warps per SM;
+// their evaluate blocks need none of it, so the range is cut where k_run's own loop cuts it (rlb_run_kernel.inc):
+// each training segment runs in k_run with eval_episodes = 0 and its records at their place in the range's block, each
+// evaluate block in k_eval (no records, as the injected evaluate writes none).  The HBM stores
+// and Dyna agents run the range fused, and so do engines of fewer than RLB_EVAL_SPLIT_MIN_AGENTS agents.  `rec`: bytes
+// per episode record; `launches` counts the dispatches (rlb_train_out.kernel_launches).
+cudaError_t run_chunk(rlb_engine* e, const DevParams& p, size_t rec, uint32_t& launches) {
+    if (!RLB_EVAL_SPLIT || !(e->store == STORE_HYBRID || e->store == STORE_SMEM) || p.planning_steps ||
+        e->cfg.n_agents < RLB_EVAL_SPLIT_MIN_AGENTS) {
+        launches += 1;
+        return dispatch_run(e, p);
+    }
+    if (p.mode == 1) {
+        launches += 1;
+        return dispatch_run(e, p, true);
+    }
+    const uint64_t N = e->cfg.n_agents;
+    for (uint64_t ep = p.ep0; ep < p.ep1;) {
+        const uint64_t rem = ep % p.eval_at;
+        const uint64_t gap = rem ? p.eval_at - rem : 0;
+        const uint64_t trig = gap < p.ep1 - ep ? ep + gap : p.ep1;
+        const uint64_t seg_end = trig < p.ep1 ? trig + 1 : p.ep1;
+        DevParams t = p;
+        t.ep0 = ep; t.ep1 = seg_end;
+        t.eval_episodes = 0;   // k_run's own evaluate block at `trig` runs no episode
+        if (p.episodes) t.episodes = (char*)p.episodes + (ep - p.ep0) * N * rec;
+        launches += 1;
+        cudaError_t err = dispatch_run(e, t);
+        if (err != cudaSuccess) return err;
+        if (trig < p.ep1) {   // agent.rs:107-113
+            DevParams v = p;
+            v.mode = 1; v.n_eval = p.eval_episodes; v.episodes = nullptr;
+            launches += 1;
+            err = dispatch_run(e, v, true);
+            if (err != cudaSuccess) return err;
+        }
+        ep = seg_end;
+    }
+    return cudaSuccess;
 }
 
 // Where k_run keeps the per-agent tables.  The shared-memory (thread-group) store pays when every step sweeps many
@@ -677,7 +746,6 @@ rlb_status finish_oldest(rlb_engine* e) {
         float ms = 0.f;
         if (cudaEventElapsedTime(&ms, pd.events[k], pd.events[k + 1]) == cudaSuccess) ms_total += ms; else cudaGetLastError();
     }
-    const uint32_t launches = (uint32_t)(pd.events.size() / 2);
     for (cudaEvent_t ev : pd.events) e->event_pool.push_back(ev);
     e->event_pool.push_back(pd.done);
     if (pd.copies_done) e->event_pool.push_back(pd.copies_done);
@@ -696,7 +764,7 @@ rlb_status finish_oldest(rlb_engine* e) {
     if (pd.mode == 0 && pd.out) {
         pd.out->train_steps = totals[0]; pd.out->eval_steps = totals[1]; pd.out->eval_episodes = totals[2];
         pd.out->eval_return_sum = (double)(long long)totals[3];   // an exact integer (rlb_device.cuh, LaneTotals)
-        pd.out->kernel_ms = ms_total; pd.out->kernel_launches = launches; pd.out->trace_rows = totals[4];
+        pd.out->kernel_ms = ms_total; pd.out->kernel_launches = pd.launches; pd.out->trace_rows = totals[4];
     }
     if (pd.mode == 1 && pd.eval_steps_out) *pd.eval_steps_out = totals[1];
     return status;
@@ -817,7 +885,7 @@ rlb_status enqueue_range(rlb_engine* e, int mode, uint64_t begin, uint64_t end, 
             snprintf(label, sizeof label, "rlb %s env=%d agents=%llu episodes=[%llu,%llu)", mode == 0 ? "train" : "evaluate", e->cfg.env_kind,
                      (unsigned long long)N, (unsigned long long)c0, (unsigned long long)c1);
             nvtxRangePushA(label);
-            cudaError_t lerr = dispatch_run(e, p);
+            cudaError_t lerr = run_chunk(e, p, rec, pd.launches);
             nvtxRangePop();
             if (lerr != cudaSuccess) return cuda_fail(lerr, "k_run launch");
         }

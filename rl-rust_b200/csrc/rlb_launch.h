@@ -44,6 +44,10 @@ enum StepOp {
 // HP = true: the agents run with their own hyper-parameter sets `h` (k_run_hp); instantiated in rlb_inst_<env>_hp.cu
 template <int ENV, bool HP = false> cudaError_t launch_run(const Variant& v, const DevParams& p, int store, cudaStream_t stream,
                                                           const HpParams& h = HpParams{});
+// Agent::evaluate of p.n_eval episodes alone (k_eval, HBM tables): the evaluate blocks of the thread-group and hybrid
+// stores' engines.  FrozenLake and CliffWalking only (cudaErrorInvalidValue otherwise); with HP over the positions of h.
+template <int ENV, bool HP = false> cudaError_t launch_eval(const Variant& v, const DevParams& p, cudaStream_t stream,
+                                                           const HpParams& h = HpParams{});
 // the same with the Dyna model attached (InternalModelAgent): HBM store only; instantiated in rlb_inst_<env>_model.cu, and
 // with HP = true (k_run_hp, per-set planning counts h.planning) in rlb_inst_<env>_model_hp.cu
 template <int ENV, bool HP = false> cudaError_t launch_run_model(const Variant& v, const DevParams& p, cudaStream_t stream,

@@ -152,6 +152,26 @@ cudaError_t launch_run(const Variant& v, const DevParams& p, int store, cudaStre
 }
 
 template <int ENV, bool HP>
+cudaError_t launch_eval(const Variant& v, const DevParams& p, cudaStream_t stream, const HpParams& h) {
+    if constexpr (!SmemCapable<ENV>::value) {
+        return cudaErrorInvalidValue;   // only the on-chip stores' evaluate blocks run apart from k_run
+    } else {
+        const uint64_t n = HP ? h.n_launch : p.n_agents;
+        if (n == 0) return cudaSuccess;
+        const unsigned grid = grid_for(n);
+        const size_t smem = EnvTab<ENV>::smem_bytes(p.S);
+#define RLB_CALL(R, P, SL, T)                                                     \
+    {                                                                             \
+        prefer_l1(k_eval<ENV, R, P, SL, HP>, smem);                               \
+        k_eval<ENV, R, P, SL, HP><<<grid, kBlock, smem, stream>>>(p, h);          \
+    }
+        RLB_VARIANT_SWITCH(v, RLB_CALL)
+#undef RLB_CALL
+        return cudaGetLastError();
+    }
+}
+
+template <int ENV, bool HP>
 cudaError_t launch_run_model(const Variant& v, const DevParams& p, cudaStream_t stream, const HpParams& h) {
     // as launch_run: with per-agent sets the grid covers the launch positions of h (the active sets' agents)
     const uint64_t n = HP ? h.n_launch : p.n_agents;
@@ -267,6 +287,7 @@ cudaError_t launch_step(StepOp op, const Variant& v, const DevParams& p, const S
 
 #define RLB_INSTANTIATE_ENV(ENV)                                                                         \
     template cudaError_t launch_run<ENV, false>(const Variant&, const DevParams&, int, cudaStream_t, const HpParams&); \
+    template cudaError_t launch_eval<ENV, false>(const Variant&, const DevParams&, cudaStream_t, const HpParams&);     \
     template size_t smem_store_bytes<ENV>(const Variant&, int, uint32_t, uint32_t, uint32_t);                           \
     template cudaError_t launch_step<ENV, false>(StepOp, const Variant&, const DevParams&, const StepArgs&, cudaStream_t); \
     template cudaError_t run_kernel_attributes<ENV, false>(const Variant&, int, cudaFuncAttributes*);
@@ -274,6 +295,7 @@ cudaError_t launch_step(StepOp op, const Variant& v, const DevParams& p, const S
 // the same entry points with per-agent hyper-parameter sets (k_run_hp and the _hp step kernels); rlb_inst_<env>_hp.cu
 #define RLB_INSTANTIATE_ENV_HP(ENV)                                                                      \
     template cudaError_t launch_run<ENV, true>(const Variant&, const DevParams&, int, cudaStream_t, const HpParams&);  \
+    template cudaError_t launch_eval<ENV, true>(const Variant&, const DevParams&, cudaStream_t, const HpParams&);      \
     template cudaError_t launch_step<ENV, true>(StepOp, const Variant&, const DevParams&, const StepArgs&, cudaStream_t); \
     template cudaError_t run_kernel_attributes<ENV, true>(const Variant&, int, cudaFuncAttributes*);
 
